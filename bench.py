@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env steps/sec of batched 6-player random playouts (BASELINE.json metric, configs[1]) and MCCFR iterations/sec.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--games G] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--games G] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: G independent preset games per GPU, dealt on the device from
 (seed, global game id) and played uniformly at random to terminal by the fused playout kernel.
@@ -331,6 +331,30 @@ def bench_mccfr(args, rank, world, local, torch):
     return ints, floats, out
 
 
+DUMP_MAX_GAMES = 1 << 20      # 40 B per game written (winner, points[6], steps as float32, game id as float64): 40 MiB at most, plus headers
+
+
+def dump_outputs(eng, out_dir, games, first_gid, ruleset, timed_stats):
+    """Writes the last timed step of the headline figure as a caller of Engine.playout receives it, one float32 / float64 .npy
+    per array, so that two builds can be compared output for output.  stats_*: the outcome statistics the timed call returned.
+    winner, points, steps: per game, from one untimed replay of the same games with per-game outputs; the replay's statistics
+    must equal the timed call's.  Above DUMP_MAX_GAMES games, a fixed seeded sample of the games is written (game_id says which)."""
+    import numpy as np
+    out = eng.playout(games, seed=SEED, first_gid=first_gid, ruleset=ruleset)
+    if any(out["stats"][k] != timed_stats[k] for k in out["stats"]):
+        raise SystemExit("bench.py: the replay of the last timed step differs from it: %r vs %r" % (out["stats"], timed_stats))
+    idx = np.arange(games)
+    if games > DUMP_MAX_GAMES:
+        idx = np.sort(np.random.default_rng(SEED).choice(games, DUMP_MAX_GAMES, replace=False))
+    arrays = {"game_id": (first_gid + idx).astype(np.float64), "winner": out["winner"][idx].astype(np.float32),
+              "points": out["points"][idx].astype(np.float32), "steps": out["steps"][idx].astype(np.float32)}
+    for k, v in out["stats"].items():
+        arrays["stats_" + k] = np.atleast_1d(np.asarray(v, dtype=np.float64))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------- GPU arm
 def main():
     ap = argparse.ArgumentParser()
@@ -345,7 +369,13 @@ def main():
     ap.add_argument("--no-mccfr", action="store_true", help="skip the secondary MCCFR measurement")
     ap.add_argument("--no-classic", action="store_true", help="skip the classic-eight playout figure")
     ap.add_argument("--mccfr-roots", type=int, default=4096)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last weak-scaling step computed as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -391,7 +421,8 @@ def main():
         torch.cuda.synchronize()
 
     def timed_playouts(games, first_gid_of, steps, ruleset):
-        """K steps of `games` fused playouts on this rank.  -> (wall s, kernel ms, env steps, errors, wins[6], launches)"""
+        """K steps of `games` fused playouts on this rank.
+        -> (wall s, kernel ms, env steps, errors, wins[6], launches, statistics of the last step)"""
         launches0 = eng.launches
         kernel_ms, env_steps, errors, wins = 0.0, 0, 0, [0] * 6
         barrier()
@@ -405,7 +436,7 @@ def main():
             errors += st["errors"]
             wins = [a + b for a, b in zip(wins, st["wins"])]
         barrier()
-        return time.perf_counter() - t0, kernel_ms, env_steps, errors, wins, eng.launches - launches0
+        return time.perf_counter() - t0, kernel_ms, env_steps, errors, wins, eng.launches - launches0, st
 
     # warm-up (untimed)
     for w in range(args.warmup):
@@ -417,11 +448,11 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    wall, kernel_ms, env_steps, errors, wins, launches = timed_playouts(G, gid0, args.steps, args.ruleset)
+    wall, kernel_ms, env_steps, errors, wins, launches, last_stats = timed_playouts(G, gid0, args.steps, args.ruleset)
 
     # ---- strong scaling: the same K steps with G games in total, ceil(G / world) per rank ----
     Gs = (G + world - 1) // world
-    s_wall, s_kernel_ms, s_steps, _, _, _ = timed_playouts(Gs, lambda k: (3000 + k) * G + rank * Gs, args.steps, args.ruleset)
+    s_wall, s_kernel_ms, s_steps, _, _, _, _ = timed_playouts(Gs, lambda k: (3000 + k) * G + rank * Gs, args.steps, args.ruleset)
 
     # ---- end-to-end through the public API with HOST buffers: every step copies G packed game records (256 B each) from
     # pinned host memory into the engine's slots (ctd_load_states), plays them to terminal (ctd_playout_slots) and reads
@@ -455,11 +486,14 @@ def main():
     classic = None
     if not args.no_classic and args.ruleset == 0:
         eng.playout(G, seed=SEED, first_gid=gid0(5000), ruleset=1, outputs=False)
-        c_wall, c_ms, c_steps, c_err, _, _ = timed_playouts(G, lambda k: gid0(5001 + k), 2, 1)
+        c_wall, c_ms, c_steps, c_err, _, _, _ = timed_playouts(G, lambda k: gid0(5001 + k), 2, 1)
         classic = [c_wall, c_ms, c_steps, c_err]
 
     # ---- secondary metric: MCCFR iterations/s ----
     mccfr = None if args.no_mccfr else bench_mccfr(args, rank, world, local, torch)
+
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs, G, gid0(args.steps - 1), args.ruleset, last_stats)
 
     # ---- the only collectives: outcome statistics and times, after the timed regions ----
     def reduce(vals, op, dtype):
