@@ -17,6 +17,12 @@ class PlayoutStats(ctypes.Structure):
                 ("errors", ctypes.c_uint64), ("max_steps", ctypes.c_uint64)]
 
 
+class ArenaSeat(ctypes.Structure):
+    """ctd_arena_seat"""
+    _fields_ = [("kind", ctypes.c_int32), ("iterations", ctypes.c_uint32), ("max_depth", ctypes.c_uint32),
+                ("reward_weight", ctypes.c_float)]
+
+
 # every symbol include/citadels_b200.h declares: name -> (restype, argtypes)
 _u32, _u64, _i = ctypes.c_uint32, ctypes.c_uint64, ctypes.c_int
 SIGNATURES = {
@@ -39,6 +45,8 @@ SIGNATURES = {
     "ctd_playout_slots": (_i, [c_void, _u32, _u32, c_void, c_void]),
     "ctd_playout_dev": (_i, [c_void, _u64, _u64, _u64, _i, _u32, ctypes.POINTER(PlayoutStats),
                              ctypes.POINTER(ctypes.c_float)]),
+    "ctd_arena": (_i, [c_void, _u64, _u64, _u64, _i, ctypes.POINTER(ArenaSeat), _u32, c_void, c_void, c_void, c_void,
+                       ctypes.POINTER(PlayoutStats), ctypes.POINTER(ctypes.c_float)]),
     "ctd_launch_count": (_u64, [c_void]),
     "ctd_make_roots": (_i, [c_void, _u32, _u64, _u64, _i, _u32, _u32, _i, c_void]),
     "ctd_load_roots": (_i, [c_void, _u32, c_void, c_void, c_void, c_void]),

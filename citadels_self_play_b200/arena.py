@@ -10,6 +10,10 @@ seats 2-5 uniformly at random; forced moves (one legal option) are played withou
                                           (resp. ctd_mccfr) launch, one tree per game, and the live decision
                                           (CFRNode.action_choice(live=True), algorithms/deep_mccfr.py:67-75, with the
                                           role-preference quirk of game/game.py:312-317) is taken from the result records.
+  play_arena(n_games, seats, model)       the experiment with any player on any seat (random_seat(), pure(it), deep(it,
+                                          depth, weight)), every game resident on the device from deal to end (ctd_arena): the
+                                          host only loops over decision rounds.  Random seats draw from Philox stream 4
+                                          keyed by the game's step count, so results do not depend on batch sizes.
 
 Every search of game g at decision number t runs on the Philox stream keyed (seed, g | t << 40), so successive decisions of
 one game do not reuse draws.  There is no CPU path: games live in 256-byte records, every transition and every search
@@ -20,7 +24,7 @@ import random
 import numpy as np
 
 from .engine import Engine, EngineError, DEFAULT_SEED, RULESET_PRESET
-from .layout import KNOW_BYTES
+from .layout import KNOW_BYTES, SEAT_RANDOM, SEAT_PURE, SEAT_DEEP
 from . import facade as F
 
 
@@ -120,3 +124,67 @@ def play_games_batched(n_games, model=None, engine=None, seed=DEFAULT_SEED, firs
             stats.update(deep_searches=n_search[0], pure_searches=n_search[1], search_launches=search_engine.launches)
         search_engine.close()
     return winners
+
+
+def random_seat():
+    """A seat on random.choice (compare_to_random.py:31)."""
+    return (SEAT_RANDOM, 0, 0, 0.0)
+
+
+def pure(iterations):
+    """A seat on run_mccfr(game, max_iterations=iterations): cfr_train."""
+    return (SEAT_PURE, int(iterations), 0, 0.0)
+
+
+def deep(iterations, max_depth=10, weight=5.0):
+    """A seat on run_mccfr(game, model, max_iterations=iterations): cfr_pred(iterations, max_depth) with the engine's value model."""
+    return (SEAT_DEEP, int(iterations), int(max_depth), float(weight))
+
+
+def default_seats():
+    """compare_to_random.py's layout: seat 0 deep(200, depth 10), seat 1 pure(2000), seats 2-5 random."""
+    return [deep(200, 10, 5.0), pure(2000)] + [random_seat()] * 4
+
+
+def rank_block(n_games, rank, world):
+    """(first game, number of games) of rank `rank` out of `world`: contiguous blocks of ceil(n_games / world) games."""
+    from . import sharding
+    per = -(-int(n_games) // int(world))
+    first = min(int(n_games), sharding.first_gid(0, rank, world, per))
+    return first, min(int(n_games), first + per) - first
+
+
+def play_arena(n_games, seats=None, model=None, engine=None, seed=DEFAULT_SEED, first_gid=0, ruleset=RULESET_PRESET,
+               max_steps=4096, group=None):
+    """compare_to_random.play_games with a player per seat, every game on the device (Engine.arena).  Under torch.distributed
+    each rank plays its own block of game ids (sharding.first_gid over rank_block's split) and the statistics are summed.
+    Without `engine` the games run on torch's current CUDA device (under torchrun: the rank's own GPU after
+    torch.cuda.set_device(LOCAL_RANK)); the statistics are reduced on the engine's device.
+    -> dict(winners[6] and stats over all ranks; this rank's local_stats, first_gid of its games, their per-game arrays
+    winner / points / steps / searches and its phase_ms)."""
+    import torch
+    import torch.distributed as dist
+    from . import sharding
+    seats = default_seats() if seats is None else list(seats)
+    if any(s[0] == SEAT_DEEP for s in seats) and model is None and engine is None:
+        raise ValueError("a deep seat needs a value model")
+    dist_on = dist.is_available() and dist.is_initialized()
+    rank = dist.get_rank(group) if dist_on else 0
+    world = dist.get_world_size(group) if dist_on else 1
+    first, count = rank_block(n_games, rank, world)
+    own = engine is None
+    eng = engine or Engine(capacity=max(1, min(count, 8192)), 
+                            device=torch.cuda.current_device() if torch.cuda.is_available() else 0)
+    try:
+        if model is not None:
+            eng.set_value_model(model)
+        out = eng.arena(count, seats, seed=seed, first_gid=first_gid + first, ruleset=ruleset, max_steps=max_steps)
+    finally:
+        if own:
+            eng.close()
+    local = out["stats"]
+    dev = "cuda:%d" % eng.device if dist_on and dist.get_backend(group) == "nccl" else "cpu"
+    stats = sharding.reduce_stats(local, dev, group=group)
+    stats["max_steps"] = int(sharding.reduce_max([local["max_steps"]], dev, group=group)[0])
+    out.update(winners=list(stats["wins"]), stats=stats, local_stats=local, first_gid=first_gid + first)
+    return out

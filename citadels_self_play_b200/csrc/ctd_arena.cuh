@@ -1,0 +1,206 @@
+// ctd_arena.cuh -- the device-resident arena (ctd_arena): compare_to_random.py:8-37 with a player per seat, every game in HBM
+// from deal to end.  Between two searches ctd_k_arena_advance plays all random and forced moves of every game; a game whose
+// player to move is a search seat with a real choice queues itself for its seat's search group, ctd_k_arena_gather copies the
+// queued roots into the engine's root buffers, the ordinary search runs on them and ctd_k_arena_apply plays the decisions.
+#pragma once
+#include "ctd_playout.cuh"
+#include "ctd_mccfr.cuh"
+
+#define CTD_ARENA_STREAM 4u   // Philox counter word 1 of the random seats' choices (0 game chance, 1 trees, 2 root draws, 3 targets)
+#define CTD_ARENA_GID_BITS 40 // facade.tree_gid: bits 40.. of a tree id carry the game's search number
+
+// what one game keeps between launches
+struct CtdArenaGame {
+  ctd_state rec;
+  CtdKnow kn[6];          // what every seat has learnt (the root of a search is rec + kn[player] + used_cards)
+  uint8_t used_cards[76];
+  uint32_t searches;      // searches made so far: the next one runs on tree id tree_gid(gid, searches)
+};
+
+struct CtdArenaArgs {
+  uint32_t n;
+  uint64_t seed, first_gid;
+  int ruleset;
+  uint32_t max_steps;
+  int8_t seat_group[6];   // search group of each seat, -1 for a random seat
+  CtdArenaGame* games;
+  uint32_t* queue;        // [groups][n] games waiting for a search of that group
+  uint32_t* queued;       // [groups]
+};
+
+// u uniform over [0, n) for the move at step s of game gid: k = (u * n) >> 32, u = word s & 3 of Philox block (s >> 2, 4, gid).
+// Keyed by the step rather than by a running counter, so forced and searched moves consume nothing.
+CTD_HD inline uint32_t ctd_arena_pick(uint64_t seed, uint64_t gid, uint32_t s, uint32_t n) {
+  uint32_t r[4];
+  ctd_philox(s >> 2, CTD_ARENA_STREAM, (uint32_t)gid, (uint32_t)(gid >> 32), (uint32_t)seed, (uint32_t)(seed >> 32), r);
+  return (uint32_t)(((uint64_t)r[s & 3] * n) >> 32);
+}
+
+// Play game `w` (all six observers' knowledge in kn6) from where it stands: every move of a random seat and every forced move,
+// one enumeration per step as in run_utils.py:37-41.  Stops when the game is over (terminal, an error, max_steps) -> -1, or
+// when the player to move belongs to a search group and has >= 2 options -> that group; the record then keeps what the
+// enumeration did to it (Seer / Scholar), as the facade's get_options_from_state before run_mccfr does.
+CTD_HD CTD_NI inline int ctd_arena_advance(CtdWork& w, CtdKnow* kn6, const int8_t* seat_group, uint64_t seed, uint32_t max_steps) {
+  const CtdKnowSet ks{kn6, 6};
+  const uint64_t gid = (uint64_t)w.g0 | ((uint64_t)w.g1 << 32);
+  for (;;) {
+    if ((w.gflags & 2) || w.err) return -1;
+    if (w.steps >= max_steps) { w.err |= CTD_ERR_MAXSTEPS; return -1; }
+    const uint32_t s = w.steps < 65535u ? w.steps : 65535u;   // the record's (saturating) steps field
+    const CtdEnumSave sv = ctd_enum_save(w);
+    CtdEmit e{nullptr, 0, 0, 0xFFFFFFFFu, 0};
+    ctd_enumerate(w, e, kn6);
+    if (e.n == 0) { w.err |= CTD_ERR_REF_RAISE; return -1; }
+    const int g = w.player < 6 ? seat_group[w.player] : -1;
+    if (g >= 0 && e.n >= 2) return g;
+    const uint32_t k = e.n == 1 ? 0u : ctd_arena_pick(seed, gid, s, e.n);
+    ctd_apply(w, ctd_enum_select(w, kn6, sv, k), ks);
+    CTD_LOOP for (int o = 0; o < 6; ++o) w.err |= kn6[o].err;
+  }
+}
+
+// a search's decision on its game (ctd_mccfr_result.live_option); a failed search ends the game with an error flag
+CTD_HD CTD_NI inline void ctd_arena_decide(CtdWork& w, CtdKnow* kn6, uint32_t status, uint64_t live_option) {
+  if (status != 0 || live_option == 0) {
+    w.err |= (status & CTD_TREE_REF_RAISE) || status == 0 ? CTD_ERR_REF_RAISE : CTD_ERR_OVERFLOW;
+    return;
+  }
+  ctd_apply(w, live_option, CtdKnowSet{kn6, 6});
+  CTD_LOOP for (int o = 0; o < 6; ++o) w.err |= kn6[o].err;
+}
+
+#ifdef __CUDACC__
+__device__ __forceinline__ void ctd_arena_know_copy(CtdKnow* dst, const CtdKnow* src, int lane) {
+  for (int i = lane; i < (int)(6 * sizeof(CtdKnow) / 16); i += 32) ((uint4*)dst)[i] = ((const uint4*)src)[i];
+}
+
+// run_utils.create_game for every game, knowledge of all six observers tracked from the deal (ctd_k_one op 0)
+__global__ void __launch_bounds__(CTD_BLOCK) ctd_k_arena_deal(CtdArenaArgs a) {
+  __shared__ CtdWork works[CTD_WARPS_PER_BLOCK];
+  __shared__ CtdKnow knows[CTD_WARPS_PER_BLOCK][6];
+  __shared__ ctd_state stage[CTD_WARPS_PER_BLOCK];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const uint32_t i = blockIdx.x * CTD_WARPS_PER_BLOCK + wib;
+  if (i >= a.n) return;
+  CtdWork& w = works[wib];
+  CtdKnow* kn = knows[wib];
+  CtdArenaGame& G = a.games[i];
+  if (lane == 0) {
+    ctd_chance_init(w, a.seed, a.first_gid + i, 0);
+    ctd_deal_preset(w, a.ruleset, G.used_cards);
+    for (int o = 0; o < 6; ++o) ctd_kn_init(kn[o], o);
+    ctd_setup_round(w, CtdKnowSet{kn, 6});
+    ctd_pack(w, &stage[wib]);
+    G.searches = 0;
+  }
+  __syncwarp();
+  ctd_record_store(&G.rec, &stage[wib], lane);
+  ctd_arena_know_copy(G.kn, kn, lane);
+}
+
+// one warp per game: play on until the game is over or a search seat has to decide (then queue the game for its group)
+__global__ void __launch_bounds__(CTD_BLOCK) ctd_k_arena_advance(CtdArenaArgs a) {
+  __shared__ CtdWork works[CTD_WARPS_PER_BLOCK];
+  __shared__ CtdKnow knows[CTD_WARPS_PER_BLOCK][6];
+  __shared__ ctd_state stage[CTD_WARPS_PER_BLOCK];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const uint32_t i = blockIdx.x * CTD_WARPS_PER_BLOCK + wib;
+  if (i >= a.n) return;
+  CtdWork& w = works[wib];
+  CtdKnow* kn = knows[wib];
+  CtdArenaGame& G = a.games[i];
+  ctd_record_load(&G.rec, &stage[wib], lane);
+  if ((stage[wib].gflags & 2) || stage[wib].err) return;   // over: nothing to do (the warp agrees, the staged record is shared)
+  ctd_arena_know_copy(kn, G.kn, lane);
+  __syncwarp();
+  if (lane == 0) {
+    ctd_unpack(&stage[wib], w);
+    w.k0 = (uint32_t)a.seed; w.k1 = (uint32_t)(a.seed >> 32);
+    w.stream = 0; w.tape = nullptr; w.tape_len = 0;
+    const int g = ctd_arena_advance(w, kn, a.seat_group, a.seed, a.max_steps);
+    ctd_pack(w, &stage[wib]);
+    if (g >= 0) a.queue[(size_t)g * a.n + atomicAdd(&a.queued[g], 1u)] = i;
+  }
+  __syncwarp();
+  ctd_record_store(&G.rec, &stage[wib], lane);
+  ctd_arena_know_copy(G.kn, kn, lane);
+}
+
+// roots [0, count) of a search: queue entries [first, first + count) of `list` -> the engine's root buffers
+__global__ void __launch_bounds__(CTD_BLOCK) ctd_k_arena_gather(const CtdArenaGame* games, const uint32_t* list, uint32_t count,
+                                                                ctd_state* roots, CtdKnow* knows, uint8_t* used_cards, uint64_t* gids) {
+  const int lane = threadIdx.x & 31;
+  const uint32_t j = blockIdx.x * CTD_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+  if (j >= count) return;
+  const CtdArenaGame& G = games[list[j]];
+  reinterpret_cast<uint64_t*>(&roots[j])[lane] = reinterpret_cast<const uint64_t*>(&G.rec)[lane];
+  const int p = G.rec.player < 6 ? G.rec.player : 0;
+  for (int k = lane; k < (int)(sizeof(CtdKnow) / 16); k += 32) ((uint4*)&knows[j])[k] = ((const uint4*)&G.kn[p])[k];
+  for (int k = lane; k < 76; k += 32) used_cards[(size_t)j * 76 + k] = G.used_cards[k];
+  if (lane == 0)
+    gids[j] = (G.rec.gid & ((1ull << CTD_ARENA_GID_BITS) - 1)) | ((uint64_t)G.searches << CTD_ARENA_GID_BITS);
+}
+
+// the decisions of searches [0, count) on the games they came from
+__global__ void __launch_bounds__(CTD_BLOCK) ctd_k_arena_apply(CtdArenaArgs a, const uint32_t* list, uint32_t count,
+                                                               const ctd_mccfr_result* results) {
+  __shared__ CtdWork works[CTD_WARPS_PER_BLOCK];
+  __shared__ CtdKnow knows[CTD_WARPS_PER_BLOCK][6];
+  __shared__ ctd_state stage[CTD_WARPS_PER_BLOCK];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const uint32_t j = blockIdx.x * CTD_WARPS_PER_BLOCK + wib;
+  if (j >= count) return;
+  CtdWork& w = works[wib];
+  CtdKnow* kn = knows[wib];
+  CtdArenaGame& G = a.games[list[j]];
+  ctd_record_load(&G.rec, &stage[wib], lane);
+  ctd_arena_know_copy(kn, G.kn, lane);
+  __syncwarp();
+  if (lane == 0) {
+    ctd_unpack(&stage[wib], w);
+    w.k0 = (uint32_t)a.seed; w.k1 = (uint32_t)(a.seed >> 32);
+    w.stream = 0; w.tape = nullptr; w.tape_len = 0;
+    ctd_arena_decide(w, kn, results[j].status, results[j].live_option);
+    ctd_pack(w, &stage[wib]);
+    G.searches += 1;
+  }
+  __syncwarp();
+  ctd_record_store(&G.rec, &stage[wib], lane);
+  ctd_arena_know_copy(G.kn, kn, lane);
+}
+
+// per-game outputs and the outcome statistics of the finished games (block totals in shared memory, as in the playout kernel)
+__global__ void __launch_bounds__(256) ctd_k_arena_finish(const CtdArenaGame* games, uint32_t n, int8_t* winner, int8_t* points6,
+                                                          uint16_t* steps, uint32_t* searches, ctd_playout_stats* stats) {
+  __shared__ unsigned long long bst[sizeof(ctd_playout_stats) / 8];
+  if (threadIdx.x < sizeof(ctd_playout_stats) / 8) bst[threadIdx.x] = 0;
+  __syncthreads();
+  ctd_playout_stats* bs = reinterpret_cast<ctd_playout_stats*>(bst);
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) {
+    const ctd_state& r = games[i].rec;
+    const int8_t win = r.err ? (int8_t)-1 : r.winner;
+    const unsigned long long ns = r.steps;
+    winner[i] = win; steps[i] = r.steps; searches[i] = games[i].searches;
+    for (int p = 0; p < 6; ++p) {
+      const int pts = r.points[p];
+      points6[(size_t)i * 6 + p] = r.points[p];
+      atomicAdd((unsigned long long*)&bs->points_sum[p], (unsigned long long)(long long)pts);
+      atomicAdd((unsigned long long*)&bs->points_sq[p], (unsigned long long)(pts * pts));
+    }
+    if (win >= 0) atomicAdd((unsigned long long*)&bs->wins[win], 1ull);
+    atomicAdd((unsigned long long*)&bs->games, 1ull);
+    atomicAdd((unsigned long long*)&bs->steps, ns);
+    atomicAdd((unsigned long long*)&bs->steps_sq, ns * ns);
+    if (r.err) atomicAdd((unsigned long long*)&bs->errors, 1ull);
+    atomicMax((unsigned long long*)&bs->max_steps, ns);
+  }
+  __syncthreads();
+  if (threadIdx.x < sizeof(ctd_playout_stats) / 8 && bst[threadIdx.x] != 0) {
+    unsigned long long* gs = reinterpret_cast<unsigned long long*>(stats);
+    const int maxi = offsetof(ctd_playout_stats, max_steps) / 8;
+    if ((int)threadIdx.x == maxi) atomicMax(&gs[maxi], bst[threadIdx.x]);
+    else atomicAdd(&gs[threadIdx.x], bst[threadIdx.x]);
+  }
+}
+#endif  // __CUDACC__

@@ -24,6 +24,7 @@
 #include "ctd_playout.cuh"
 #include "ctd_mccfr.cuh"
 #include "ctd_search.cuh"
+#include "ctd_arena.cuh"
 #include "ctd_value_tc.cuh"
 #include "ctd_train.cuh"
 
@@ -710,7 +711,7 @@ void ctd_destroy(ctd_engine* e) {
 
 const char* ctd_last_error(const ctd_engine* e) { return e ? e->err : "null engine"; }
 // sizes of the records that cross the boundary (binding self-check): 0 ctd_state, 1 ctd_mccfr_result, 2 ctd_target_meta,
-// 3 knowledge block, 4 exported tree header, 5 exported node, 6 child entry, 7 ctd_playout_stats
+// 3 knowledge block, 4 exported tree header, 5 exported node, 6 child entry, 7 ctd_playout_stats, 8 ctd_arena_seat
 uint32_t ctd_sizeof(int what) {
   switch (what) {
     case 0: return (uint32_t)sizeof(ctd_state);
@@ -721,6 +722,7 @@ uint32_t ctd_sizeof(int what) {
     case 5: return (uint32_t)sizeof(CtdNodeOut);
     case 6: return (uint32_t)sizeof(CtdChild);
     case 7: return (uint32_t)sizeof(ctd_playout_stats);
+    case 8: return (uint32_t)sizeof(ctd_arena_seat);
     default: return 0;
   }
 }
@@ -1819,6 +1821,146 @@ ctd_status ctd_mccfr_pred(ctd_engine* e, uint32_t n_roots, uint64_t seed, uint32
   if (n_roots == 0) return CTD_OK;
   CtdSearch sp{n_roots, seed, iterations, ruleset, true, max_depth, reward_weight, false};
   return ctd_search(e, sp, results, elapsed_ms, waves_out);
+}
+
+// ------------------------------------------------------------------------------------------ arena (ctd_arena.cuh)
+// what one ctd_arena call allocates, released on every way out
+struct CtdArenaRun {
+  void* mem[3] = {nullptr, nullptr, nullptr};
+  cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+  ~CtdArenaRun() {
+    for (void* p : mem) if (p) cudaFree(p);
+    for (cudaEvent_t v : ev) if (v) cudaEventDestroy(v);
+  }
+};
+
+ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t first_gid, int ruleset, const ctd_arena_seat seats[6],
+                     uint32_t max_steps, int8_t* winner, int8_t* points6, uint16_t* steps, uint32_t* searches,
+                     ctd_playout_stats* stats, float* elapsed_ms) {
+  // max_steps: the record's steps field saturates at 65535, a larger limit would never be reached
+  if (!e || !seats || n_games > 0xFFFFFFFFull || max_steps > 65535u || (ruleset < CTD_RULESET_PRESET || ruleset > CTD_RULESET_RANDOM))
+    return CTD_EARG;
+  CtdArenaArgs a;
+  memset(&a, 0, sizeof(a));
+  // seats with the same player share a search group: one batch of roots per group and decision round
+  CtdSearch groups[6];
+  int n_groups = 0;
+  for (int s = 0; s < 6; ++s) {
+    const ctd_arena_seat& p = seats[s];
+    a.seat_group[s] = -1;
+    if (p.kind == CTD_SEAT_RANDOM) continue;
+    if ((p.kind != CTD_SEAT_PURE && p.kind != CTD_SEAT_DEEP) || p.iterations == 0 || (p.kind == CTD_SEAT_DEEP && !e->d_model))
+      return CTD_EARG;
+    for (int t = 0; t < s && a.seat_group[s] < 0; ++t)
+      if (a.seat_group[t] >= 0 && seats[t].kind == p.kind && seats[t].iterations == p.iterations && seats[t].max_depth == p.max_depth &&
+          seats[t].reward_weight == p.reward_weight)
+        a.seat_group[s] = a.seat_group[t];
+    if (a.seat_group[s] < 0) {
+      groups[n_groups] = CtdSearch{0, seed, p.iterations, ruleset, p.kind == CTD_SEAT_DEEP, p.max_depth, p.reward_weight, false};
+      a.seat_group[s] = (int8_t)n_groups++;
+    }
+  }
+  float ms[3] = {0.f, 0.f, 0.f};
+  if (n_games == 0) {
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (elapsed_ms) memcpy(elapsed_ms, ms, sizeof(ms));
+    return CTD_OK;
+  }
+  const uint32_t n = (uint32_t)n_games;
+  CTD_CUDA(e, cudaSetDevice(e->device));
+  ctd_status s = ctd_root_buffers(e);
+  if (s != CTD_OK) return s;
+  CtdArenaRun run;
+  const size_t wb = ((size_t)n + 255) & ~(size_t)255, pb = ((size_t)n * 6 + 255) & ~(size_t)255, sb = ((size_t)n * 2 + 255) & ~(size_t)255,
+               cb = (size_t)n * 4;
+  CTD_CUDA(e, cudaMalloc(&run.mem[0], (size_t)n * sizeof(CtdArenaGame)));
+  CTD_CUDA(e, cudaMalloc(&run.mem[1], 256 + (size_t)n_groups * n * sizeof(uint32_t)));
+  CTD_CUDA(e, cudaMalloc(&run.mem[2], wb + pb + sb + ((cb + 255) & ~(size_t)255) + sizeof(ctd_playout_stats)));
+  for (cudaEvent_t& v : run.ev) CTD_CUDA(e, cudaEventCreate(&v));
+  int8_t* d_winner = (int8_t*)run.mem[2];
+  int8_t* d_points = d_winner + wb;
+  uint16_t* d_steps = (uint16_t*)(d_winner + wb + pb);
+  uint32_t* d_searches = (uint32_t*)(d_winner + wb + pb + sb);
+  ctd_playout_stats* d_stats = (ctd_playout_stats*)(d_winner + wb + pb + sb + ((cb + 255) & ~(size_t)255));
+  a.n = n; a.seed = seed; a.first_gid = first_gid; a.ruleset = ruleset; a.max_steps = max_steps;
+  a.games = (CtdArenaGame*)run.mem[0];
+  a.queued = (uint32_t*)run.mem[1];
+  a.queue = a.queued + 64;
+  e->slots_rs_n = 0;
+  // Phase times.  The advance and the search phases end where the host waits anyway (the queue counts, the search's own
+  // read-backs); an apply launch is not waited for: its event pair (ev[2], ev[3]) is read at the next of those waits.
+  bool apply_pending = false;
+  auto timed = [&](int phase) -> ctd_status {
+    CTD_CUDA(e, cudaEventRecord(run.ev[1], e->stream));
+    CTD_CUDA(e, cudaEventSynchronize(run.ev[1]));
+    float t = 0.f;
+    CTD_CUDA(e, cudaEventElapsedTime(&t, run.ev[0], run.ev[1]));
+    ms[phase] += t;
+    if (apply_pending) {
+      CTD_CUDA(e, cudaEventElapsedTime(&t, run.ev[2], run.ev[3]));
+      ms[2] += t;
+      apply_pending = false;
+    }
+    return CTD_OK;
+  };
+  CTD_CUDA(e, cudaEventRecord(run.ev[0], e->stream));
+  ctd_k_arena_deal<<<ctd_blocks(n), CTD_BLOCK, 0, e->stream>>>(a);
+  e->launches++;
+  CTD_CUDA(e, cudaGetLastError());
+  uint32_t queued[6];
+  for (;;) {   // one decision round: every live game plays on to its next search (or its end), then each group searches
+    CTD_CUDA(e, cudaMemsetAsync(a.queued, 0, sizeof(queued), e->stream));
+    ctd_k_arena_advance<<<ctd_blocks(n), CTD_BLOCK, 0, e->stream>>>(a);
+    e->launches++;
+    CTD_CUDA(e, cudaGetLastError());
+    CTD_CUDA(e, cudaMemcpyAsync(queued, a.queued, sizeof(queued), cudaMemcpyDeviceToHost, e->stream));
+    if ((s = timed(0)) != CTD_OK) return s;
+    uint32_t total = 0;
+    for (int g = 0; g < n_groups; ++g) total += queued[g];
+    if (total == 0) break;
+    for (int g = 0; g < n_groups; ++g) {
+      for (uint32_t first = 0; first < queued[g]; first += e->capacity) {   // roots go through the engine's slots, capacity at a time
+        const uint32_t cnt = queued[g] - first < e->capacity ? queued[g] - first : e->capacity;
+        const uint32_t* list = a.queue + (size_t)g * n + first;
+        CTD_CUDA(e, cudaEventRecord(run.ev[0], e->stream));
+        ctd_k_arena_gather<<<ctd_blocks(cnt), CTD_BLOCK, 0, e->stream>>>(a.games, list, cnt, e->d_slots, e->d_knows, e->d_used_cards, e->d_gids);
+        e->launches++;
+        CTD_CUDA(e, cudaGetLastError());
+        CtdSearch sp = groups[g];
+        sp.n_roots = cnt;
+        if ((s = ctd_search(e, sp, nullptr, nullptr, nullptr)) != CTD_OK) return s;   // results stay in d_results
+        if ((s = timed(1)) != CTD_OK) return s;
+        CTD_CUDA(e, cudaEventRecord(run.ev[2], e->stream));
+        ctd_k_arena_apply<<<ctd_blocks(cnt), CTD_BLOCK, 0, e->stream>>>(a, list, cnt, e->d_results);
+        e->launches++;
+        CTD_CUDA(e, cudaGetLastError());
+        CTD_CUDA(e, cudaEventRecord(run.ev[3], e->stream));
+        apply_pending = true;
+      }
+    }
+    CTD_CUDA(e, cudaEventRecord(run.ev[0], e->stream));
+  }
+  CTD_CUDA(e, cudaEventRecord(run.ev[0], e->stream));
+  CTD_CUDA(e, cudaMemsetAsync(d_stats, 0, sizeof(ctd_playout_stats), e->stream));
+  ctd_k_arena_finish<<<(n + 255) / 256, 256, 0, e->stream>>>(a.games, n, d_winner, d_points, d_steps, d_searches, d_stats);
+  e->launches++;
+  CTD_CUDA(e, cudaGetLastError());
+  CTD_CUDA(e, cudaEventRecord(run.ev[1], e->stream));
+  // the final records of the first games stay readable through ctd_store_states
+  const uint32_t keep = n < e->capacity ? n : e->capacity;
+  CTD_CUDA(e, cudaMemcpy2DAsync(e->d_slots, sizeof(ctd_state), &a.games[0].rec, sizeof(CtdArenaGame), sizeof(ctd_state), keep,
+                                cudaMemcpyDeviceToDevice, e->stream));
+  if (winner) CTD_CUDA(e, cudaMemcpyAsync(winner, d_winner, n, cudaMemcpyDeviceToHost, e->stream));
+  if (points6) CTD_CUDA(e, cudaMemcpyAsync(points6, d_points, (size_t)n * 6, cudaMemcpyDeviceToHost, e->stream));
+  if (steps) CTD_CUDA(e, cudaMemcpyAsync(steps, d_steps, (size_t)n * 2, cudaMemcpyDeviceToHost, e->stream));
+  if (searches) CTD_CUDA(e, cudaMemcpyAsync(searches, d_searches, cb, cudaMemcpyDeviceToHost, e->stream));
+  if (stats) CTD_CUDA(e, cudaMemcpyAsync(stats, d_stats, sizeof(ctd_playout_stats), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  float t = 0.f;
+  CTD_CUDA(e, cudaEventElapsedTime(&t, run.ev[0], run.ev[1]));   // the final kernel
+  ms[0] += t;
+  if (elapsed_ms) memcpy(elapsed_ms, ms, sizeof(ms));
+  return CTD_OK;
 }
 
 

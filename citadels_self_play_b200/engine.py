@@ -119,6 +119,25 @@ class Engine:
         d["kernel_ms"] = ms.value
         return dict(stats=d)
 
+    def arena(self, n_games, seats, seed=DEFAULT_SEED, first_gid=0, ruleset=RULESET_PRESET, max_steps=4096):
+        """Games (seed, first_gid + i) played to the end on the device, one player per seat (ctd_arena).
+        seats: six (kind, iterations, max_depth, reward_weight) tuples, kind in layout.SEAT_RANDOM / SEAT_PURE / SEAT_DEEP.
+        -> dict(winner[n] i8 (-1: error), points[n, 6] i8, steps[n] u16, searches[n] u32, stats, phase_ms)."""
+        if len(seats) != 6:
+            raise ValueError("ctd_arena takes one player per seat (6), got %d" % len(seats))
+        arr = (_lib.ArenaSeat * 6)(*[_lib.ArenaSeat(int(k), int(it), int(d), float(wt)) for k, it, d, wt in seats])
+        winner = np.empty(n_games, dtype=np.int8)
+        points = np.empty((n_games, 6), dtype=np.int8)
+        steps = np.empty(n_games, dtype=np.uint16)
+        searches = np.empty(n_games, dtype=np.uint32)
+        stats = _lib.PlayoutStats()
+        ms = (ctypes.c_float * 3)()
+        self._check(self._lib.ctd_arena(self._h, n_games, seed, first_gid, ruleset, arr, max_steps, winner.ctypes.data,
+                                        points.ctypes.data, steps.ctypes.data, searches.ctypes.data, ctypes.byref(stats), ms),
+                    "ctd_arena")
+        return dict(winner=winner, points=points, steps=steps, searches=searches, stats=stats_dict(stats),
+                    phase_ms=dict(advance=ms[0], search=ms[1], apply=ms[2]))
+
     def playout_slots(self, n, max_steps=4096):
         winner = np.empty(n, dtype=np.int8)
         steps = np.empty(n, dtype=np.uint16)

@@ -131,6 +131,9 @@ assert TREE_HDR_DTYPE.itemsize == 128
 NF_ROLE_PICK, NF_TERMINAL = 1, 2
 # tree status bits (include/citadels_b200.h ctd_mccfr_result.status)
 TREE_TERMINAL_ROOT, TREE_EPOOL, TREE_EENGINE, TREE_REF_RAISE = 1, 2, 4, 16
+# ctd_arena_seat.kind, and the Philox counter word 1 of the arena's random seats (draw s of game gid: block s >> 2, word s & 3)
+SEAT_RANDOM, SEAT_PURE, SEAT_DEEP = 0, 1, 2
+ARENA_STREAM = 4
 
 
 def tree_bytes(n_nodes, child_used, arr_used):

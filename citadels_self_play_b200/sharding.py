@@ -24,18 +24,18 @@ def tensor_to_stats(t):
     return d
 
 
-def reduce_stats(stats, device="cpu"):
-    """all_reduce(SUM) of the outcome statistics over the default process group (no-op for a single process)."""
+def reduce_stats(stats, device="cpu", group=None):
+    """all_reduce(SUM) of the outcome statistics over `group` (default: the default process group; no-op for a single process)."""
     import torch.distributed as dist
     t = stats_to_tensor(stats, device)
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        dist.all_reduce(t, op=dist.ReduceOp.SUM)
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
     return tensor_to_stats(t)
 
 
-def reduce_max(values, device="cpu"):
+def reduce_max(values, device="cpu", group=None):
     import torch.distributed as dist
     t = torch.tensor(list(values), dtype=torch.float64, device=device)
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX, group=group)
     return [float(x) for x in t.tolist()]

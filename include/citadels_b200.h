@@ -130,7 +130,8 @@ ctd_status ctd_create(int device, uint32_t capacity, ctd_engine** out);
 void ctd_destroy(ctd_engine* e);
 const char* ctd_last_error(const ctd_engine* e);
 /* sizeof of the records that cross this boundary, for a binding to check its own layouts against: 0 ctd_state, 1 ctd_mccfr_result,
- * 2 ctd_target_meta, 3 knowledge block, 4 exported tree header, 5 exported node, 6 exported child entry, 7 ctd_playout_stats */
+ * 2 ctd_target_meta, 3 knowledge block, 4 exported tree header, 5 exported node, 6 exported child entry, 7 ctd_playout_stats,
+ * 8 ctd_arena_seat */
 uint32_t ctd_sizeof(int what);
 ctd_status ctd_sync(ctd_engine* e);
 /* use an existing CUDA stream (cudaStream_t as void*); default is a stream the engine owns */
@@ -347,6 +348,32 @@ ctd_status ctd_train_get_grads(ctd_engine* e, float* const* tensors16);
  * learning rate lr, then the evaluation pass.  Dropout masks are Philox(seed, optimiser step, layer, element). */
 ctd_status ctd_train_epoch(ctd_engine* e, uint64_t seed, float lr, const uint32_t* perm, double* train_loss, double* eval_loss);
 void ctd_train_end(ctd_engine* e);
+
+/* ---- arena (compare_to_random.py:8-37 with a player per seat) ----
+ * Every game lives on the device from deal to end.  One kernel plays the random and forced moves of all games until each is
+ * over or waits for a search seat with >= 2 legal options; those roots are searched in batches (one tree per game, tree id
+ * (gid & (2^40 - 1)) | t << 40 for the game's t-th search) and the searches' live decisions are applied on the device.
+ * Launches grow with decision rounds, not with env steps. */
+#define CTD_SEAT_RANDOM 0  /* uniform over the legal options: Philox stream 4, draw (s >> 2, s & 3) for the record's steps s */
+#define CTD_SEAT_PURE 1    /* run_mccfr -> cfr_train(iterations) */
+#define CTD_SEAT_DEEP 2    /* run_mccfr -> cfr_pred(iterations, max_depth) with the engine's value model (ctd_set_value_model) */
+typedef struct ctd_arena_seat {
+  int32_t kind;
+  uint32_t iterations;
+  uint32_t max_depth;    /* CTD_SEAT_DEEP only */
+  float reward_weight;   /* CTD_SEAT_DEEP only: model_reward_weights */
+} ctd_arena_seat;
+/* compare_to_random.py:8-37 with a player per seat: n_games games to the end, on the device.  Outputs may be NULL.
+ * searches[n] = searches made in game i.  Like ctd_mccfr, the call replaces the engine's slots and trees: on return slots
+ * [0, min(n_games, capacity)) hold the final records of games [0, min(n_games, capacity)) (ctd_store_states reads them).
+ * Game i is ctd_game_new(seed, first_gid + i, ruleset); a game ends at terminal, on an engine error, on a search status other
+ * than 0 (the game's err gets CTD_ERR_REF_RAISE for status 16, else CTD_ERR_OVERFLOW) or after max_steps steps
+ * (CTD_ERR_MAXSTEPS; max_steps <= 65535, the range of the record's steps field).  Errored games report winner -1 and count in stats->errors.  elapsed_ms (may be NULL) receives three
+ * CUDA-event times: the advance phase (deal, advance and final kernels), the search phase (root gathers and searches) and the
+ * apply phase. */
+ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t first_gid, int ruleset,
+                     const ctd_arena_seat seats[6], uint32_t max_steps, int8_t* winner, int8_t* points6,
+                     uint16_t* steps, uint32_t* searches, ctd_playout_stats* stats, float* elapsed_ms);
 
 /* number of kernels this engine has launched so far */
 uint64_t ctd_launch_count(const ctd_engine* e);
