@@ -11,6 +11,8 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
+#include <initializer_list>
+#include <memory>
 #include <new>
 #include <stddef.h>
 
@@ -535,74 +537,114 @@ __global__ void __launch_bounds__(CTD_BLOCK) ctd_k_encode(const ctd_state* slots
 }
 
 // ------------------------------------------------------------------------------------------ host side / C ABI
+// Device memory (page-locked host memory with Pinned) owned by one holder and freed with it.  grow() reallocates only when
+// asked for more than it holds, freeing the old block first; the size is recorded once the new block exists.
+template <class T, bool Pinned = false>
+struct CtdBuf {
+  T* p = nullptr;
+  size_t bytes = 0;
+  CtdBuf() = default;
+  CtdBuf(const CtdBuf&) = delete;
+  CtdBuf& operator=(const CtdBuf&) = delete;
+  CtdBuf(CtdBuf&& o) noexcept : p(o.p), bytes(o.bytes) { o.p = nullptr; o.bytes = 0; }
+  CtdBuf& operator=(CtdBuf&& o) noexcept {
+    if (this != &o) { reset(); p = o.p; bytes = o.bytes; o.p = nullptr; o.bytes = 0; }
+    return *this;
+  }
+  ~CtdBuf() { reset(); }
+  operator T*() const { return p; }
+  T* get() const { return p; }
+  cudaError_t reset() {
+    const cudaError_t c = p == nullptr ? cudaSuccess : Pinned ? cudaFreeHost(p) : cudaFree(p);
+    p = nullptr; bytes = 0;
+    return c;
+  }
+  cudaError_t grow(size_t n) {
+    if (n <= bytes) return cudaSuccess;
+    cudaError_t c = reset();
+    if (c == cudaSuccess) c = Pinned ? cudaHostAlloc((void**)&p, n, cudaHostAllocDefault) : cudaMalloc((void**)&p, n);
+    if (c == cudaSuccess) bytes = n;
+    else p = nullptr;
+    return c;
+  }
+};
+
+// value-network training (algorithms/train.py:13-86, train_node_value_only) on the device; kernels in ctd_train.cuh.  Every
+// buffer starts zeroed (ctd_train_begin).
+struct CtdTrainer {
+  uint32_t n_train, n_val, batch, bp;   // bp: batch rounded up to a multiple of 32 (the K extent of the weight-gradient products)
+  uint32_t step;                        // optimiser steps taken (Adam bias correction, dropout mask counter)
+  CtdBuf<float> feat_tr, feat_va;
+  CtdBuf<double> val_tr, val_va;
+  CtdBuf<uint32_t> perm;
+  CtdBuf<float> P, G, M, V;             // CtdTrainLayout
+  CtdBuf<float> rm1, rv1, rm2, rv2;     // BatchNorm running statistics
+  CtdBuf<float> X, XT, Z1, H1, H1T, Z2, H2, H2T, H3, dY, dZ3, dZ3T, dH2, dZ2T, dH1, dZ1T, W2T, W3T, inv1, inv2, zero;
+  CtdBuf<double> T, loss;
+};
+
 #define CTD_MAX_ARENAS 6
 struct ctd_engine {
   int device;
   uint32_t slots_rs_n;      // slots [0, slots_rs_n) are known to hold games of ruleset slots_rs (ctd_reset / ctd_load_states):
   int slots_rs;             // lets ctd_playout_slots pick a specialised kernel
   uint32_t capacity;
-  ctd_state* d_slots;
+  CtdBuf<ctd_state> d_slots;
   cudaStream_t stream;
   cudaStream_t stream2;            // second stream of the deep-MCCFR wave pipeline (created on first use)
-  unsigned long long* d_counter2;
-  uint32_t* d_n_pending2;
+  CtdBuf<unsigned long long> d_counter2;
+  CtdBuf<uint32_t> d_n_pending2;
   cudaEvent_t ev_join;
-  uint32_t* h_np;                  // pinned host words the waves report into
+  CtdBuf<uint32_t, true> h_np;     // pinned host words the waves report into
   bool own_stream;
   uint64_t seed;
   uint64_t launches;
   // replay tapes
-  uint8_t* d_tape;
-  uint32_t* d_tape_off;
+  CtdBuf<uint8_t> d_tape;
+  CtdBuf<uint32_t> d_tape_off;
   uint32_t n_tapes;
   // scratch
-  void* d_scratch;
-  size_t scratch_bytes;
-  unsigned long long* d_counter;
-  ctd_playout_stats* d_stats;
+  CtdBuf<uint8_t> d_scratch;
+  CtdBuf<unsigned long long> d_counter;
+  CtdBuf<ctd_playout_stats> d_stats;
   cudaEvent_t ev0, ev1;
   int sm_count;
   // CFR roots (device): parallel to slots
-  CtdKnow* d_knows;
-  uint8_t* d_used_cards;
-  uint64_t* d_gids;
-  uint32_t* d_root_step;
+  CtdBuf<CtdKnow> d_knows;
+  CtdBuf<uint8_t> d_used_cards;
+  CtdBuf<uint64_t> d_gids;
+  CtdBuf<uint32_t> d_root_step;
   // MCCFR trees: one 256-byte header per root + arenas the trees allocate from (arena 0: the whole batch; 1..: retries of
   // trees that found an arena exhausted, each with a larger budget per tree)
-  CtdTreeHdr* d_hdrs;
-  uint8_t* d_arena[CTD_MAX_ARENAS];
-  size_t arena_bytes[CTD_MAX_ARENAS];
-  unsigned long long* d_arena_used;   // [CTD_MAX_ARENAS]
-  uint32_t trees_n;                   // roots searched by the last ctd_mccfr / ctd_mccfr_pred call
-  ctd_mccfr_result* d_results;
-  size_t results_n;
-  uint32_t* d_list;                   // retry lists
-  size_t list_n;
-  uint64_t* d_opts_scratch;
-  size_t opts_scratch_bytes;
+  CtdBuf<CtdTreeHdr> d_hdrs;
+  CtdBuf<uint8_t> d_arena[CTD_MAX_ARENAS];
+  CtdBuf<unsigned long long> d_arena_used;   // [CTD_MAX_ARENAS]
+  uint32_t trees_n;                          // roots searched by the last ctd_mccfr / ctd_mccfr_pred call
+  CtdBuf<ctd_mccfr_result> d_results;
+  CtdBuf<uint32_t> d_list;                   // retry lists
+  CtdBuf<uint64_t> d_opts_scratch;
   // value model (BN folded, transposed) and deep-MCCFR batch buffers
-  float* d_model;
+  CtdBuf<float> d_model;
   CtdValueModel model;
-  float* d_feat;
-  float* d_pred;
-  uint8_t* d_pending;
-  uint32_t* d_n_pending;
-  uint32_t* d_n_epool;   // [1] trees that found their arena exhausted in the passes since it was last cleared
+  CtdBuf<float> d_feat;
+  CtdBuf<float> d_pred;
+  CtdBuf<uint8_t> d_pending;
+  CtdBuf<uint32_t> d_n_pending;
+  CtdBuf<uint32_t> d_n_epool;   // [1] trees that found their arena exhausted in the passes since it was last cleared
   // tensor-core path of the value model: weights as [out][in], activations between layers, error flag
-  float* d_model_tc;
+  CtdBuf<float> d_model_tc;
   const float *tc_w1, *tc_w2, *tc_w3;
-  float *d_h1, *d_h2, *d_h3;
-  int* d_tc_err;
+  CtdBuf<float> d_h1, d_h2, d_h3;
+  CtdBuf<int> d_tc_err;
   // the weights pre-split into their three TF32 terms, [3][N][K] per layer, and their tensor maps (TMA loads of the B operand)
-  float* d_wsplit;
+  CtdBuf<float> d_wsplit;
   CUtensorMap tmap[3];
   bool tmap_ok;
   int value_backend;  // batched evaluations: 0 = fp32 CUDA cores (ctd_k_value_mlp), 1 = tcgen05 split-TF32 (ctd_k_linear_tc)
   int fused;          // deep MCCFR: 1 = one launch, every warp evaluates its own leaves (ctd_value_inline); 0 = waves + batched evaluation
-  uint8_t* h_pinned;  // pinned host staging for result copies
-  size_t pinned_bytes;
-  struct CtdTrainer* trainer;   // value-network training (ctd_train_*), created on first use
-  uint8_t* d_one;  // single-game staging: state | know6 | used_cards | count | winner | opts
+  CtdBuf<uint8_t, true> h_pinned;        // pinned host staging for result copies
+  std::unique_ptr<CtdTrainer> trainer;   // value-network training (ctd_train_*), created on first use
+  CtdBuf<uint8_t> d_one;  // single-game staging: state | know6 | used_cards | count | winner | opts
   char err[256];
 };
 
@@ -616,26 +658,39 @@ static ctd_status ctd_fail(ctd_engine* e, cudaError_t c, const char* where) {
     if (_c != cudaSuccess) return ctd_fail(e, _c, #call);   \
   } while (0)
 
-static ctd_status ctd_scratch(ctd_engine* e, size_t bytes) {
-  if (bytes <= e->scratch_bytes) return CTD_OK;
-  if (e->d_scratch) CTD_CUDA(e, cudaFree(e->d_scratch));
-  e->d_scratch = nullptr;
-  e->scratch_bytes = 0;
-  CTD_CUDA(e, cudaMalloc(&e->d_scratch, bytes));
-  e->scratch_bytes = bytes;
-  return CTD_OK;
-}
-static ctd_status ctd_pinned(ctd_engine* e, size_t bytes) {
-  if (bytes <= e->pinned_bytes) return CTD_OK;
-  if (e->h_pinned) CTD_CUDA(e, cudaFreeHost(e->h_pinned));
-  e->h_pinned = nullptr;
-  e->pinned_bytes = 0;
-  CTD_CUDA(e, cudaHostAlloc((void**)&e->h_pinned, bytes, cudaHostAllocDefault));
-  e->pinned_bytes = bytes;
-  return CTD_OK;
-}
 static CtdTapes ctd_tapes(const ctd_engine* e) { return CtdTapes{e->d_tape, e->d_tape_off, e->n_tapes}; }
 static inline uint32_t ctd_blocks(uint32_t n) { return (n + CTD_WARPS_PER_BLOCK - 1) / CTD_WARPS_PER_BLOCK; }
+
+// A persistent kernel as compiled in its own unit (DESIGN.md 3): its launch and how many of its blocks one SM holds.
+template <class Args>
+struct CtdPersistent {
+  int sm_count;
+  int per_sm;
+  cudaError_t (*launch)(const Args&, int grid, cudaStream_t);
+  // enough blocks to fill every SM at the kernel's occupancy, fewer when the warps of `n` items need fewer (at least one)
+  int grid(uint64_t n) const {
+    const uint64_t want = (uint64_t)sm_count * (per_sm < 1 ? 1 : per_sm), need = (n + CTD_WARPS_PER_BLOCK - 1) / CTD_WARPS_PER_BLOCK;
+    return need == 0 ? 1 : (int)(need < want ? need : want);
+  }
+};
+// the specialised kernel of each family for games of ruleset `rs` (any other value: the generic one)
+static cudaError_t ctd_playout_kernel(int rs, CtdPersistent<CtdPlayoutArgs>& k) {
+  if (rs == CTD_RULESET_PRESET) { k.launch = ctd_playout_preset_launch; return ctd_playout_preset_blocks_per_sm(&k.per_sm); }
+  if (rs == CTD_RULESET_CLASSIC) { k.launch = ctd_playout_classic_launch; return ctd_playout_classic_blocks_per_sm(&k.per_sm); }
+  k.launch = ctd_playout_generic_launch;
+  return ctd_playout_generic_blocks_per_sm(&k.per_sm);
+}
+static cudaError_t ctd_mccfr_kernel(int rs, CtdPersistent<CtdMccfrArgs>& k) {
+  if (rs == CTD_RULESET_PRESET) { k.launch = ctd_mccfr_preset_launch; return ctd_mccfr_preset_blocks_per_sm(&k.per_sm); }
+  k.launch = ctd_mccfr_generic_launch;
+  return ctd_mccfr_generic_blocks_per_sm(&k.per_sm);
+}
+// fused != 0: the fused mode's occupancy (its dynamic shared memory)
+static cudaError_t ctd_pred_kernel(int rs, int fused, CtdPersistent<CtdPredArgs>& k) {
+  if (rs == CTD_RULESET_PRESET) { k.launch = ctd_mccfr_pred_preset_launch; return ctd_mccfr_pred_preset_blocks_per_sm(&k.per_sm, fused); }
+  k.launch = ctd_mccfr_pred_generic_launch;
+  return ctd_mccfr_pred_generic_blocks_per_sm(&k.per_sm, fused);
+}
 
 extern "C" {
 
@@ -643,7 +698,6 @@ ctd_status ctd_create(int device, uint32_t capacity, ctd_engine** out) {
   if (!out || capacity == 0) return CTD_EARG;
   ctd_engine* e = new (std::nothrow) ctd_engine();
   if (!e) return CTD_ENOMEM;
-  memset(e, 0, sizeof(*e));
   e->device = device;
   e->capacity = capacity;
   e->value_backend = 1;  // batched evaluations: dense layers on the tensor cores
@@ -652,11 +706,11 @@ ctd_status ctd_create(int device, uint32_t capacity, ctd_engine** out) {
   CTD_CUDA(e, cudaSetDevice(device));
   CTD_CUDA(e, cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
   e->own_stream = true;
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_slots, (size_t)capacity * sizeof(ctd_state)));
+  CTD_CUDA(e, e->d_slots.grow((size_t)capacity * sizeof(ctd_state)));
   CTD_CUDA(e, cudaMemsetAsync(e->d_slots, 0, (size_t)capacity * sizeof(ctd_state), e->stream));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_counter, sizeof(unsigned long long)));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_n_epool, sizeof(uint32_t)));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_stats, sizeof(ctd_playout_stats)));
+  CTD_CUDA(e, e->d_counter.grow(sizeof(unsigned long long)));
+  CTD_CUDA(e, e->d_n_epool.grow(sizeof(uint32_t)));
+  CTD_CUDA(e, e->d_stats.grow(sizeof(ctd_playout_stats)));
   CTD_CUDA(e, cudaEventCreate(&e->ev0));
   CTD_CUDA(e, cudaEventCreate(&e->ev1));
   CTD_CUDA(e, cudaDeviceGetAttribute(&e->sm_count, cudaDevAttrMultiProcessorCount, device));
@@ -664,49 +718,16 @@ ctd_status ctd_create(int device, uint32_t capacity, ctd_engine** out) {
   return CTD_OK;
 }
 
-void ctd_train_end(ctd_engine* e);
 void ctd_destroy(ctd_engine* e) {
   if (!e) return;
   cudaSetDevice(e->device);
-  ctd_train_end(e);
-  if (e->d_slots) cudaFree(e->d_slots);
-  if (e->d_tape) cudaFree(e->d_tape);
-  if (e->d_tape_off) cudaFree(e->d_tape_off);
-  if (e->d_scratch) cudaFree(e->d_scratch);
-  if (e->d_counter) cudaFree(e->d_counter);
-  if (e->d_counter2) cudaFree(e->d_counter2);
-  if (e->d_n_pending2) cudaFree(e->d_n_pending2);
-  if (e->h_np) cudaFreeHost(e->h_np);
-  if (e->stream2) { cudaStreamDestroy(e->stream2); cudaEventDestroy(e->ev_join); }
-  if (e->d_stats) cudaFree(e->d_stats);
-  if (e->d_knows) cudaFree(e->d_knows);
-  if (e->d_used_cards) cudaFree(e->d_used_cards);
-  if (e->d_gids) cudaFree(e->d_gids);
-  if (e->d_root_step) cudaFree(e->d_root_step);
-  if (e->d_hdrs) cudaFree(e->d_hdrs);
-  for (int i = 0; i < CTD_MAX_ARENAS; ++i) if (e->d_arena[i]) cudaFree(e->d_arena[i]);
-  if (e->d_arena_used) cudaFree(e->d_arena_used);
-  if (e->d_results) cudaFree(e->d_results);
-  if (e->d_list) cudaFree(e->d_list);
-  if (e->d_opts_scratch) cudaFree(e->d_opts_scratch);
-  if (e->d_model) cudaFree(e->d_model);
-  if (e->d_feat) cudaFree(e->d_feat);
-  if (e->d_pred) cudaFree(e->d_pred);
-  if (e->d_pending) cudaFree(e->d_pending);
-  if (e->d_n_pending) cudaFree(e->d_n_pending);
-  if (e->d_n_epool) cudaFree(e->d_n_epool);
-  if (e->d_one) cudaFree(e->d_one);
-  if (e->h_pinned) cudaFreeHost(e->h_pinned);
-  if (e->d_model_tc) cudaFree(e->d_model_tc);
-  if (e->d_h1) cudaFree(e->d_h1);
-  if (e->d_h2) cudaFree(e->d_h2);
-  if (e->d_h3) cudaFree(e->d_h3);
-  if (e->d_tc_err) cudaFree(e->d_tc_err);
-  if (e->d_wsplit) cudaFree(e->d_wsplit);
+  cudaStreamSynchronize(e->stream);
+  if (e->stream2) cudaStreamDestroy(e->stream2);
+  if (e->ev_join) cudaEventDestroy(e->ev_join);
   if (e->ev0) cudaEventDestroy(e->ev0);
   if (e->ev1) cudaEventDestroy(e->ev1);
   if (e->own_stream && e->stream) cudaStreamDestroy(e->stream);
-  delete e;
+  delete e;   // the buffers and the trainer free themselves
 }
 
 const char* ctd_last_error(const ctd_engine* e) { return e ? e->err : "null engine"; }
@@ -802,14 +823,14 @@ ctd_status ctd_set_tapes(ctd_engine* e, uint32_t n, const uint8_t* tape, const u
   if (!e || n > e->capacity) return CTD_EARG;
   CTD_CUDA(e, cudaSetDevice(e->device));
   CTD_CUDA(e, cudaStreamSynchronize(e->stream));
-  if (e->d_tape) { CTD_CUDA(e, cudaFree(e->d_tape)); e->d_tape = nullptr; }
-  if (e->d_tape_off) { CTD_CUDA(e, cudaFree(e->d_tape_off)); e->d_tape_off = nullptr; }
+  CTD_CUDA(e, e->d_tape.reset());
+  CTD_CUDA(e, e->d_tape_off.reset());
   e->n_tapes = 0;
   if (n == 0) return CTD_OK;
   if (!tape || !tape_off) return CTD_EARG;
   size_t bytes = tape_off[n];
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_tape, bytes ? bytes : 1));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_tape_off, (size_t)(n + 1) * sizeof(uint32_t)));
+  CTD_CUDA(e, e->d_tape.grow(bytes ? bytes : 1));
+  CTD_CUDA(e, e->d_tape_off.grow((size_t)(n + 1) * sizeof(uint32_t)));
   CTD_CUDA(e, cudaMemcpy(e->d_tape, tape, bytes, cudaMemcpyHostToDevice));
   CTD_CUDA(e, cudaMemcpy(e->d_tape_off, tape_off, (size_t)(n + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice));
   e->n_tapes = n;
@@ -822,13 +843,12 @@ ctd_status ctd_enumerate(ctd_engine* e, uint32_t n, ctd_option* opts, uint32_t* 
   CTD_CUDA(e, cudaSetDevice(e->device));
   size_t ob = (size_t)n * stride * sizeof(ctd_option), cb = (size_t)n * sizeof(uint32_t);
   size_t cb_al = (cb + 255) & ~(size_t)255, eb_al = ((size_t)n + 255) & ~(size_t)255;
-  ctd_status s = ctd_scratch(e, ob + cb_al + eb_al + 256 + (size_t)n * sizeof(ctd_state));
-  if (s != CTD_OK) return s;
-  ctd_option* d_opts = (ctd_option*)e->d_scratch;
-  uint32_t* d_counts = (uint32_t*)((char*)e->d_scratch + ob);
-  uint8_t* d_errs = (uint8_t*)e->d_scratch + ob + cb_al;
-  uint32_t* d_dirty = (uint32_t*)((char*)e->d_scratch + ob + cb_al + eb_al);
-  ctd_state* d_shadow = (ctd_state*)((char*)e->d_scratch + ob + cb_al + eb_al + 256);
+  CTD_CUDA(e, e->d_scratch.grow(ob + cb_al + eb_al + 256 + (size_t)n * sizeof(ctd_state)));
+  ctd_option* d_opts = (ctd_option*)e->d_scratch.get();
+  uint32_t* d_counts = (uint32_t*)(e->d_scratch + ob);
+  uint8_t* d_errs = e->d_scratch + ob + cb_al;
+  uint32_t* d_dirty = (uint32_t*)(e->d_scratch + ob + cb_al + eb_al);
+  ctd_state* d_shadow = (ctd_state*)(e->d_scratch + ob + cb_al + eb_al + 256);
   CTD_CUDA(e, cudaMemsetAsync(d_dirty, 0, 4, e->stream));
   ctd_k_enumerate<<<ctd_blocks(n), CTD_BLOCK, 0, e->stream>>>(e->d_slots, n, d_opts, d_counts, stride, d_errs, e->seed, ctd_tapes(e),
                                                               d_shadow, d_dirty);
@@ -854,10 +874,9 @@ ctd_status ctd_choose_check(ctd_engine* e, uint32_t n, uint32_t* mismatches) {
   CTD_CUDA(e, cudaSetDevice(e->device));
   const uint32_t cap = 4096;
   size_t ob = (size_t)n * cap * sizeof(ctd_option);
-  ctd_status s = ctd_scratch(e, ob + (size_t)n * 4);
-  if (s != CTD_OK) return s;
-  uint32_t* d_mis = (uint32_t*)((char*)e->d_scratch + ob);
-  ctd_k_choose_check<<<ctd_blocks(n), CTD_BLOCK, 0, e->stream>>>(e->d_slots, n, d_mis, (uint64_t*)e->d_scratch, cap);
+  CTD_CUDA(e, e->d_scratch.grow(ob + (size_t)n * 4));
+  uint32_t* d_mis = (uint32_t*)(e->d_scratch + ob);
+  ctd_k_choose_check<<<ctd_blocks(n), CTD_BLOCK, 0, e->stream>>>(e->d_slots, n, d_mis, (uint64_t*)e->d_scratch.get(), cap);
   e->launches++;
   CTD_CUDA(e, cudaGetLastError());
   CTD_CUDA(e, cudaMemcpyAsync(mismatches, d_mis, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
@@ -870,10 +889,9 @@ ctd_status ctd_step(ctd_engine* e, uint32_t n, const ctd_option* chosen, int8_t*
   if (n == 0) return CTD_OK;
   CTD_CUDA(e, cudaSetDevice(e->device));
   size_t ob = (size_t)n * sizeof(ctd_option);
-  ctd_status s = ctd_scratch(e, ob + n);
-  if (s != CTD_OK) return s;
-  ctd_option* d_chosen = (ctd_option*)e->d_scratch;
-  int8_t* d_winner = (int8_t*)e->d_scratch + ob;
+  CTD_CUDA(e, e->d_scratch.grow(ob + n));
+  ctd_option* d_chosen = (ctd_option*)e->d_scratch.get();
+  int8_t* d_winner = (int8_t*)e->d_scratch.get() + ob;
   CTD_CUDA(e, cudaMemcpyAsync(d_chosen, chosen, ob, cudaMemcpyHostToDevice, e->stream));
   ctd_k_step<<<ctd_blocks(n), CTD_BLOCK, 0, e->stream>>>(e->d_slots, n, d_chosen, d_winner, e->seed, ctd_tapes(e));
   e->launches++;
@@ -883,39 +901,17 @@ ctd_status ctd_step(ctd_engine* e, uint32_t n, const ctd_option* chosen, int8_t*
   return CTD_OK;
 }
 
-// persistent grid: enough CTAs to fill every SM at the kernel's occupancy
-static ctd_status ctd_playout_grid(ctd_engine* e, uint64_t n_games, int* grid, bool preset, bool classic) {
-  int per_sm = 0;
-  if (preset) CTD_CUDA(e, ctd_playout_preset_blocks_per_sm(&per_sm));
-  else if (classic) CTD_CUDA(e, ctd_playout_classic_blocks_per_sm(&per_sm));
-  else CTD_CUDA(e, ctd_playout_generic_blocks_per_sm(&per_sm));
-  if (per_sm < 1) per_sm = 1;
-  uint64_t want = (uint64_t)e->sm_count * per_sm;
-  uint64_t need = (n_games + CTD_WARPS_PER_BLOCK - 1) / CTD_WARPS_PER_BLOCK;
-  *grid = (int)(need < want ? need : want);
-  if (*grid < 1) *grid = 1;
-  return CTD_OK;
-}
-
 static ctd_status ctd_playout_launch(ctd_engine* e, CtdPlayoutArgs& a, ctd_playout_stats* stats, float* elapsed_ms) {
   // every game of this launch is known to play the preset eight: the specialised kernel (ctd_preset_playout.cu)
   const int rs = a.slots == nullptr ? a.ruleset : (a.n_games <= e->slots_rs_n ? e->slots_rs : -1);
-  const bool preset = rs == CTD_RULESET_PRESET, classic = rs == CTD_RULESET_CLASSIC;
-  int grid = 1;
-  ctd_status s = ctd_playout_grid(e, a.n_games, &grid, preset, classic);
-  if (s != CTD_OK) return s;
+  CtdPersistent<CtdPlayoutArgs> k{e->sm_count, 0, nullptr};
+  CTD_CUDA(e, ctd_playout_kernel(rs, k));
   CTD_CUDA(e, cudaMemsetAsync(e->d_counter, 0, sizeof(unsigned long long), e->stream));
   CTD_CUDA(e, cudaMemsetAsync(e->d_stats, 0, sizeof(ctd_playout_stats), e->stream));
   a.counter = e->d_counter;
   a.stats = e->d_stats;
   CTD_CUDA(e, cudaEventRecord(e->ev0, e->stream));
-  if (preset) {
-    CTD_CUDA(e, ctd_playout_preset_launch(a, grid, e->stream));
-  } else if (classic) {
-    CTD_CUDA(e, ctd_playout_classic_launch(a, grid, e->stream));
-  } else {
-    CTD_CUDA(e, ctd_playout_generic_launch(a, grid, e->stream));
-  }
+  CTD_CUDA(e, k.launch(a, k.grid(a.n_games), e->stream));
   e->launches++;
   CTD_CUDA(e, cudaEventRecord(e->ev1, e->stream));
   if (stats) CTD_CUDA(e, cudaMemcpyAsync(stats, e->d_stats, sizeof(ctd_playout_stats), cudaMemcpyDeviceToHost, e->stream));
@@ -943,17 +939,15 @@ ctd_status ctd_playout(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t 
   if (n_games == 0) { if (stats) memset(stats, 0, sizeof(*stats)); return CTD_OK; }
   CTD_CUDA(e, cudaSetDevice(e->device));
   size_t wb = (n_games + 255) & ~(size_t)255, pb = (n_games * 6 + 255) & ~(size_t)255, sb = n_games * 2;
-  ctd_status s = ctd_scratch(e, wb + pb + sb);
-  if (s != CTD_OK) return s;
+  CTD_CUDA(e, e->d_scratch.grow(wb + pb + sb));
   CtdPlayoutArgs a;
   memset(&a, 0, sizeof(a));
   a.n_games = n_games; a.seed = seed; a.first_gid = first_gid; a.ruleset = ruleset; a.max_steps = max_steps;
-  a.winner = (int8_t*)e->d_scratch;
-  a.points6 = (int8_t*)e->d_scratch + wb;
-  a.steps = (uint16_t*)((char*)e->d_scratch + wb + pb);
-  s = ctd_pinned(e, wb + pb + sb);   // results come back through pinned host memory in one DMA
-  if (s != CTD_OK) return s;
-  s = ctd_playout_launch(e, a, stats, nullptr);
+  a.winner = (int8_t*)e->d_scratch.get();
+  a.points6 = (int8_t*)e->d_scratch.get() + wb;
+  a.steps = (uint16_t*)(e->d_scratch + wb + pb);
+  CTD_CUDA(e, e->h_pinned.grow(wb + pb + sb));   // results come back through pinned host memory in one DMA
+  ctd_status s = ctd_playout_launch(e, a, stats, nullptr);
   if (s != CTD_OK) return s;
   CTD_CUDA(e, cudaMemcpyAsync(e->h_pinned, e->d_scratch, wb + pb + sb, cudaMemcpyDeviceToHost, e->stream));
   CTD_CUDA(e, cudaStreamSynchronize(e->stream));
@@ -968,14 +962,13 @@ ctd_status ctd_playout_slots(ctd_engine* e, uint32_t n, uint32_t max_steps, int8
   if (n == 0) return CTD_OK;
   CTD_CUDA(e, cudaSetDevice(e->device));
   size_t wb = ((size_t)n + 255) & ~(size_t)255, sb = (size_t)n * 2;
-  ctd_status s = ctd_scratch(e, wb + sb);
-  if (s != CTD_OK) return s;
+  CTD_CUDA(e, e->d_scratch.grow(wb + sb));
   CtdPlayoutArgs a;
   memset(&a, 0, sizeof(a));
   a.n_games = n; a.seed = e->seed; a.max_steps = max_steps; a.slots = e->d_slots;
-  a.winner = (int8_t*)e->d_scratch;
-  a.steps = (uint16_t*)((char*)e->d_scratch + wb);
-  s = ctd_playout_launch(e, a, nullptr, nullptr);
+  a.winner = (int8_t*)e->d_scratch.get();
+  a.steps = (uint16_t*)(e->d_scratch + wb);
+  ctd_status s = ctd_playout_launch(e, a, nullptr, nullptr);
   if (s != CTD_OK) return s;
   if (winner) CTD_CUDA(e, cudaMemcpyAsync(winner, a.winner, n, cudaMemcpyDeviceToHost, e->stream));
   if (steps) CTD_CUDA(e, cudaMemcpyAsync(steps, a.steps, sb, cudaMemcpyDeviceToHost, e->stream));
@@ -983,15 +976,20 @@ ctd_status ctd_playout_slots(ctd_engine* e, uint32_t n, uint32_t max_steps, int8
   return CTD_OK;
 }
 
+// d_knows stands for the whole group: it is handed to the engine only once every buffer is allocated and cleared, so a
+// failure part way leaves the group absent and the next call tries again
 static ctd_status ctd_root_buffers(ctd_engine* e) {
   if (e->d_knows) return CTD_OK;
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_knows, (size_t)e->capacity * sizeof(CtdKnow)));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_used_cards, (size_t)e->capacity * 76));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_gids, (size_t)e->capacity * sizeof(uint64_t)));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_root_step, (size_t)e->capacity * sizeof(uint32_t)));
-  CTD_CUDA(e, cudaMemsetAsync(e->d_knows, 0, (size_t)e->capacity * sizeof(CtdKnow), e->stream));
-  CTD_CUDA(e, cudaMemsetAsync(e->d_used_cards, 0, (size_t)e->capacity * 76, e->stream));
-  CTD_CUDA(e, cudaMemsetAsync(e->d_gids, 0, (size_t)e->capacity * sizeof(uint64_t), e->stream));
+  const size_t n = e->capacity;
+  CtdBuf<CtdKnow> knows;
+  CTD_CUDA(e, knows.grow(n * sizeof(CtdKnow)));
+  CTD_CUDA(e, e->d_used_cards.grow(n * 76));
+  CTD_CUDA(e, e->d_gids.grow(n * sizeof(uint64_t)));
+  CTD_CUDA(e, e->d_root_step.grow(n * sizeof(uint32_t)));
+  CTD_CUDA(e, cudaMemsetAsync(knows, 0, n * sizeof(CtdKnow), e->stream));
+  CTD_CUDA(e, cudaMemsetAsync(e->d_used_cards, 0, n * 76, e->stream));
+  CTD_CUDA(e, cudaMemsetAsync(e->d_gids, 0, n * sizeof(uint64_t), e->stream));
+  e->d_knows = std::move(knows);
   return CTD_OK;
 }
 
@@ -1073,47 +1071,28 @@ void ctd_mccfr_tree_shape(uint32_t iterations, int ruleset, uint32_t n_roots, ui
 }
 
 static ctd_status ctd_ensure_arena(ctd_engine* e, int idx, size_t bytes) {
-  if (!e->d_arena_used) {
-    CTD_CUDA(e, cudaMalloc((void**)&e->d_arena_used, CTD_MAX_ARENAS * sizeof(unsigned long long)));
-  }
+  CTD_CUDA(e, e->d_arena_used.grow(CTD_MAX_ARENAS * sizeof(unsigned long long)));
   if (!e->d_hdrs) {
-    CTD_CUDA(e, cudaMalloc((void**)&e->d_hdrs, (size_t)e->capacity * sizeof(CtdTreeHdr)));
+    CTD_CUDA(e, e->d_hdrs.grow((size_t)e->capacity * sizeof(CtdTreeHdr)));
     CTD_CUDA(e, cudaMemsetAsync(e->d_hdrs, 0, (size_t)e->capacity * sizeof(CtdTreeHdr), e->stream));
   }
-  if (bytes > e->arena_bytes[idx]) {
-    if (e->d_arena[idx]) { CTD_CUDA(e, cudaStreamSynchronize(e->stream)); CTD_CUDA(e, cudaFree(e->d_arena[idx])); }
-    e->d_arena[idx] = nullptr; e->arena_bytes[idx] = 0;
+  CtdBuf<uint8_t>& arena = e->d_arena[idx];
+  if (bytes > arena.bytes) {
+    if (arena) CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+    CTD_CUDA(e, arena.reset());
     size_t free_b = 0, total_b = 0;
     CTD_CUDA(e, cudaMemGetInfo(&free_b, &total_b));
     if (bytes > free_b - free_b / 8) bytes = free_b - free_b / 8;   // leave an eighth of what is free to everybody else
     bytes &= ~(size_t)255;
-    cudaError_t c = cudaMalloc((void**)&e->d_arena[idx], bytes);
+    cudaError_t c = arena.grow(bytes);
     if (c != cudaSuccess) { (void)cudaGetLastError(); snprintf(e->err, sizeof(e->err), "tree arena of %zu bytes: %s", bytes, cudaGetErrorString(c)); return CTD_ENOMEM; }
-    e->arena_bytes[idx] = bytes;
   }
   const unsigned long long one = 1;   // offset 0 means "none"
   CTD_CUDA(e, cudaMemcpyAsync(e->d_arena_used + idx, &one, sizeof(one), cudaMemcpyHostToDevice, e->stream));
   return CTD_OK;
 }
 static CtdArena ctd_arena_of(ctd_engine* e, int idx) {
-  return CtdArena{e->d_arena[idx], e->d_arena_used + idx, (unsigned long long)(e->arena_bytes[idx] / CTD_ARENA_UNIT)};
-}
-static ctd_status ctd_ensure_results(ctd_engine* e, uint32_t n) {
-  if (n <= e->results_n) return CTD_OK;
-  if (e->d_results) CTD_CUDA(e, cudaFree(e->d_results));
-  e->d_results = nullptr; e->results_n = 0;
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_results, (size_t)n * sizeof(ctd_mccfr_result)));
-  e->results_n = n;
-  return CTD_OK;
-}
-static ctd_status ctd_ensure_opts(ctd_engine* e, size_t warps) {
-  const size_t ob = warps * CTD_MCCFR_OPT_CAP * sizeof(uint64_t);
-  if (ob <= e->opts_scratch_bytes) return CTD_OK;
-  if (e->d_opts_scratch) CTD_CUDA(e, cudaFree(e->d_opts_scratch));
-  e->d_opts_scratch = nullptr; e->opts_scratch_bytes = 0;
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_opts_scratch, ob));
-  e->opts_scratch_bytes = ob;
-  return CTD_OK;
+  return CtdArena{e->d_arena[idx], e->d_arena_used + idx, (unsigned long long)(e->d_arena[idx].bytes / CTD_ARENA_UNIT)};
 }
 
 // what one search call asks for
@@ -1132,15 +1111,10 @@ static ctd_status ctd_pred_buffers(ctd_engine* e);
 
 // one pass of pure MCCFR over `n` trees (d_list: their root indices, or null for roots [0, n)) allocating from arena `ai`
 static ctd_status ctd_pure_pass(ctd_engine* e, const CtdSearch& sp, const uint32_t* d_list, uint32_t n, int ai) {
-  const bool preset = sp.ruleset == CTD_RULESET_PRESET;   // the roots were made / loaded for this ruleset: specialised kernel
-  int per_sm = 0;
-  if (preset) CTD_CUDA(e, ctd_mccfr_preset_blocks_per_sm(&per_sm));
-  else CTD_CUDA(e, ctd_mccfr_generic_blocks_per_sm(&per_sm));
-  if (per_sm < 1) per_sm = 1;
-  const uint64_t want = (uint64_t)e->sm_count * per_sm, needb = (n + CTD_WARPS_PER_BLOCK - 1) / CTD_WARPS_PER_BLOCK;
-  const int grid = (int)(needb < want ? needb : want);
-  ctd_status s = ctd_ensure_opts(e, (size_t)grid * CTD_WARPS_PER_BLOCK);
-  if (s != CTD_OK) return s;
+  CtdPersistent<CtdMccfrArgs> k{e->sm_count, 0, nullptr};   // the roots were made / loaded for this ruleset: its kernel
+  CTD_CUDA(e, ctd_mccfr_kernel(sp.ruleset, k));
+  const int grid = k.grid(n);
+  CTD_CUDA(e, e->d_opts_scratch.grow((size_t)grid * CTD_WARPS_PER_BLOCK * CTD_MCCFR_OPT_CAP * sizeof(uint64_t)));
   CtdMccfrArgs a;
   memset(&a, 0, sizeof(a));
   a.n_roots = n; a.tree_list = d_list; a.roots = e->d_slots; a.knows = e->d_knows; a.used_cards = e->d_used_cards; a.gids = e->d_gids;
@@ -1148,8 +1122,7 @@ static ctd_status ctd_pure_pass(ctd_engine* e, const CtdSearch& sp, const uint32
   a.results = e->d_results; a.counter = e->d_counter; a.opts_scratch = e->d_opts_scratch; a.resume = sp.resume ? 1 : 0;
   a.n_epool = e->d_n_epool;
   CTD_CUDA(e, cudaMemsetAsync(e->d_counter, 0, sizeof(unsigned long long), e->stream));
-  if (preset) CTD_CUDA(e, ctd_mccfr_preset_launch(a, grid, e->stream));
-  else CTD_CUDA(e, ctd_mccfr_generic_launch(a, grid, e->stream));
+  CTD_CUDA(e, k.launch(a, grid, e->stream));
   e->launches++;
   CTD_CUDA(e, cudaGetLastError());
   return CTD_OK;
@@ -1170,25 +1143,19 @@ static ctd_status ctd_deep_pass(ctd_engine* e, const CtdSearch& sp, const uint32
     if (p.budget == 0) p.budget = 0xFFFFFFFFu;
   }
   p.max_depth = sp.max_depth; p.feat = e->d_feat; p.pred = e->d_pred; p.pending = e->d_pending;
-  int per_sm = 0;
-  const bool preset = sp.ruleset == CTD_RULESET_PRESET;
-  if (preset) CTD_CUDA(e, ctd_mccfr_pred_preset_blocks_per_sm(&per_sm, e->fused));
-  else CTD_CUDA(e, ctd_mccfr_pred_generic_blocks_per_sm(&per_sm, e->fused));
-  if (per_sm < 1) per_sm = 1;
+  CtdPersistent<CtdPredArgs> k{e->sm_count, 0, nullptr};
+  CTD_CUDA(e, ctd_pred_kernel(sp.ruleset, e->fused, k));
   if (e->fused) {
     // fused: one launch; every warp walks its tree to the end and evaluates the leaves it meets itself (ctd_value_inline)
     p.fused = 1; p.budget = 0xFFFFFFFFu; p.first = 1;
     p.net = CtdValueNet{e->model.w1t, e->model.b1, e->model.w2t, e->model.b2, e->model.w3t, e->model.b3, e->model.w4t, e->model.b4, sp.weight};
-    const uint64_t want = (uint64_t)e->sm_count * per_sm, needb = (n + CTD_WARPS_PER_BLOCK - 1) / CTD_WARPS_PER_BLOCK;
-    const int grid = (int)(needb < want ? needb : want);
-    ctd_status s = ctd_ensure_opts(e, (size_t)grid * CTD_WARPS_PER_BLOCK);
-    if (s != CTD_OK) return s;
+    const int grid = k.grid(n);
+    CTD_CUDA(e, e->d_opts_scratch.grow((size_t)grid * CTD_WARPS_PER_BLOCK * CTD_MCCFR_OPT_CAP * sizeof(uint64_t)));
     a.tree_list = d_list; a.first_root = 0; a.n_roots = n; a.counter = e->d_counter; a.opts_scratch = e->d_opts_scratch;
     p.n_pending = e->d_n_pending;
     CTD_CUDA(e, cudaMemsetAsync(e->d_counter, 0, sizeof(unsigned long long), e->stream));
     CTD_CUDA(e, cudaMemsetAsync(e->d_n_pending, 0, 2 * sizeof(uint32_t), e->stream));
-    if (preset) CTD_CUDA(e, ctd_mccfr_pred_preset_launch(p, grid, e->stream));
-    else CTD_CUDA(e, ctd_mccfr_pred_generic_launch(p, grid, e->stream));
+    CTD_CUDA(e, k.launch(p, grid, e->stream));
     e->launches++;
     CTD_CUDA(e, cudaGetLastError());
     if (waves_out) *waves_out = 1;
@@ -1199,10 +1166,10 @@ static ctd_status ctd_deep_pass(ctd_engine* e, const CtdSearch& sp, const uint32
   // group's kernel instead of idling the GPU.  Trees are independent, results do not depend on the grouping.
   const char* genv = getenv("CTD_PRED_GROUPS");
   const int G = (genv ? atoi(genv) : 2) >= 2 && n >= 1024 ? 2 : 1;
-  if (G == 2 && !e->stream2) {
-    CTD_CUDA(e, cudaStreamCreateWithFlags(&e->stream2, cudaStreamNonBlocking));
-    CTD_CUDA(e, cudaMalloc((void**)&e->d_counter2, sizeof(unsigned long long)));
-    CTD_CUDA(e, cudaMalloc((void**)&e->d_n_pending2, 2 * sizeof(uint32_t)));
+  if (G == 2 && !e->ev_join) {   // the join event comes last: a failure part way is completed by the next call
+    if (!e->stream2) CTD_CUDA(e, cudaStreamCreateWithFlags(&e->stream2, cudaStreamNonBlocking));
+    CTD_CUDA(e, e->d_counter2.grow(sizeof(unsigned long long)));
+    CTD_CUDA(e, e->d_n_pending2.grow(2 * sizeof(uint32_t)));
     CTD_CUDA(e, cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming));
   }
   const uint32_t split = G == 2 ? ((n / 2 + 7) & ~7u) : n;
@@ -1213,13 +1180,12 @@ static ctd_status ctd_deep_pass(ctd_engine* e, const CtdSearch& sp, const uint32
   int g_grid[2];
   size_t g_opts_off[2] = {0, 0}, warps = 0;
   for (int g = 0; g < G; ++g) {
-    uint64_t want = (uint64_t)e->sm_count * per_sm, needb = (g_n[g] + CTD_WARPS_PER_BLOCK - 1) / CTD_WARPS_PER_BLOCK;
-    g_grid[g] = (int)(needb < want ? needb : want);
+    g_grid[g] = k.grid(g_n[g]);
     g_opts_off[g] = warps * CTD_MCCFR_OPT_CAP;
     warps += (size_t)g_grid[g] * CTD_WARPS_PER_BLOCK;
   }
-  ctd_status s = ctd_ensure_opts(e, warps);
-  if (s != CTD_OK) return s;
+  CTD_CUDA(e, e->d_opts_scratch.grow(warps * CTD_MCCFR_OPT_CAP * sizeof(uint64_t)));
+  ctd_status s = CTD_OK;
   if (G == 2) {
     CTD_CUDA(e, cudaEventRecord(e->ev_join, e->stream));
     CTD_CUDA(e, cudaStreamWaitEvent(e->stream2, e->ev_join, 0));
@@ -1235,8 +1201,7 @@ static ctd_status ctd_deep_pass(ctd_engine* e, const CtdSearch& sp, const uint32
     q.first = g_waves[g] == 0;
     CTD_CUDA(e, cudaMemsetAsync(g_counter[g], 0, sizeof(unsigned long long), g_stream[g]));
     CTD_CUDA(e, cudaMemsetAsync(g_pending[g], 0, 2 * sizeof(uint32_t), g_stream[g]));
-    if (preset) CTD_CUDA(e, ctd_mccfr_pred_preset_launch(q, g_grid[g], g_stream[g]));
-    else CTD_CUDA(e, ctd_mccfr_pred_generic_launch(q, g_grid[g], g_stream[g]));
+    CTD_CUDA(e, k.launch(q, g_grid[g], g_stream[g]));
     e->launches++;
     CTD_CUDA(e, cudaMemcpyAsync(h_np + 2 * g, g_pending[g], 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, g_stream[g]));
     ++g_waves[g];
@@ -1284,8 +1249,8 @@ static ctd_status ctd_deep_pass(ctd_engine* e, const CtdSearch& sp, const uint32
 // tree, and so on (a tree is a pure function of (seed, root, gid), so the second search is the same search).
 static ctd_status ctd_search(ctd_engine* e, const CtdSearch& sp, ctd_mccfr_result* results, float* elapsed_ms, uint32_t* waves_out) {
   CTD_CUDA(e, cudaSetDevice(e->device));
-  ctd_status s = ctd_ensure_results(e, sp.n_roots);
-  if (s != CTD_OK) return s;
+  CTD_CUDA(e, e->d_results.grow((size_t)sp.n_roots * sizeof(ctd_mccfr_result)));
+  ctd_status s = CTD_OK;
   if (sp.deep) { s = ctd_pred_buffers(e); if (s != CTD_OK) return s; }
   if (sp.resume) {   // the trees stay where they are (arena 0 keeps its bump pointer); trees that run out of arena now keep status 2
     if (!e->d_hdrs || sp.n_roots > e->trees_n || sp.deep) return CTD_EARG;
@@ -1302,7 +1267,7 @@ static ctd_status ctd_search(ctd_engine* e, const CtdSearch& sp, ctd_mccfr_resul
   size_t arena0 = (size_t)(budget * sp.n_roots + (64ull << 20));
   if (const char* env = getenv("CTD_ARENA0_BYTES")) {   // test hook: a squeezed first arena exercises the retry path
     arena0 = (size_t)strtoull(env, nullptr, 10);
-    if (e->d_arena[0] && e->arena_bytes[0] != arena0) { CTD_CUDA(e, cudaStreamSynchronize(e->stream)); CTD_CUDA(e, cudaFree(e->d_arena[0])); e->d_arena[0] = nullptr; e->arena_bytes[0] = 0; }
+    if (e->d_arena[0] && e->d_arena[0].bytes != arena0) { CTD_CUDA(e, cudaStreamSynchronize(e->stream)); CTD_CUDA(e, e->d_arena[0].reset()); }
   }
   s = ctd_ensure_arena(e, 0, arena0);
   if (s != CTD_OK) return s;
@@ -1313,42 +1278,30 @@ static ctd_status ctd_search(ctd_engine* e, const CtdSearch& sp, ctd_mccfr_resul
   if (s != CTD_OK) return s;
   CTD_CUDA(e, cudaEventRecord(e->ev1, e->stream));
   // which trees ran out of arena?  (status word of every header: 256-byte stride, 4 bytes each)
-  uint32_t* st = new (std::nothrow) uint32_t[sp.n_roots];
+  std::unique_ptr<uint32_t[]> st(new (std::nothrow) uint32_t[sp.n_roots]);
   if (!st) return CTD_ENOMEM;
-  ctd_status rs = CTD_OK;
   for (int ai = 1; ai < CTD_MAX_ARENAS; ++ai) {
     uint32_t any = 0;   // one word first: the strided read-back of every header's status costs a DMA descriptor per tree
-    cudaError_t c = cudaMemcpyAsync(&any, e->d_n_epool, sizeof(uint32_t), cudaMemcpyDeviceToHost, e->stream);
-    if (c == cudaSuccess) c = cudaStreamSynchronize(e->stream);
-    if (c != cudaSuccess) { rs = ctd_fail(e, c, "exhausted-tree count read-back"); break; }
+    CTD_CUDA(e, cudaMemcpyAsync(&any, e->d_n_epool, sizeof(uint32_t), cudaMemcpyDeviceToHost, e->stream));
+    CTD_CUDA(e, cudaStreamSynchronize(e->stream));
     if (any == 0) break;
-    c = cudaMemsetAsync(e->d_n_epool, 0, sizeof(uint32_t), e->stream);
-    if (c == cudaSuccess) c = cudaMemcpy2DAsync(st, sizeof(uint32_t), (const uint8_t*)e->d_hdrs + offsetof(CtdTreeHdr, status), sizeof(CtdTreeHdr),
-                                      sizeof(uint32_t), sp.n_roots, cudaMemcpyDeviceToHost, e->stream);
-    if (c == cudaSuccess) c = cudaStreamSynchronize(e->stream);
-    if (c != cudaSuccess) { rs = ctd_fail(e, c, "tree status read-back"); break; }
+    CTD_CUDA(e, cudaMemsetAsync(e->d_n_epool, 0, sizeof(uint32_t), e->stream));
+    CTD_CUDA(e, cudaMemcpy2DAsync(st.get(), sizeof(uint32_t), (const uint8_t*)e->d_hdrs.get() + offsetof(CtdTreeHdr, status),
+                                  sizeof(CtdTreeHdr), sizeof(uint32_t), sp.n_roots, cudaMemcpyDeviceToHost, e->stream));
+    CTD_CUDA(e, cudaStreamSynchronize(e->stream));
     uint32_t nf = 0;
     for (uint32_t t = 0; t < sp.n_roots; ++t) if (st[t] & CTD_TREE_EPOOL) st[nf++] = t;
     if (nf == 0) break;
-    if (nf > e->list_n) {
-      if (e->d_list) cudaFree(e->d_list);
-      e->d_list = nullptr; e->list_n = 0;
-      c = cudaMalloc((void**)&e->d_list, (size_t)nf * sizeof(uint32_t));
-      if (c != cudaSuccess) { rs = ctd_fail(e, c, "retry list"); break; }
-      e->list_n = nf;
-    }
-    c = cudaMemcpyAsync(e->d_list, st, (size_t)nf * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream);
-    if (c != cudaSuccess) { rs = ctd_fail(e, c, "retry list upload"); break; }
+    CTD_CUDA(e, e->d_list.grow((size_t)nf * sizeof(uint32_t)));
+    CTD_CUDA(e, cudaMemcpyAsync(e->d_list, st.get(), (size_t)nf * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
     budget *= 16;
-    rs = ctd_ensure_arena(e, ai, (size_t)(budget * nf + (64ull << 20)));
-    if (rs != CTD_OK) break;
-    rs = sp.deep ? ctd_deep_pass(e, sp, e->d_list, nf, ai, nullptr) : ctd_pure_pass(e, sp, e->d_list, nf, ai);
-    if (rs != CTD_OK) break;
-    if (cudaEventRecord(e->ev1, e->stream) != cudaSuccess) { rs = CTD_ECUDA; break; }   // the reported kernel time covers every pass
-    CTD_CUDA(e, cudaStreamSynchronize(e->stream));   // `st` is reused as the upload source
+    s = ctd_ensure_arena(e, ai, (size_t)(budget * nf + (64ull << 20)));
+    if (s != CTD_OK) return s;
+    s = sp.deep ? ctd_deep_pass(e, sp, e->d_list, nf, ai, nullptr) : ctd_pure_pass(e, sp, e->d_list, nf, ai);
+    if (s != CTD_OK) return s;
+    CTD_CUDA(e, cudaEventRecord(e->ev1, e->stream));   // the reported kernel time covers every pass
+    CTD_CUDA(e, cudaStreamSynchronize(e->stream));     // `st` is reused as the upload source
   }
-  delete[] st;
-  if (rs != CTD_OK) return rs;
   if (results) CTD_CUDA(e, cudaMemcpyAsync(results, e->d_results, (size_t)sp.n_roots * sizeof(ctd_mccfr_result), cudaMemcpyDeviceToHost, e->stream));
   CTD_CUDA(e, cudaStreamSynchronize(e->stream));
   if (elapsed_ms) CTD_CUDA(e, cudaEventElapsedTime(elapsed_ms, e->ev0, e->ev1));
@@ -1398,9 +1351,8 @@ ctd_status ctd_mccfr_root_set(ctd_engine* e, uint32_t n_roots, uint32_t stride, 
   if (n_roots == 0) return CTD_OK;
   CTD_CUDA(e, cudaSetDevice(e->device));
   const size_t ab = (size_t)n_roots * stride * sizeof(double), vb = (size_t)n_roots * 6 * sizeof(double);
-  ctd_status s = ctd_scratch(e, 2 * ab + vb);
-  if (s != CTD_OK) return s;
-  double* d = (double*)e->d_scratch;
+  CTD_CUDA(e, e->d_scratch.grow(2 * ab + vb));
+  double* d = (double*)e->d_scratch.get();
   CTD_CUDA(e, cudaMemcpyAsync(d, cumulative_regrets, ab, cudaMemcpyHostToDevice, e->stream));
   CTD_CUDA(e, cudaMemcpyAsync(d + (size_t)n_roots * stride, cumulative_strategy, ab, cudaMemcpyHostToDevice, e->stream));
   CTD_CUDA(e, cudaMemcpyAsync(d + 2 * (size_t)n_roots * stride, node_value, vb, cudaMemcpyHostToDevice, e->stream));
@@ -1416,42 +1368,31 @@ ctd_status ctd_mccfr_export(ctd_engine* e, uint32_t first, uint32_t n, uint64_t*
   if (!e || !sizes || !e->d_hdrs || (uint64_t)first + n > e->trees_n) return CTD_EARG;
   if (n == 0) return CTD_OK;
   CTD_CUDA(e, cudaSetDevice(e->device));
-  CtdTreeHdr* hh = new (std::nothrow) CtdTreeHdr[n];
-  if (!hh) return CTD_ENOMEM;
-  cudaError_t c = cudaMemcpyAsync(hh, e->d_hdrs + first, (size_t)n * sizeof(CtdTreeHdr), cudaMemcpyDeviceToHost, e->stream);
-  if (c == cudaSuccess) c = cudaStreamSynchronize(e->stream);
-  if (c != cudaSuccess) { delete[] hh; return ctd_fail(e, c, "tree headers"); }
+  std::unique_ptr<CtdTreeHdr[]> hh(new (std::nothrow) CtdTreeHdr[n]);
+  std::unique_ptr<uint64_t[]> off(new (std::nothrow) uint64_t[n]);
+  if (!hh || !off) return CTD_ENOMEM;
+  CTD_CUDA(e, cudaMemcpyAsync(hh.get(), e->d_hdrs + first, (size_t)n * sizeof(CtdTreeHdr), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
   uint64_t total = 0;
-  uint64_t* off = new (std::nothrow) uint64_t[n];
-  if (!off) { delete[] hh; return CTD_ENOMEM; }
   for (uint32_t i = 0; i < n; ++i) {
     sizes[i] = (ctd_tree_export_bytes(hh[i].n_nodes, hh[i].child_used, hh[i].arr_used) + 15) & ~(uint64_t)15;
     off[i] = total;
     total += sizes[i];
   }
-  delete[] hh;
-  ctd_status rs = CTD_OK;
-  if (buf) {
-    if (buf_bytes < total) { delete[] off; return CTD_ECAP; }
-    uint8_t* d_out = nullptr;
-    uint64_t* d_off = nullptr;
-    c = cudaMalloc((void**)&d_out, total);
-    if (c == cudaSuccess) c = cudaMalloc((void**)&d_off, (size_t)n * sizeof(uint64_t));
-    if (c == cudaSuccess) c = cudaMemcpyAsync(d_off, off, (size_t)n * sizeof(uint64_t), cudaMemcpyHostToDevice, e->stream);
-    if (c == cudaSuccess) c = cudaMemsetAsync(d_out, 0, total, e->stream);
-    if (c == cudaSuccess) {
-      ctd_k_export_trees<<<ctd_blocks(n), CTD_BLOCK, 0, e->stream>>>(e->d_hdrs, first, n, d_off, d_out);
-      e->launches++;
-      c = cudaGetLastError();
-    }
-    if (c == cudaSuccess) c = cudaMemcpyAsync(buf, d_out, total, cudaMemcpyDeviceToHost, e->stream);
-    if (c == cudaSuccess) c = cudaStreamSynchronize(e->stream);
-    if (d_out) cudaFree(d_out);
-    if (d_off) cudaFree(d_off);
-    if (c != cudaSuccess) rs = ctd_fail(e, c, "tree export");
-  }
-  delete[] off;
-  return rs;
+  if (!buf) return CTD_OK;
+  if (buf_bytes < total) return CTD_ECAP;
+  CtdBuf<uint8_t> d_out;
+  CtdBuf<uint64_t> d_off;
+  CTD_CUDA(e, d_out.grow(total));
+  CTD_CUDA(e, d_off.grow((size_t)n * sizeof(uint64_t)));
+  CTD_CUDA(e, cudaMemcpyAsync(d_off, off.get(), (size_t)n * sizeof(uint64_t), cudaMemcpyHostToDevice, e->stream));
+  CTD_CUDA(e, cudaMemsetAsync(d_out, 0, total, e->stream));
+  ctd_k_export_trees<<<ctd_blocks(n), CTD_BLOCK, 0, e->stream>>>(e->d_hdrs, first, n, d_off, d_out);
+  e->launches++;
+  CTD_CUDA(e, cudaGetLastError());
+  CTD_CUDA(e, cudaMemcpyAsync(buf, d_out, total, cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  return CTD_OK;
 }
 
 // children [first, first + count) of the root of tree `tree`: descriptors and, for vector nodes, regrets / strategy / cumulative
@@ -1462,10 +1403,9 @@ ctd_status ctd_mccfr_root_children(ctd_engine* e, uint32_t tree, uint32_t first,
   if (count == 0) return CTD_OK;
   CTD_CUDA(e, cudaSetDevice(e->device));
   const size_t ob = (size_t)count * sizeof(ctd_option), db = (size_t)count * sizeof(double);
-  ctd_status s = ctd_scratch(e, ob + 3 * db);
-  if (s != CTD_OK) return s;
-  ctd_option* d_o = (ctd_option*)e->d_scratch;
-  double* d_r = (double*)((char*)e->d_scratch + ob);
+  CTD_CUDA(e, e->d_scratch.grow(ob + 3 * db));
+  ctd_option* d_o = (ctd_option*)e->d_scratch.get();
+  double* d_r = (double*)(e->d_scratch + ob);
   CTD_CUDA(e, cudaMemsetAsync(e->d_scratch, 0, ob + 3 * db, e->stream));
   ctd_k_root_children<<<(count + 255) / 256 < 64 ? (count + 255) / 256 : 64, 256, 0, e->stream>>>(e->d_hdrs, tree, first, count, d_o, d_r, d_r + count, d_r + 2 * count);
   e->launches++;
@@ -1486,103 +1426,75 @@ ctd_status ctd_mccfr_root_children(ctd_engine* e, uint32_t tree, uint32_t first,
 #define CTD_ONE_WINNER_OFF (CTD_ONE_COUNT_OFF + 4)
 #define CTD_ONE_OPTS_OFF (CTD_ONE_COUNT_OFF + 8)
 #define CTD_ONE_BYTES (CTD_ONE_OPTS_OFF + CTD_ONE_OPTS * 8)
-static ctd_status ctd_one_buffer(ctd_engine* e) {
-  if (e->d_one) return CTD_OK;
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_one, CTD_ONE_BYTES));
+// a block of the staging buffer (offset, bytes) and the host memory it is copied from or to (null: not copied)
+struct CtdOneCopy {
+  const void* host;
+  size_t off, bytes;
+};
+// one ctd_k_one op on the staging buffer: upload `up`, run `a` (its op fields set by the caller; know: with the knowledge
+// block), download `down`, synchronise
+static ctd_status ctd_game_op(ctd_engine* e, CtdOneArgs a, bool know, std::initializer_list<CtdOneCopy> up,
+                              std::initializer_list<CtdOneCopy> down) {
+  CTD_CUDA(e, cudaSetDevice(e->device));
+  CTD_CUDA(e, e->d_one.grow(CTD_ONE_BYTES));
+  uint8_t* one = e->d_one;
+  for (const CtdOneCopy& c : up)
+    if (c.host) CTD_CUDA(e, cudaMemcpyAsync(one + c.off, c.host, c.bytes, cudaMemcpyHostToDevice, e->stream));
+  a.state = (ctd_state*)one;
+  a.know6 = know ? (CtdKnow*)(one + CTD_ONE_KNOW_OFF) : nullptr;
+  a.used_cards = one + CTD_ONE_USED_OFF;
+  a.count = (uint32_t*)(one + CTD_ONE_COUNT_OFF);
+  a.winner = (int8_t*)(one + CTD_ONE_WINNER_OFF);
+  a.opts = (ctd_option*)(one + CTD_ONE_OPTS_OFF);
+  ctd_k_one<<<1, 32, 0, e->stream>>>(a);
+  e->launches++;
+  CTD_CUDA(e, cudaGetLastError());
+  for (const CtdOneCopy& c : down)
+    if (c.host) CTD_CUDA(e, cudaMemcpyAsync((void*)c.host, one + c.off, c.bytes, cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
   return CTD_OK;
-}
-static CtdOneArgs ctd_one_args(ctd_engine* e, int op, bool know) {
-  CtdOneArgs a;
-  memset(&a, 0, sizeof(a));
-  a.op = op; a.seed = e->seed;
-  a.state = (ctd_state*)e->d_one;
-  a.know6 = know ? (CtdKnow*)(e->d_one + CTD_ONE_KNOW_OFF) : nullptr;
-  a.used_cards = e->d_one + CTD_ONE_USED_OFF;
-  a.count = (uint32_t*)(e->d_one + CTD_ONE_COUNT_OFF);
-  a.winner = (int8_t*)(e->d_one + CTD_ONE_WINNER_OFF);
-  a.opts = (ctd_option*)(e->d_one + CTD_ONE_OPTS_OFF);
-  a.cap = CTD_ONE_OPTS;
-  return a;
 }
 
 ctd_status ctd_game_new(ctd_engine* e, uint64_t seed, uint64_t gid, int ruleset, ctd_state* state, void* know6, uint8_t* used_cards) {
   if (!e || !state || (ruleset < CTD_RULESET_PRESET || ruleset > CTD_RULESET_RANDOM)) return CTD_EARG;
-  CTD_CUDA(e, cudaSetDevice(e->device));
-  ctd_status s = ctd_one_buffer(e);
-  if (s != CTD_OK) return s;
-  CtdOneArgs a = ctd_one_args(e, 0, true);
-  a.seed = seed; a.gid = gid; a.ruleset = ruleset;
-  ctd_k_one<<<1, 32, 0, e->stream>>>(a);
-  e->launches++;
-  CTD_CUDA(e, cudaGetLastError());
-  CTD_CUDA(e, cudaMemcpyAsync(state, e->d_one, sizeof(ctd_state), cudaMemcpyDeviceToHost, e->stream));
-  if (know6) CTD_CUDA(e, cudaMemcpyAsync(know6, e->d_one + CTD_ONE_KNOW_OFF, CTD_ONE_KNOW6, cudaMemcpyDeviceToHost, e->stream));
-  if (used_cards) CTD_CUDA(e, cudaMemcpyAsync(used_cards, e->d_one + CTD_ONE_USED_OFF, 76, cudaMemcpyDeviceToHost, e->stream));
-  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
-  return CTD_OK;
+  CtdOneArgs a{};
+  a.op = 0; a.seed = seed; a.gid = gid; a.ruleset = ruleset;
+  return ctd_game_op(e, a, true, {},
+                     {{state, 0, sizeof(ctd_state)}, {know6, CTD_ONE_KNOW_OFF, CTD_ONE_KNOW6}, {used_cards, CTD_ONE_USED_OFF, 76}});
 }
 
 ctd_status ctd_game_options(ctd_engine* e, uint64_t seed, ctd_state* state, const void* know6, ctd_option* opts, uint32_t cap,
                             uint32_t* count) {
   if (!e || !state || !opts || !count) return CTD_EARG;
-  CTD_CUDA(e, cudaSetDevice(e->device));
-  ctd_status s = ctd_one_buffer(e);
+  CtdOneArgs a{};
+  a.op = 1; a.seed = seed;
+  a.cap = cap < CTD_ONE_OPTS ? cap : CTD_ONE_OPTS;   // a list the caller cannot take leaves the record untouched
+  ctd_status s = ctd_game_op(e, a, know6 != nullptr, {{state, 0, sizeof(ctd_state)}, {know6, CTD_ONE_KNOW_OFF, CTD_ONE_KNOW6}},
+                             {{count, CTD_ONE_COUNT_OFF, sizeof(uint32_t)}, {state, 0, sizeof(ctd_state)}});
   if (s != CTD_OK) return s;
-  CTD_CUDA(e, cudaMemcpyAsync(e->d_one, state, sizeof(ctd_state), cudaMemcpyHostToDevice, e->stream));
-  if (know6) CTD_CUDA(e, cudaMemcpyAsync(e->d_one + CTD_ONE_KNOW_OFF, know6, CTD_ONE_KNOW6, cudaMemcpyHostToDevice, e->stream));
-  CtdOneArgs a = ctd_one_args(e, 1, know6 != nullptr);
-  a.seed = seed;
-  if (cap < a.cap) a.cap = cap;   // a list the caller cannot take leaves the record untouched
-  ctd_k_one<<<1, 32, 0, e->stream>>>(a);
-  e->launches++;
-  CTD_CUDA(e, cudaGetLastError());
-  CTD_CUDA(e, cudaMemcpyAsync(count, a.count, sizeof(uint32_t), cudaMemcpyDeviceToHost, e->stream));
-  CTD_CUDA(e, cudaMemcpyAsync(state, e->d_one, sizeof(ctd_state), cudaMemcpyDeviceToHost, e->stream));
-  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
   uint32_t n = *count < cap ? *count : cap;
   if (n > CTD_ONE_OPTS) n = CTD_ONE_OPTS;
-  CTD_CUDA(e, cudaMemcpyAsync(opts, a.opts, (size_t)n * sizeof(ctd_option), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaMemcpyAsync(opts, e->d_one + CTD_ONE_OPTS_OFF, (size_t)n * sizeof(ctd_option), cudaMemcpyDeviceToHost, e->stream));
   CTD_CUDA(e, cudaStreamSynchronize(e->stream));
   return *count > cap || *count > CTD_ONE_OPTS ? CTD_ECAP : CTD_OK;
 }
 
 ctd_status ctd_game_step(ctd_engine* e, uint64_t seed, ctd_state* state, void* know6, ctd_option chosen, int8_t* winner) {
   if (!e || !state || !winner) return CTD_EARG;
-  CTD_CUDA(e, cudaSetDevice(e->device));
-  ctd_status s = ctd_one_buffer(e);
-  if (s != CTD_OK) return s;
-  CTD_CUDA(e, cudaMemcpyAsync(e->d_one, state, sizeof(ctd_state), cudaMemcpyHostToDevice, e->stream));
-  if (know6) CTD_CUDA(e, cudaMemcpyAsync(e->d_one + CTD_ONE_KNOW_OFF, know6, CTD_ONE_KNOW6, cudaMemcpyHostToDevice, e->stream));
-  CtdOneArgs a = ctd_one_args(e, 2, know6 != nullptr);
-  a.seed = seed; a.chosen = chosen;
-  ctd_k_one<<<1, 32, 0, e->stream>>>(a);
-  e->launches++;
-  CTD_CUDA(e, cudaGetLastError());
-  CTD_CUDA(e, cudaMemcpyAsync(state, e->d_one, sizeof(ctd_state), cudaMemcpyDeviceToHost, e->stream));
-  if (know6) CTD_CUDA(e, cudaMemcpyAsync(know6, e->d_one + CTD_ONE_KNOW_OFF, CTD_ONE_KNOW6, cudaMemcpyDeviceToHost, e->stream));
-  CTD_CUDA(e, cudaMemcpyAsync(winner, a.winner, 1, cudaMemcpyDeviceToHost, e->stream));
-  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
-  return CTD_OK;
+  CtdOneArgs a{};
+  a.op = 2; a.seed = seed; a.chosen = chosen;
+  return ctd_game_op(e, a, know6 != nullptr, {{state, 0, sizeof(ctd_state)}, {know6, CTD_ONE_KNOW_OFF, CTD_ONE_KNOW6}},
+                     {{state, 0, sizeof(ctd_state)}, {know6, CTD_ONE_KNOW_OFF, CTD_ONE_KNOW6}, {winner, CTD_ONE_WINNER_OFF, 1}});
 }
 
 ctd_status ctd_game_sample(ctd_engine* e, uint64_t seed, ctd_state* state, void* know6, const uint8_t* used_cards, int viewer,
                            int role_sample) {
   if (!e || !state || !know6 || !used_cards || viewer < 0 || viewer > 5) return CTD_EARG;
-  CTD_CUDA(e, cudaSetDevice(e->device));
-  ctd_status s = ctd_one_buffer(e);
-  if (s != CTD_OK) return s;
-  CTD_CUDA(e, cudaMemcpyAsync(e->d_one, state, sizeof(ctd_state), cudaMemcpyHostToDevice, e->stream));
-  CTD_CUDA(e, cudaMemcpyAsync(e->d_one + CTD_ONE_KNOW_OFF, know6, CTD_ONE_KNOW6, cudaMemcpyHostToDevice, e->stream));
-  CTD_CUDA(e, cudaMemcpyAsync(e->d_one + CTD_ONE_USED_OFF, used_cards, 76, cudaMemcpyHostToDevice, e->stream));
-  CtdOneArgs a = ctd_one_args(e, 3, true);
-  a.seed = seed; a.viewer = viewer; a.role_sample = role_sample;
-  ctd_k_one<<<1, 32, 0, e->stream>>>(a);
-  e->launches++;
-  CTD_CUDA(e, cudaGetLastError());
-  CTD_CUDA(e, cudaMemcpyAsync(state, e->d_one, sizeof(ctd_state), cudaMemcpyDeviceToHost, e->stream));
-  CTD_CUDA(e, cudaMemcpyAsync(know6, e->d_one + CTD_ONE_KNOW_OFF, CTD_ONE_KNOW6, cudaMemcpyDeviceToHost, e->stream));
-  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
-  return CTD_OK;
+  CtdOneArgs a{};
+  a.op = 3; a.seed = seed; a.viewer = viewer; a.role_sample = role_sample;
+  return ctd_game_op(e, a, true,
+                     {{state, 0, sizeof(ctd_state)}, {know6, CTD_ONE_KNOW_OFF, CTD_ONE_KNOW6}, {used_cards, CTD_ONE_USED_OFF, 76}},
+                     {{state, 0, sizeof(ctd_state)}, {know6, CTD_ONE_KNOW_OFF, CTD_ONE_KNOW6}});
 }
 
 // CFRNode.get_all_targets over the trees of the last ctd_mccfr / ctd_mccfr_pred call (they stay on the device).
@@ -1597,76 +1509,71 @@ ctd_status ctd_mccfr_targets(ctd_engine* e, uint32_t n_roots, uint64_t seed, uin
   if (s != CTD_OK) return s;
   // counts
   size_t cb = (size_t)n_roots * sizeof(uint32_t);
-  uint32_t* d_cnt = nullptr;
-  CTD_CUDA(e, cudaMalloc((void**)&d_cnt, 4 * cb));
+  CtdBuf<uint32_t> d_cnt;
+  CTD_CUDA(e, d_cnt.grow(4 * cb));
   CtdTargetArgs a;
   memset(&a, 0, sizeof(a));
   a.n_roots = n_roots; a.hdrs = e->d_hdrs; a.seed = seed;
   a.threshold = threshold; a.n_targets = d_cnt; a.n_options = d_cnt + n_roots;
   ctd_k_targets<<<ctd_blocks(n_roots), CTD_BLOCK, 0, e->stream>>>(a);
   e->launches++;
-  uint32_t* h_cnt = new (std::nothrow) uint32_t[4 * (size_t)n_roots];
-  if (!h_cnt) { cudaFree(d_cnt); return CTD_ENOMEM; }
-  cudaError_t c = cudaMemcpyAsync(h_cnt, d_cnt, 2 * cb, cudaMemcpyDeviceToHost, e->stream);
-  if (c == cudaSuccess) c = cudaStreamSynchronize(e->stream);
-  if (c != cudaSuccess) { delete[] h_cnt; cudaFree(d_cnt); return ctd_fail(e, c, "ctd_k_targets count"); }
+  std::unique_ptr<uint32_t[]> h_cnt(new (std::nothrow) uint32_t[4 * (size_t)n_roots]);
+  if (!h_cnt) return CTD_ENOMEM;
+  CTD_CUDA(e, cudaMemcpyAsync(h_cnt.get(), d_cnt, 2 * cb, cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
   uint32_t nrec = 0, nopt = 0;
   for (uint32_t t = 0; t < n_roots; ++t) {
     h_cnt[2 * n_roots + t] = nrec; h_cnt[3 * n_roots + t] = nopt;
     nrec += h_cnt[t]; nopt += h_cnt[n_roots + t];
   }
   const bool fill = features && meta && options && regrets;
-  if (fill && (nrec > *n_records || nopt > *n_option_slots)) { delete[] h_cnt; cudaFree(d_cnt); return CTD_ECAP; }
+  if (fill && (nrec > *n_records || nopt > *n_option_slots)) return CTD_ECAP;
   *n_records = nrec; *n_option_slots = nopt;
-  ctd_status rs = CTD_OK;
-  if (fill && nrec != 0) {
-    float* d_feat = nullptr; ctd_target_meta* d_meta = nullptr; ctd_option* d_opt = nullptr; double* d_reg = nullptr;
-    c = cudaMemcpyAsync(d_cnt + 2 * n_roots, h_cnt + 2 * n_roots, 2 * cb, cudaMemcpyHostToDevice, e->stream);
-    if (c == cudaSuccess) c = cudaMalloc((void**)&d_feat, (size_t)nrec * CTD_FEATURES_PAD * sizeof(float));
-    if (c == cudaSuccess) c = cudaMalloc((void**)&d_meta, (size_t)nrec * sizeof(ctd_target_meta));
-    if (c == cudaSuccess) c = cudaMalloc((void**)&d_opt, (size_t)(nopt + 1) * sizeof(ctd_option));
-    if (c == cudaSuccess) c = cudaMalloc((void**)&d_reg, (size_t)(nopt + 1) * sizeof(double));
-    if (c == cudaSuccess) {
-      a.fill = 1; a.rec_off = d_cnt + 2 * n_roots; a.opt_off = d_cnt + 3 * n_roots;
-      a.feat = d_feat; a.meta = d_meta; a.options = d_opt; a.regrets = d_reg;
-      ctd_k_targets<<<ctd_blocks(n_roots), CTD_BLOCK, 0, e->stream>>>(a);
-      e->launches++;
-      c = cudaGetLastError();
-    }
-    if (c == cudaSuccess) c = cudaMemcpyAsync(features, d_feat, (size_t)nrec * CTD_FEATURES_PAD * sizeof(float), cudaMemcpyDeviceToHost, e->stream);
-    if (c == cudaSuccess) c = cudaMemcpyAsync(meta, d_meta, (size_t)nrec * sizeof(ctd_target_meta), cudaMemcpyDeviceToHost, e->stream);
-    if (c == cudaSuccess) c = cudaMemcpyAsync(options, d_opt, (size_t)nopt * sizeof(ctd_option), cudaMemcpyDeviceToHost, e->stream);
-    if (c == cudaSuccess) c = cudaMemcpyAsync(regrets, d_reg, (size_t)nopt * sizeof(double), cudaMemcpyDeviceToHost, e->stream);
-    if (c == cudaSuccess) c = cudaStreamSynchronize(e->stream);
-    if (d_feat) cudaFree(d_feat);
-    if (d_meta) cudaFree(d_meta);
-    if (d_opt) cudaFree(d_opt);
-    if (d_reg) cudaFree(d_reg);
-    if (c != cudaSuccess) rs = ctd_fail(e, c, "ctd_k_targets fill");
-  }
-  delete[] h_cnt;
-  cudaFree(d_cnt);
-  return rs;
+  if (!fill || nrec == 0) return CTD_OK;
+  CtdBuf<float> d_feat;
+  CtdBuf<ctd_target_meta> d_meta;
+  CtdBuf<ctd_option> d_opt;
+  CtdBuf<double> d_reg;
+  CTD_CUDA(e, cudaMemcpyAsync(d_cnt + 2 * n_roots, h_cnt.get() + 2 * n_roots, 2 * cb, cudaMemcpyHostToDevice, e->stream));
+  CTD_CUDA(e, d_feat.grow((size_t)nrec * CTD_FEATURES_PAD * sizeof(float)));
+  CTD_CUDA(e, d_meta.grow((size_t)nrec * sizeof(ctd_target_meta)));
+  CTD_CUDA(e, d_opt.grow((size_t)(nopt + 1) * sizeof(ctd_option)));
+  CTD_CUDA(e, d_reg.grow((size_t)(nopt + 1) * sizeof(double)));
+  a.fill = 1; a.rec_off = d_cnt + 2 * n_roots; a.opt_off = d_cnt + 3 * n_roots;
+  a.feat = d_feat; a.meta = d_meta; a.options = d_opt; a.regrets = d_reg;
+  ctd_k_targets<<<ctd_blocks(n_roots), CTD_BLOCK, 0, e->stream>>>(a);
+  e->launches++;
+  CTD_CUDA(e, cudaGetLastError());
+  CTD_CUDA(e, cudaMemcpyAsync(features, d_feat, (size_t)nrec * CTD_FEATURES_PAD * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaMemcpyAsync(meta, d_meta, (size_t)nrec * sizeof(ctd_target_meta), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaMemcpyAsync(options, d_opt, (size_t)nopt * sizeof(ctd_option), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaMemcpyAsync(regrets, d_reg, (size_t)nopt * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  return CTD_OK;
 }
 
+// d_feat stands for the whole group, as d_knows does for the root buffers (ctd_root_buffers)
 static ctd_status ctd_pred_buffers(ctd_engine* e) {
   if (e->d_feat) return CTD_OK;
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_feat, (size_t)e->capacity * CTD_FEATURES_PAD * sizeof(float)));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_pred, (size_t)e->capacity * 8 * sizeof(float)));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_pending, (size_t)e->capacity));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_n_pending, 2 * sizeof(uint32_t)));
-  CTD_CUDA(e, cudaMallocHost((void**)&e->h_np, 4 * sizeof(uint32_t)));
-  CTD_CUDA(e, cudaMemsetAsync(e->d_feat, 0, (size_t)e->capacity * CTD_FEATURES_PAD * sizeof(float), e->stream));
-  CTD_CUDA(e, cudaMemsetAsync(e->d_pred, 0, (size_t)e->capacity * 8 * sizeof(float), e->stream));
-  CTD_CUDA(e, cudaMemsetAsync(e->d_pending, 0, (size_t)e->capacity, e->stream));
+  const size_t n = e->capacity;
+  CtdBuf<float> feat;
+  CTD_CUDA(e, feat.grow(n * CTD_FEATURES_PAD * sizeof(float)));
+  CTD_CUDA(e, e->d_pred.grow(n * 8 * sizeof(float)));
+  CTD_CUDA(e, e->d_pending.grow(n));
+  CTD_CUDA(e, e->d_n_pending.grow(2 * sizeof(uint32_t)));
+  CTD_CUDA(e, e->h_np.grow(4 * sizeof(uint32_t)));
+  CTD_CUDA(e, cudaMemsetAsync(feat, 0, n * CTD_FEATURES_PAD * sizeof(float), e->stream));
+  CTD_CUDA(e, cudaMemsetAsync(e->d_pred, 0, n * 8 * sizeof(float), e->stream));
+  CTD_CUDA(e, cudaMemsetAsync(e->d_pending, 0, n, e->stream));
   CTD_CUDA(e, cudaFuncSetAttribute(ctd_k_value_mlp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CTD_MLP_SMEM));
   CTD_CUDA(e, cudaFuncSetAttribute(ctd_k_linear_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CTD_TC_SMEM));
   CTD_CUDA(e, cudaFuncSetAttribute(ctd_k_linear_tc_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CTD_TC_SMEM));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_h1, (size_t)e->capacity * 512 * sizeof(float)));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_h2, (size_t)e->capacity * 256 * sizeof(float)));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_h3, (size_t)e->capacity * 128 * sizeof(float)));
-  CTD_CUDA(e, cudaMalloc((void**)&e->d_tc_err, sizeof(int)));
+  CTD_CUDA(e, e->d_h1.grow(n * 512 * sizeof(float)));
+  CTD_CUDA(e, e->d_h2.grow(n * 256 * sizeof(float)));
+  CTD_CUDA(e, e->d_h3.grow(n * 128 * sizeof(float)));
+  CTD_CUDA(e, e->d_tc_err.grow(sizeof(int)));   // ctd_train_begin may have made it already
   CTD_CUDA(e, cudaMemsetAsync(e->d_tc_err, 0, sizeof(int), e->stream));
+  e->d_feat = std::move(feat);
   return CTD_OK;
 }
 
@@ -1740,7 +1647,7 @@ ctd_status ctd_set_value_model(ctd_engine* e, const float* w1t, const float* b1,
   CTD_CUDA(e, cudaSetDevice(e->device));
   const size_t n1 = (size_t)CTD_FEATURES_PAD * 512, n2 = 512 * 256, n3 = 256 * 128, n4 = 128 * 6 + 2;
   const size_t total = n1 + 512 + n2 + 256 + n3 + 128 + n4 + 8;
-  if (!e->d_model) CTD_CUDA(e, cudaMalloc((void**)&e->d_model, total * sizeof(float)));
+  CTD_CUDA(e, e->d_model.grow(total * sizeof(float)));
   float* p = e->d_model;
   CtdValueModel& m = e->model;
   const float* src[8] = {w1t, b1, w2t, b2, w3t, b3, w4t, b4};
@@ -1754,18 +1661,16 @@ ctd_status ctd_set_value_model(ctd_engine* e, const float* w1t, const float* b1,
   }
   {  // tensor-core layout: [out][in] (the reference's own nn.Linear layout), BN already folded
     const size_t t1 = (size_t)512 * CTD_FEATURES_PAD, t2 = (size_t)256 * 512, t3 = (size_t)128 * 256;
-    float* h = new (std::nothrow) float[t1 + t2 + t3];
+    std::unique_ptr<float[]> h(new (std::nothrow) float[t1 + t2 + t3]);
     if (!h) return CTD_ENOMEM;
     for (int o = 0; o < 512; ++o) for (int k = 0; k < CTD_FEATURES_PAD; ++k) h[(size_t)o * CTD_FEATURES_PAD + k] = w1t[(size_t)k * 512 + o];
     for (int o = 0; o < 256; ++o) for (int k = 0; k < 512; ++k) h[t1 + (size_t)o * 512 + k] = w2t[(size_t)k * 256 + o];
     for (int o = 0; o < 128; ++o) for (int k = 0; k < 256; ++k) h[t1 + t2 + (size_t)o * 256 + k] = w3t[(size_t)k * 128 + o];
-    if (!e->d_model_tc) CTD_CUDA(e, cudaMalloc((void**)&e->d_model_tc, (t1 + t2 + t3) * sizeof(float)));
-    cudaError_t c = cudaMemcpy(e->d_model_tc, h, (t1 + t2 + t3) * sizeof(float), cudaMemcpyHostToDevice);
-    delete[] h;
-    if (c != cudaSuccess) return ctd_fail(e, c, "upload tc weights");
+    CTD_CUDA(e, e->d_model_tc.grow((t1 + t2 + t3) * sizeof(float)));
+    CTD_CUDA(e, cudaMemcpy(e->d_model_tc, h.get(), (t1 + t2 + t3) * sizeof(float), cudaMemcpyHostToDevice));
     e->tc_w1 = e->d_model_tc; e->tc_w2 = e->d_model_tc + t1; e->tc_w3 = e->d_model_tc + t1 + t2;
     // split the static weights into their TF32 terms once and describe them to the TMA engine
-    if (!e->d_wsplit) CTD_CUDA(e, cudaMalloc((void**)&e->d_wsplit, 3 * (t1 + t2 + t3) * sizeof(float)));
+    CTD_CUDA(e, e->d_wsplit.grow(3 * (t1 + t2 + t3) * sizeof(float)));
     float* sp[3] = {e->d_wsplit, e->d_wsplit + 3 * t1, e->d_wsplit + 3 * (t1 + t2)};
     const size_t cnt[3] = {t1, t2, t3};
     const float* src[3] = {e->tc_w1, e->tc_w2, e->tc_w3};
@@ -1824,12 +1729,10 @@ ctd_status ctd_mccfr_pred(ctd_engine* e, uint32_t n_roots, uint64_t seed, uint32
 }
 
 // ------------------------------------------------------------------------------------------ arena (ctd_arena.cuh)
-// what one ctd_arena call allocates, released on every way out
-struct CtdArenaRun {
-  void* mem[3] = {nullptr, nullptr, nullptr};
+// the phase-timing events of one ctd_arena call, destroyed on every way out
+struct CtdArenaEvents {
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
-  ~CtdArenaRun() {
-    for (void* p : mem) if (p) cudaFree(p);
+  ~CtdArenaEvents() {
     for (cudaEvent_t v : ev) if (v) cudaEventDestroy(v);
   }
 };
@@ -1870,21 +1773,24 @@ ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t fi
   CTD_CUDA(e, cudaSetDevice(e->device));
   ctd_status s = ctd_root_buffers(e);
   if (s != CTD_OK) return s;
-  CtdArenaRun run;
+  CtdBuf<CtdArenaGame> games;
+  CtdBuf<uint32_t> queue;
+  CtdBuf<int8_t> out;
+  CtdArenaEvents run;
   const size_t wb = ((size_t)n + 255) & ~(size_t)255, pb = ((size_t)n * 6 + 255) & ~(size_t)255, sb = ((size_t)n * 2 + 255) & ~(size_t)255,
                cb = (size_t)n * 4;
-  CTD_CUDA(e, cudaMalloc(&run.mem[0], (size_t)n * sizeof(CtdArenaGame)));
-  CTD_CUDA(e, cudaMalloc(&run.mem[1], 256 + (size_t)n_groups * n * sizeof(uint32_t)));
-  CTD_CUDA(e, cudaMalloc(&run.mem[2], wb + pb + sb + ((cb + 255) & ~(size_t)255) + sizeof(ctd_playout_stats)));
+  CTD_CUDA(e, games.grow((size_t)n * sizeof(CtdArenaGame)));
+  CTD_CUDA(e, queue.grow(256 + (size_t)n_groups * n * sizeof(uint32_t)));
+  CTD_CUDA(e, out.grow(wb + pb + sb + ((cb + 255) & ~(size_t)255) + sizeof(ctd_playout_stats)));
   for (cudaEvent_t& v : run.ev) CTD_CUDA(e, cudaEventCreate(&v));
-  int8_t* d_winner = (int8_t*)run.mem[2];
+  int8_t* d_winner = out;
   int8_t* d_points = d_winner + wb;
   uint16_t* d_steps = (uint16_t*)(d_winner + wb + pb);
   uint32_t* d_searches = (uint32_t*)(d_winner + wb + pb + sb);
   ctd_playout_stats* d_stats = (ctd_playout_stats*)(d_winner + wb + pb + sb + ((cb + 255) & ~(size_t)255));
   a.n = n; a.seed = seed; a.first_gid = first_gid; a.ruleset = ruleset; a.max_steps = max_steps;
-  a.games = (CtdArenaGame*)run.mem[0];
-  a.queued = (uint32_t*)run.mem[1];
+  a.games = games;
+  a.queued = queue;
   a.queue = a.queued + 64;
   e->slots_rs_n = 0;
   // Phase times.  The advance and the search phases end where the host waits anyway (the queue counts, the search's own
@@ -1965,38 +1871,12 @@ ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t fi
 
 
 // ------------------------------------------------------------------------------------------ value-network training
-// algorithms/train.py:13-86 (train_node_value_only) on the device; kernels in ctd_train.cuh
-struct CtdTrainer {
-  uint32_t n_train, n_val, batch, bp;   // bp: batch rounded up to a multiple of 32 (the K extent of the weight-gradient products)
-  uint32_t step;                        // optimiser steps taken (Adam bias correction, dropout mask counter)
-  float *feat_tr, *feat_va;
-  double *val_tr, *val_va;
-  uint32_t* perm;
-  float *P, *G, *M, *V;                 // CtdTrainLayout
-  float *rm1, *rv1, *rm2, *rv2;         // BatchNorm running statistics
-  float *X, *XT, *Z1, *H1, *H1T, *Z2, *H2, *H2T, *H3, *dY, *dZ3, *dZ3T, *dH2, *dZ2T, *dH1, *dZ1T, *W2T, *W3T, *inv1, *inv2, *zero;
-  double *T, *loss;
-};
-static void ctd_tr_free(CtdTrainer* t) {
-  void* ptrs[] = {t->feat_tr, t->feat_va, t->val_tr, t->val_va, t->perm, t->P, t->G, t->M, t->V, t->rm1, t->rv1, t->rm2, t->rv2, t->X, t->XT,
-                  t->Z1, t->H1, t->H1T, t->Z2, t->H2, t->H2T, t->H3, t->dY, t->dZ3, t->dZ3T, t->dH2, t->dZ2T, t->dH1, t->dZ1T, t->W2T, t->W3T,
-                  t->inv1, t->inv2, t->zero, t->T, t->loss};
-  for (void* p : ptrs) if (p) cudaFree(p);
-  delete t;
-}
 void ctd_train_end(ctd_engine* e) {
   if (!e || !e->trainer) return;
   cudaSetDevice(e->device);
   cudaStreamSynchronize(e->stream);
-  ctd_tr_free(e->trainer);
-  e->trainer = nullptr;
+  e->trainer.reset();
 }
-#define CTD_TR_ALLOC(ptr, count)                                                                          \
-  do {                                                                                                    \
-    cudaError_t _c = cudaMalloc((void**)&(ptr), (size_t)(count) * sizeof(*(ptr)));                        \
-    if (_c == cudaSuccess) _c = cudaMemsetAsync((ptr), 0, (size_t)(count) * sizeof(*(ptr)), e->stream);   \
-    if (_c != cudaSuccess) { ctd_tr_free(t); return ctd_fail(e, _c, "training buffers"); }              \
-  } while (0)
 
 ctd_status ctd_train_begin(ctd_engine* e, uint32_t n_train, const float* features, const double* node_values, uint32_t n_val,
                            const float* val_features, const double* val_node_values, uint32_t batch_size) {
@@ -2004,33 +1884,43 @@ ctd_status ctd_train_begin(ctd_engine* e, uint32_t n_train, const float* feature
     return CTD_EARG;
   CTD_CUDA(e, cudaSetDevice(e->device));
   ctd_train_end(e);
-  CtdTrainer* t = new (std::nothrow) CtdTrainer();
+  std::unique_ptr<CtdTrainer> t(new (std::nothrow) CtdTrainer());
   if (!t) return CTD_ENOMEM;
-  memset(t, 0, sizeof(*t));
   t->n_train = n_train; t->n_val = n_val; t->batch = batch_size; t->bp = (batch_size + 31) & ~31u;
   const size_t bp = t->bp;
-  CTD_TR_ALLOC(t->feat_tr, (size_t)n_train * 418); CTD_TR_ALLOC(t->val_tr, (size_t)n_train * 6);
-  CTD_TR_ALLOC(t->feat_va, (size_t)(n_val ? n_val : 1) * 418); CTD_TR_ALLOC(t->val_va, (size_t)(n_val ? n_val : 1) * 6);
-  CTD_TR_ALLOC(t->perm, n_train);
-  CTD_TR_ALLOC(t->P, CtdTrainLayout::total); CTD_TR_ALLOC(t->G, CtdTrainLayout::total); CTD_TR_ALLOC(t->M, CtdTrainLayout::total); CTD_TR_ALLOC(t->V, CtdTrainLayout::total);
-  CTD_TR_ALLOC(t->rm1, CTD_TR_H1); CTD_TR_ALLOC(t->rv1, CTD_TR_H1); CTD_TR_ALLOC(t->rm2, CTD_TR_H2); CTD_TR_ALLOC(t->rv2, CTD_TR_H2);
-  CTD_TR_ALLOC(t->X, bp * CTD_TR_IN); CTD_TR_ALLOC(t->XT, bp * CTD_TR_IN);
-  CTD_TR_ALLOC(t->Z1, bp * CTD_TR_H1); CTD_TR_ALLOC(t->H1, bp * CTD_TR_H1); CTD_TR_ALLOC(t->H1T, bp * CTD_TR_H1);
-  CTD_TR_ALLOC(t->Z2, bp * CTD_TR_H2); CTD_TR_ALLOC(t->H2, bp * CTD_TR_H2); CTD_TR_ALLOC(t->H2T, bp * CTD_TR_H2);
-  CTD_TR_ALLOC(t->H3, bp * CTD_TR_H3); CTD_TR_ALLOC(t->dY, bp * 8); CTD_TR_ALLOC(t->dZ3, bp * CTD_TR_H3); CTD_TR_ALLOC(t->dZ3T, bp * CTD_TR_H3);
-  CTD_TR_ALLOC(t->dH2, bp * CTD_TR_H2); CTD_TR_ALLOC(t->dZ2T, bp * CTD_TR_H2); CTD_TR_ALLOC(t->dH1, bp * CTD_TR_H1); CTD_TR_ALLOC(t->dZ1T, bp * CTD_TR_H1);
-  CTD_TR_ALLOC(t->W2T, (size_t)CTD_TR_H1 * CTD_TR_H2); CTD_TR_ALLOC(t->W3T, (size_t)CTD_TR_H2 * CTD_TR_H3);
-  CTD_TR_ALLOC(t->inv1, CTD_TR_H1); CTD_TR_ALLOC(t->inv2, CTD_TR_H2); CTD_TR_ALLOC(t->zero, 512);
-  CTD_TR_ALLOC(t->T, bp * 6); CTD_TR_ALLOC(t->loss, 2);
-  cudaError_t c = cudaMemcpyAsync(t->feat_tr, features, (size_t)n_train * 418 * sizeof(float), cudaMemcpyHostToDevice, e->stream);
-  if (c == cudaSuccess) c = cudaMemcpyAsync(t->val_tr, node_values, (size_t)n_train * 6 * sizeof(double), cudaMemcpyHostToDevice, e->stream);
-  if (c == cudaSuccess && n_val) c = cudaMemcpyAsync(t->feat_va, val_features, (size_t)n_val * 418 * sizeof(float), cudaMemcpyHostToDevice, e->stream);
-  if (c == cudaSuccess && n_val) c = cudaMemcpyAsync(t->val_va, val_node_values, (size_t)n_val * 6 * sizeof(double), cudaMemcpyHostToDevice, e->stream);
-  if (c == cudaSuccess) c = cudaFuncSetAttribute(ctd_k_linear_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CTD_TC_SMEM);
-  if (c == cudaSuccess && !e->d_tc_err) { c = cudaMalloc((void**)&e->d_tc_err, sizeof(int)); if (c == cudaSuccess) c = cudaMemsetAsync(e->d_tc_err, 0, sizeof(int), e->stream); }
-  if (c == cudaSuccess) c = cudaStreamSynchronize(e->stream);
-  if (c != cudaSuccess) { ctd_tr_free(t); return ctd_fail(e, c, "training data upload"); }
-  e->trainer = t;
+  cudaError_t c = cudaSuccess;
+  auto zeroed = [&](auto& buf, size_t count) {   // allocate and clear, until the first failure
+    const size_t bytes = count * sizeof(*buf.get());
+    if (c == cudaSuccess) c = buf.grow(bytes);
+    if (c == cudaSuccess) c = cudaMemsetAsync(buf, 0, bytes, e->stream);
+  };
+  zeroed(t->feat_tr, (size_t)n_train * 418); zeroed(t->val_tr, (size_t)n_train * 6);
+  zeroed(t->feat_va, (size_t)(n_val ? n_val : 1) * 418); zeroed(t->val_va, (size_t)(n_val ? n_val : 1) * 6);
+  zeroed(t->perm, n_train);
+  zeroed(t->P, CtdTrainLayout::total); zeroed(t->G, CtdTrainLayout::total); zeroed(t->M, CtdTrainLayout::total); zeroed(t->V, CtdTrainLayout::total);
+  zeroed(t->rm1, CTD_TR_H1); zeroed(t->rv1, CTD_TR_H1); zeroed(t->rm2, CTD_TR_H2); zeroed(t->rv2, CTD_TR_H2);
+  zeroed(t->X, bp * CTD_TR_IN); zeroed(t->XT, bp * CTD_TR_IN);
+  zeroed(t->Z1, bp * CTD_TR_H1); zeroed(t->H1, bp * CTD_TR_H1); zeroed(t->H1T, bp * CTD_TR_H1);
+  zeroed(t->Z2, bp * CTD_TR_H2); zeroed(t->H2, bp * CTD_TR_H2); zeroed(t->H2T, bp * CTD_TR_H2);
+  zeroed(t->H3, bp * CTD_TR_H3); zeroed(t->dY, bp * 8); zeroed(t->dZ3, bp * CTD_TR_H3); zeroed(t->dZ3T, bp * CTD_TR_H3);
+  zeroed(t->dH2, bp * CTD_TR_H2); zeroed(t->dZ2T, bp * CTD_TR_H2); zeroed(t->dH1, bp * CTD_TR_H1); zeroed(t->dZ1T, bp * CTD_TR_H1);
+  zeroed(t->W2T, (size_t)CTD_TR_H1 * CTD_TR_H2); zeroed(t->W3T, (size_t)CTD_TR_H2 * CTD_TR_H3);
+  zeroed(t->inv1, CTD_TR_H1); zeroed(t->inv2, CTD_TR_H2); zeroed(t->zero, 512);
+  zeroed(t->T, bp * 6); zeroed(t->loss, 2);
+  if (c != cudaSuccess) return ctd_fail(e, c, "training buffers");
+  CTD_CUDA(e, cudaMemcpyAsync(t->feat_tr, features, (size_t)n_train * 418 * sizeof(float), cudaMemcpyHostToDevice, e->stream));
+  CTD_CUDA(e, cudaMemcpyAsync(t->val_tr, node_values, (size_t)n_train * 6 * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+  if (n_val) {
+    CTD_CUDA(e, cudaMemcpyAsync(t->feat_va, val_features, (size_t)n_val * 418 * sizeof(float), cudaMemcpyHostToDevice, e->stream));
+    CTD_CUDA(e, cudaMemcpyAsync(t->val_va, val_node_values, (size_t)n_val * 6 * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+  }
+  CTD_CUDA(e, cudaFuncSetAttribute(ctd_k_linear_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CTD_TC_SMEM));
+  if (!e->d_tc_err) {
+    CTD_CUDA(e, e->d_tc_err.grow(sizeof(int)));
+    CTD_CUDA(e, cudaMemsetAsync(e->d_tc_err, 0, sizeof(int), e->stream));
+  }
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  e->trainer = std::move(t);
   return CTD_OK;
 }
 
@@ -2048,7 +1938,7 @@ static float* ctd_tr_slot(CtdTrainer* t, int i) {
 ctd_status ctd_train_set_state(ctd_engine* e, const float* const* tensors16) {
   if (!e || !e->trainer || !tensors16) return CTD_EARG;
   CTD_CUDA(e, cudaSetDevice(e->device));
-  CtdTrainer* t = e->trainer;
+  CtdTrainer* t = e->trainer.get();
   CTD_CUDA(e, cudaMemsetAsync(t->P, 0, CtdTrainLayout::total * sizeof(float), e->stream));
   CTD_CUDA(e, cudaMemsetAsync(t->M, 0, CtdTrainLayout::total * sizeof(float), e->stream));
   CTD_CUDA(e, cudaMemsetAsync(t->V, 0, CtdTrainLayout::total * sizeof(float), e->stream));
@@ -2066,7 +1956,7 @@ ctd_status ctd_train_set_state(ctd_engine* e, const float* const* tensors16) {
 ctd_status ctd_train_get_state(ctd_engine* e, float* const* tensors16) {
   if (!e || !e->trainer || !tensors16) return CTD_EARG;
   CTD_CUDA(e, cudaSetDevice(e->device));
-  CtdTrainer* t = e->trainer;
+  CtdTrainer* t = e->trainer.get();
   for (int i = 0; i < 16; ++i) {
     if (!tensors16[i]) return CTD_EARG;
     if (i == 0)
@@ -2082,7 +1972,7 @@ ctd_status ctd_train_get_state(ctd_engine* e, float* const* tensors16) {
 ctd_status ctd_train_get_grads(ctd_engine* e, float* const* tensors16) {
   if (!e || !e->trainer || !tensors16) return CTD_EARG;
   CTD_CUDA(e, cudaSetDevice(e->device));
-  CtdTrainer* t = e->trainer;
+  CtdTrainer* t = e->trainer.get();
   for (int i = 0; i < 16; ++i) {
     if (!tensors16[i]) return CTD_EARG;
     const bool stat = i == 4 || i == 5 || i == 10 || i == 11;
@@ -2123,7 +2013,7 @@ static void ctd_tr_forward(ctd_engine* e, CtdTrainer* t, uint32_t B, int train, 
 ctd_status ctd_train_epoch(ctd_engine* e, uint64_t seed, float lr, const uint32_t* perm, double* train_loss, double* eval_loss) {
   if (!e || !e->trainer) return CTD_EARG;
   CTD_CUDA(e, cudaSetDevice(e->device));
-  CtdTrainer* t = e->trainer;
+  CtdTrainer* t = e->trainer.get();
   typedef CtdTrainLayout L;
   const uint32_t bp = t->bp;
   if (perm) CTD_CUDA(e, cudaMemcpyAsync(t->perm, perm, (size_t)t->n_train * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
@@ -2131,7 +2021,7 @@ ctd_status ctd_train_epoch(ctd_engine* e, uint64_t seed, float lr, const uint32_
   uint32_t nb = 0;
   for (uint32_t first = 0; first < t->n_train; first += t->batch, ++nb) {
     const uint32_t B = t->n_train - first < t->batch ? t->n_train - first : t->batch;
-    ctd_k_tr_gather<<<bp, 128, 0, e->stream>>>(t->feat_tr, t->val_tr, perm ? t->perm : nullptr, first, B, bp, t->X, t->T);
+    ctd_k_tr_gather<<<bp, 128, 0, e->stream>>>(t->feat_tr, t->val_tr, perm ? t->perm.get() : nullptr, first, B, bp, t->X, t->T);
     ctd_tr_forward(e, t, B, 1, seed);
     CTD_CUDA(e, cudaMemsetAsync(t->loss, 0, sizeof(double), e->stream));
     CTD_CUDA(e, cudaMemsetAsync(t->G, 0, L::total * sizeof(float), e->stream));
