@@ -59,6 +59,7 @@ SIGNATURES = {
     "ctd_game_step": (_i, [c_void, _u64, c_void, c_void, _u64, ctypes.POINTER(ctypes.c_int8)]),
     "ctd_game_sample": (_i, [c_void, _u64, c_void, c_void, c_void, _i, _i]),
     "ctd_set_value_model": (_i, [c_void] + [c_void] * 8),
+    "ctd_set_value_model_slot": (_i, [c_void, _i] + [c_void] * 8),
     "ctd_set_value_backend": (_i, [c_void, _i]),
     "ctd_value_eval": (_i, [c_void, _u32, c_void, ctypes.c_float, c_void]),
     "ctd_encode": (_i, [c_void, _u32, _i, c_void]),

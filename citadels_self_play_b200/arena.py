@@ -11,21 +11,27 @@ seats 2-5 uniformly at random; forced moves (one legal option) are played withou
                                           (CFRNode.action_choice(live=True), algorithms/deep_mccfr.py:67-75, with the
                                           role-preference quirk of game/game.py:312-317) is taken from the result records.
   play_arena(n_games, seats, model)       the experiment with any player on any seat (random_seat(), pure(it), deep(it,
-                                          depth, weight)), every game resident on the device from deal to end (ctd_arena): the
-                                          host only loops over decision rounds.  Random seats draw from Philox stream 4
-                                          keyed by the game's step count, so results do not depend on batch sizes.
+                                          depth, weight, model=slot)), every game resident on the device from deal to end
+                                          (ctd_arena): the host only loops over decision rounds.  Random seats draw from
+                                          Philox stream 4 keyed by the game's step count, so results do not depend on batch
+                                          sizes.  models=[...] loads one value model per slot, so deep seats can differ in model.
+  head_to_head(n_games, model_a, model_b) two value models against each other: every deal is played twice, with a seat
+                                          pattern and with A and B swapped, and the pairs are counted and sign-tested.
 
 Every search of game g at decision number t runs on the Philox stream keyed (seed, g | t << 40), so successive decisions of
 one game do not reuse draws.  There is no CPU path: games live in 256-byte records, every transition and every search
 runs on the device.
 """
+import math
 import random
 
 import numpy as np
 
 from .engine import Engine, EngineError, DEFAULT_SEED, RULESET_PRESET
-from .layout import KNOW_BYTES, SEAT_RANDOM, SEAT_PURE, SEAT_DEEP
+from .layout import KNOW_BYTES, SEAT_RANDOM, SEAT_PURE, SEAT_DEEP, MAX_VALUE_MODELS, SEAT_MODEL_SHIFT
 from . import facade as F
+
+Z99 = 2.5758293035489004
 
 
 def play_games(sim_number, model=None, engine=None, seed=DEFAULT_SEED, first_gid=0, deep_iterations=200,
@@ -136,9 +142,18 @@ def pure(iterations):
     return (SEAT_PURE, int(iterations), 0, 0.0)
 
 
-def deep(iterations, max_depth=10, weight=5.0):
-    """A seat on run_mccfr(game, model, max_iterations=iterations): cfr_pred(iterations, max_depth) with the engine's value model."""
-    return (SEAT_DEEP, int(iterations), int(max_depth), float(weight))
+def deep(iterations, max_depth=10, weight=5.0, model=0):
+    """A seat on run_mccfr(game, model, max_iterations=iterations): cfr_pred(iterations, max_depth) with the value model in the
+    engine's slot `model` (CTD_SEAT_DEEP_MODEL)."""
+    return (SEAT_DEEP | (int(model) << SEAT_MODEL_SHIFT), int(iterations), int(max_depth), float(weight))
+
+
+def _seat_kind(kind):
+    return int(kind) & 0xFF
+
+
+def _seat_model(kind):
+    return (int(kind) >> SEAT_MODEL_SHIFT) & 0xFF
 
 
 def default_seats():
@@ -155,19 +170,29 @@ def rank_block(n_games, rank, world):
 
 
 def play_arena(n_games, seats=None, model=None, engine=None, seed=DEFAULT_SEED, first_gid=0, ruleset=RULESET_PRESET,
-               max_steps=4096, group=None):
+               max_steps=4096, group=None, models=None):
     """compare_to_random.play_games with a player per seat, every game on the device (Engine.arena).  Under torch.distributed
     each rank plays its own block of game ids (sharding.first_gid over rank_block's split) and the statistics are summed.
     Without `engine` the games run on torch's current CUDA device (under torchrun: the rank's own GPU after
     torch.cuda.set_device(LOCAL_RANK)); the statistics are reduced on the engine's device.
+    models: value models loaded into slots 0 .. len(models) - 1, for the seats deep(..., model=slot); `model` is short for
+    models=[model].  Without `engine` every deep seat's slot must be among them.
     -> dict(winners[6] and stats over all ranks; this rank's local_stats, first_gid of its games, their per-game arrays
     winner / points / steps / searches and its phase_ms)."""
     import torch
     import torch.distributed as dist
     from . import sharding
     seats = default_seats() if seats is None else list(seats)
-    if any(s[0] == SEAT_DEEP for s in seats) and model is None and engine is None:
-        raise ValueError("a deep seat needs a value model")
+    if model is not None:
+        if models is not None:
+            raise ValueError("pass model= or models=, not both")
+        models = [model]
+    models = [] if models is None else list(models)
+    if len(models) > MAX_VALUE_MODELS:
+        raise ValueError("an engine holds %d value models, got %d" % (MAX_VALUE_MODELS, len(models)))
+    missing = sorted({_seat_model(s[0]) for s in seats if _seat_kind(s[0]) == SEAT_DEEP} - set(range(len(models))))
+    if missing and engine is None:
+        raise ValueError("deep seats on value-model slots %s, but models= fills slots [0, %d)" % (missing, len(models)))
     dist_on = dist.is_available() and dist.is_initialized()
     rank = dist.get_rank(group) if dist_on else 0
     world = dist.get_world_size(group) if dist_on else 1
@@ -176,8 +201,8 @@ def play_arena(n_games, seats=None, model=None, engine=None, seed=DEFAULT_SEED, 
     eng = engine or Engine(capacity=max(1, min(count, 8192)), 
                             device=torch.cuda.current_device() if torch.cuda.is_available() else 0)
     try:
-        if model is not None:
-            eng.set_value_model(model)
+        for slot, m in enumerate(models):
+            eng.set_value_model(m, slot=slot)
         out = eng.arena(count, seats, seed=seed, first_gid=first_gid + first, ruleset=ruleset, max_steps=max_steps)
     finally:
         if own:
@@ -188,3 +213,82 @@ def play_arena(n_games, seats=None, model=None, engine=None, seed=DEFAULT_SEED, 
     stats["max_steps"] = int(sharding.reduce_max([local["max_steps"]], dev, group=group)[0])
     out.update(winners=list(stats["wins"]), stats=stats, local_stats=local, first_gid=first_gid + first)
     return out
+
+
+def wilson(k, n, z=Z99):
+    """Wilson score interval of k successes in n trials (default 99 %)."""
+    if n == 0:
+        return [0.0, 1.0]
+    p = k / n
+    c = (p + z * z / (2 * n)) / (1 + z * z / n)
+    h = z * math.sqrt(p * (1 - p) / n + z * z / (4 * n * n)) / (1 + z * z / n)
+    return [max(0.0, c - h), min(1.0, c + h)]
+
+
+PAIR_KEYS = ("a_both", "b_both", "split", "random", "error")
+
+
+def swap_pattern(pattern):
+    """The seat pattern with A and B exchanged (R, a random seat, stays)."""
+    return pattern.translate(str.maketrans("AB", "BA"))
+
+
+def pair_counts(pattern, winner_ab, winner_ba):
+    """Game i was played twice on the same deal: with seat pattern `pattern` (winning seat winner_ab[i]) and with A and B swapped
+    (winner_ba[i]); -1 is an errored game.  -> dict of pair counts: a_both (A's seats won both games), b_both, split (A won one,
+    B the other), random (a random seat won at least one, neither errored) and error (either game errored)."""
+    w = [np.asarray(x, dtype=np.int64) for x in (winner_ab, winner_ba)]
+    if w[0].shape != w[1].shape:
+        raise ValueError("the two passes have %d and %d games" % (w[0].size, w[1].size))
+    # the side of each winning seat, E for an error (index 6)
+    side = [np.array(list(p) + ["E"])[np.where(x < 0, 6, x)] for p, x in zip((pattern, swap_pattern(pattern)), w)]
+    err = (side[0] == "E") | (side[1] == "E")
+    a_both = ~err & (side[0] == "A") & (side[1] == "A")
+    b_both = ~err & (side[0] == "B") & (side[1] == "B")
+    rnd = ~err & ((side[0] == "R") | (side[1] == "R"))
+    split = ~err & ~rnd & ~a_both & ~b_both
+    return dict(zip(PAIR_KEYS, (int(x.sum()) for x in (a_both, b_both, split, rnd, err))))
+
+
+def head_to_head(n_games, model_a, model_b, player=deep(200, 10, 5.0), pattern="ABABAB", engine=None, seed=DEFAULT_SEED,
+                 first_gid=0, ruleset=RULESET_PRESET, max_steps=4096, group=None):
+    """Value model A against value model B: games (seed, first_gid + i) for i < n_games, each played twice through play_arena
+    (models=[model_a, model_b]), once with `pattern` (seat s: A, B or R for a random seat) and once with A and B swapped, so
+    that the luck of the deal and of the seats cancels.  A's and B's seats play `player` (a deep() seat) on their own model.
+    Under torch.distributed both passes split the games over the ranks alike, each rank pairs its own games and the counts are
+    summed.
+    -> dict(games (pairs), errors (games), a / b: wins, share of the decided games and its Wilson 99 % interval, random_wins,
+    seats and seat_wins of each pass, pairs (pair_counts over all ranks), sign_test (two-sided binomial test of a_both against b_both),
+    passes (the two play_arena results))."""
+    import torch
+    import torch.distributed as dist
+    from scipy.stats import binomtest
+    from . import sharding
+    pattern = str(pattern)
+    if len(pattern) != 6 or set(pattern) - set("ABR") or "A" not in pattern or "B" not in pattern:
+        raise ValueError("pattern: six seats of A, B or R with at least one A and one B, got %r" % (pattern,))
+    kind, its, depth, weight = player
+    if _seat_kind(kind) != SEAT_DEEP:
+        raise ValueError("player must be a deep() seat")
+    swapped = swap_pattern(pattern)
+
+    def seats(p):
+        return [deep(its, depth, weight, model="AB".index(c)) if c in "AB" else random_seat() for c in p]
+    pass_seats = [seats(pattern), seats(swapped)]
+    passes = [play_arena(n_games, s, engine=engine, seed=seed, first_gid=first_gid, ruleset=ruleset, max_steps=max_steps, group=group,
+                         models=[model_a, model_b]) for s in pass_seats]
+    dist_on = dist.is_available() and dist.is_initialized()
+    dev = "cpu"
+    if dist_on and dist.get_backend(group) == "nccl":
+        dev = "cuda:%d" % (engine.device if engine is not None else torch.cuda.current_device())
+    local = pair_counts(pattern, passes[0]["winner"], passes[1]["winner"])
+    pairs = dict(zip(PAIR_KEYS, sharding.reduce_sum([local[k] for k in PAIR_KEYS], dev, group=group)))
+    st = [r["stats"] for r in passes]
+    wins = {c: sum(s["wins"][i] for s, p in zip(st, (pattern, swapped)) for i in range(6) if p[i] == c) for c in "ABR"}
+    decided = sum(s["games"] - s["errors"] for s in st)
+    n_sign = pairs["a_both"] + pairs["b_both"]
+    p_value = float(binomtest(pairs["a_both"], n_sign, 0.5, alternative="two-sided").pvalue) if n_sign else 1.0
+    side = {c: dict(wins=wins[c], share=wins[c] / decided if decided else 0.0, wilson99=wilson(wins[c], decided)) for c in "AB"}
+    return dict(pattern=pattern, swapped=swapped, games=st[0]["games"], errors=st[0]["errors"] + st[1]["errors"], a=side["A"],
+                b=side["B"], random_wins=wins["R"], seats=[[list(x) for x in s] for s in pass_seats], seat_wins=[s["wins"] for s in st],
+                pairs=pairs, sign_test=dict(a_both=pairs["a_both"], b_both=pairs["b_both"], p_value=p_value), passes=passes)

@@ -583,6 +583,20 @@ struct CtdTrainer {
   CtdBuf<double> T, loss;
 };
 
+// one value model as the engine holds it (ctd_set_value_model_slot): the fused search and the fp32 kernel read the BN-folded
+// [in][out] weights, the tcgen05 kernels their [out][in] copy or, by TMA, its split TF32 terms
+struct CtdValueSlot {
+  bool ready;              // the last load completed
+  CtdBuf<float> d_model;   // BN folded, transposed
+  CtdValueModel model;
+  CtdBuf<float> d_model_tc;
+  const float *tc_w1, *tc_w2, *tc_w3;
+  // the weights pre-split into their three TF32 terms, [3][N][K] per layer, and their tensor maps (TMA loads of the B operand)
+  CtdBuf<float> d_wsplit;
+  CUtensorMap tmap[3];
+  bool tmap_ok;
+};
+
 #define CTD_MAX_ARENAS 6
 struct ctd_engine {
   int device;
@@ -623,23 +637,16 @@ struct ctd_engine {
   CtdBuf<ctd_mccfr_result> d_results;
   CtdBuf<uint32_t> d_list;                   // retry lists
   CtdBuf<uint64_t> d_opts_scratch;
-  // value model (BN folded, transposed) and deep-MCCFR batch buffers
-  CtdBuf<float> d_model;
-  CtdValueModel model;
+  // value models (slot 0: ctd_set_value_model) and deep-MCCFR batch buffers
+  CtdValueSlot vm[CTD_MAX_VALUE_MODELS];
   CtdBuf<float> d_feat;
   CtdBuf<float> d_pred;
   CtdBuf<uint8_t> d_pending;
   CtdBuf<uint32_t> d_n_pending;
   CtdBuf<uint32_t> d_n_epool;   // [1] trees that found their arena exhausted in the passes since it was last cleared
-  // tensor-core path of the value model: weights as [out][in], activations between layers, error flag
-  CtdBuf<float> d_model_tc;
-  const float *tc_w1, *tc_w2, *tc_w3;
+  // tensor-core path of the value model: activations between layers, error flag
   CtdBuf<float> d_h1, d_h2, d_h3;
   CtdBuf<int> d_tc_err;
-  // the weights pre-split into their three TF32 terms, [3][N][K] per layer, and their tensor maps (TMA loads of the B operand)
-  CtdBuf<float> d_wsplit;
-  CUtensorMap tmap[3];
-  bool tmap_ok;
   int value_backend;  // batched evaluations: 0 = fp32 CUDA cores (ctd_k_value_mlp), 1 = tcgen05 split-TF32 (ctd_k_linear_tc)
   int fused;          // deep MCCFR: 1 = one launch, every warp evaluates its own leaves (ctd_value_inline); 0 = waves + batched evaluation
   CtdBuf<uint8_t, true> h_pinned;        // pinned host staging for result copies
@@ -1105,8 +1112,10 @@ struct CtdSearch {
   uint32_t max_depth;
   float weight;
   bool resume;      // pure MCCFR only: continue the trees of the previous call for `iterations` more
+  int model;        // deep MCCFR: the value-model slot that evaluates the leaves
 };
-static ctd_status ctd_value_forward(ctd_engine* e, uint32_t n, const uint8_t* pending, float weight, uint32_t row0, cudaStream_t st);
+static ctd_status ctd_value_forward(ctd_engine* e, const CtdValueSlot& vm, uint32_t n, const uint8_t* pending, float weight, uint32_t row0,
+                                    cudaStream_t st);
 static ctd_status ctd_pred_buffers(ctd_engine* e);
 
 // one pass of pure MCCFR over `n` trees (d_list: their root indices, or null for roots [0, n)) allocating from arena `ai`
@@ -1148,7 +1157,8 @@ static ctd_status ctd_deep_pass(ctd_engine* e, const CtdSearch& sp, const uint32
   if (e->fused) {
     // fused: one launch; every warp walks its tree to the end and evaluates the leaves it meets itself (ctd_value_inline)
     p.fused = 1; p.budget = 0xFFFFFFFFu; p.first = 1;
-    p.net = CtdValueNet{e->model.w1t, e->model.b1, e->model.w2t, e->model.b2, e->model.w3t, e->model.b3, e->model.w4t, e->model.b4, sp.weight};
+    const CtdValueModel& m = e->vm[sp.model].model;
+    p.net = CtdValueNet{m.w1t, m.b1, m.w2t, m.b2, m.w3t, m.b3, m.w4t, m.b4, sp.weight};
     const int grid = k.grid(n);
     CTD_CUDA(e, e->d_opts_scratch.grow((size_t)grid * CTD_WARPS_PER_BLOCK * CTD_MCCFR_OPT_CAP * sizeof(uint64_t)));
     a.tree_list = d_list; a.first_root = 0; a.n_roots = n; a.counter = e->d_counter; a.opts_scratch = e->d_opts_scratch;
@@ -1219,7 +1229,7 @@ static ctd_status ctd_deep_pass(ctd_engine* e, const CtdSearch& sp, const uint32
         // the feature / pending rows are indexed by root: with a retry list the model runs over every row of the call and the
         // pending mask picks the waiting ones
         const uint32_t row0 = d_list ? 0 : g_first[g], rows = d_list ? sp.n_roots : g_n[g];
-        s = ctd_value_forward(e, rows, e->d_pending + row0, sp.weight, row0, g_stream[g]);
+        s = ctd_value_forward(e, e->vm[sp.model], rows, e->d_pending + row0, sp.weight, row0, g_stream[g]);
         if (s != CTD_OK) return s;
       }
       s = launch_wave(g);
@@ -1577,35 +1587,36 @@ static ctd_status ctd_pred_buffers(ctd_engine* e) {
   return CTD_OK;
 }
 
-// the value model on rows [0,n) of d_feat -> d_pred (rows with pending == 0 may be skipped)
-// rows [row0, row0 + n) of the feature matrix (`pending` is the mask of those rows), on `st`
-static ctd_status ctd_value_forward(ctd_engine* e, uint32_t n, const uint8_t* pending, float weight, uint32_t row0,
+// the value model `vm` on rows [row0, row0 + n) of d_feat -> d_pred (`pending` is the mask of those rows; rows with pending == 0
+// may be skipped), on `st`
+static ctd_status ctd_value_forward(ctd_engine* e, const CtdValueSlot& vm, uint32_t n, const uint8_t* pending, float weight, uint32_t row0,
                                     cudaStream_t st) {
   if (st == nullptr) st = e->stream;
   const float* feat = e->d_feat + (size_t)row0 * CTD_FEATURES_PAD;
   float* pred = e->d_pred + (size_t)row0 * 8;
+  const CtdValueModel& m = vm.model;
   if (e->value_backend == 0) {
-    ctd_k_value_mlp<<<(n + CTD_MLP_ROWS - 1) / CTD_MLP_ROWS, 256, CTD_MLP_SMEM, st>>>(feat, pending, n, e->model, pred, weight);
+    ctd_k_value_mlp<<<(n + CTD_MLP_ROWS - 1) / CTD_MLP_ROWS, 256, CTD_MLP_SMEM, st>>>(feat, pending, n, m, pred, weight);
     e->launches++;
     CTD_CUDA(e, cudaGetLastError());
     return CTD_OK;
   }
   float *h1 = e->d_h1 + (size_t)row0 * 512, *h2 = e->d_h2 + (size_t)row0 * 256, *h3 = e->d_h3 + (size_t)row0 * 128;
   const int M = (int)n, gm = (M + CTD_TC_BM - 1) / CTD_TC_BM;
-  if (e->tmap_ok) {   // weight operand by TMA from the pre-split terms
-    ctd_k_linear_tc_tma<<<dim3(gm, 512 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(feat, CTD_FEATURES_PAD, e->tmap[0], e->model.b1, h1, 512, M, CTD_FEATURES_PAD, 1, e->d_tc_err);
-    ctd_k_linear_tc_tma<<<dim3(gm, 256 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h1, 512, e->tmap[1], e->model.b2, h2, 256, M, 512, 1, e->d_tc_err);
-    ctd_k_linear_tc_tma<<<dim3(gm, 128 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h2, 256, e->tmap[2], e->model.b3, h3, 128, M, 256, 1, e->d_tc_err);
-    ctd_k_value_head<<<(n + 127) / 128, 128, 0, st>>>(h3, e->model.w4t, e->model.b4, pending, n, pred, weight);
+  if (vm.tmap_ok) {   // weight operand by TMA from the pre-split terms
+    ctd_k_linear_tc_tma<<<dim3(gm, 512 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(feat, CTD_FEATURES_PAD, vm.tmap[0], m.b1, h1, 512, M, CTD_FEATURES_PAD, 1, e->d_tc_err);
+    ctd_k_linear_tc_tma<<<dim3(gm, 256 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h1, 512, vm.tmap[1], m.b2, h2, 256, M, 512, 1, e->d_tc_err);
+    ctd_k_linear_tc_tma<<<dim3(gm, 128 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h2, 256, vm.tmap[2], m.b3, h3, 128, M, 256, 1, e->d_tc_err);
+    ctd_k_value_head<<<(n + 127) / 128, 128, 0, st>>>(h3, m.w4t, m.b4, pending, n, pred, weight);
     e->launches += 4;
     CTD_CUDA(e, cudaGetLastError());
     return CTD_OK;
   }
-  ctd_k_linear_tc<<<dim3(gm, 512 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(feat, CTD_FEATURES_PAD, e->tc_w1, CTD_FEATURES_PAD, e->model.b1, h1, 512,
+  ctd_k_linear_tc<<<dim3(gm, 512 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(feat, CTD_FEATURES_PAD, vm.tc_w1, CTD_FEATURES_PAD, m.b1, h1, 512,
                                                                        M, CTD_FEATURES_PAD, 1, e->d_tc_err);
-  ctd_k_linear_tc<<<dim3(gm, 256 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h1, 512, e->tc_w2, 512, e->model.b2, h2, 256, M, 512, 1, e->d_tc_err);
-  ctd_k_linear_tc<<<dim3(gm, 128 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h2, 256, e->tc_w3, 256, e->model.b3, h3, 128, M, 256, 1, e->d_tc_err);
-  ctd_k_value_head<<<(n + 127) / 128, 128, 0, st>>>(h3, e->model.w4t, e->model.b4, pending, n, pred, weight);
+  ctd_k_linear_tc<<<dim3(gm, 256 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h1, 512, vm.tc_w2, 512, m.b2, h2, 256, M, 512, 1, e->d_tc_err);
+  ctd_k_linear_tc<<<dim3(gm, 128 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h2, 256, vm.tc_w3, 256, m.b3, h3, 128, M, 256, 1, e->d_tc_err);
+  ctd_k_value_head<<<(n + 127) / 128, 128, 0, st>>>(h3, m.w4t, m.b4, pending, n, pred, weight);
   e->launches += 4;
   CTD_CUDA(e, cudaGetLastError());
   return CTD_OK;
@@ -1641,15 +1652,17 @@ ctd_status ctd_set_value_backend(ctd_engine* e, int backend) {
   return CTD_OK;
 }
 
-ctd_status ctd_set_value_model(ctd_engine* e, const float* w1t, const float* b1, const float* w2t, const float* b2,
-                               const float* w3t, const float* b3, const float* w4t, const float* b4) {
-  if (!e || !w1t || !b1 || !w2t || !b2 || !w3t || !b3 || !w4t || !b4) return CTD_EARG;
+ctd_status ctd_set_value_model_slot(ctd_engine* e, int slot, const float* w1t, const float* b1, const float* w2t, const float* b2,
+                                    const float* w3t, const float* b3, const float* w4t, const float* b4) {
+  if (!e || slot < 0 || slot >= CTD_MAX_VALUE_MODELS || !w1t || !b1 || !w2t || !b2 || !w3t || !b3 || !w4t || !b4) return CTD_EARG;
   CTD_CUDA(e, cudaSetDevice(e->device));
+  CtdValueSlot& v = e->vm[slot];
+  v.ready = false;   // until the whole load below has completed
   const size_t n1 = (size_t)CTD_FEATURES_PAD * 512, n2 = 512 * 256, n3 = 256 * 128, n4 = 128 * 6 + 2;
   const size_t total = n1 + 512 + n2 + 256 + n3 + 128 + n4 + 8;
-  CTD_CUDA(e, e->d_model.grow(total * sizeof(float)));
-  float* p = e->d_model;
-  CtdValueModel& m = e->model;
+  CTD_CUDA(e, v.d_model.grow(total * sizeof(float)));
+  float* p = v.d_model;
+  CtdValueModel& m = v.model;
   const float* src[8] = {w1t, b1, w2t, b2, w3t, b3, w4t, b4};
   const size_t cnt[8] = {n1, 512, n2, 256, n3, 128, 128 * 6, 6};
   const size_t pad[8] = {n1, 512, n2, 256, n3, 128, n4, 8};
@@ -1666,35 +1679,41 @@ ctd_status ctd_set_value_model(ctd_engine* e, const float* w1t, const float* b1,
     for (int o = 0; o < 512; ++o) for (int k = 0; k < CTD_FEATURES_PAD; ++k) h[(size_t)o * CTD_FEATURES_PAD + k] = w1t[(size_t)k * 512 + o];
     for (int o = 0; o < 256; ++o) for (int k = 0; k < 512; ++k) h[t1 + (size_t)o * 512 + k] = w2t[(size_t)k * 256 + o];
     for (int o = 0; o < 128; ++o) for (int k = 0; k < 256; ++k) h[t1 + t2 + (size_t)o * 256 + k] = w3t[(size_t)k * 128 + o];
-    CTD_CUDA(e, e->d_model_tc.grow((t1 + t2 + t3) * sizeof(float)));
-    CTD_CUDA(e, cudaMemcpy(e->d_model_tc, h.get(), (t1 + t2 + t3) * sizeof(float), cudaMemcpyHostToDevice));
-    e->tc_w1 = e->d_model_tc; e->tc_w2 = e->d_model_tc + t1; e->tc_w3 = e->d_model_tc + t1 + t2;
+    CTD_CUDA(e, v.d_model_tc.grow((t1 + t2 + t3) * sizeof(float)));
+    CTD_CUDA(e, cudaMemcpy(v.d_model_tc, h.get(), (t1 + t2 + t3) * sizeof(float), cudaMemcpyHostToDevice));
+    v.tc_w1 = v.d_model_tc; v.tc_w2 = v.d_model_tc + t1; v.tc_w3 = v.d_model_tc + t1 + t2;
     // split the static weights into their TF32 terms once and describe them to the TMA engine
-    CTD_CUDA(e, e->d_wsplit.grow(3 * (t1 + t2 + t3) * sizeof(float)));
-    float* sp[3] = {e->d_wsplit, e->d_wsplit + 3 * t1, e->d_wsplit + 3 * (t1 + t2)};
+    CTD_CUDA(e, v.d_wsplit.grow(3 * (t1 + t2 + t3) * sizeof(float)));
+    float* sp[3] = {v.d_wsplit, v.d_wsplit + 3 * t1, v.d_wsplit + 3 * (t1 + t2)};
     const size_t cnt[3] = {t1, t2, t3};
-    const float* src[3] = {e->tc_w1, e->tc_w2, e->tc_w3};
+    const float* src[3] = {v.tc_w1, v.tc_w2, v.tc_w3};
     const int Ns[3] = {512, 256, 128}, Ks[3] = {CTD_FEATURES_PAD, 512, 256};
-    e->tmap_ok = getenv("CTD_TC_NO_TMA") == nullptr;
+    v.tmap_ok = getenv("CTD_TC_NO_TMA") == nullptr;
     for (int l = 0; l < 3; ++l) {
       ctd_k_split3<<<(unsigned)((cnt[l] + 255) / 256), 256, 0, e->stream>>>(src[l], sp[l], cnt[l]);
       e->launches++;
-      e->tmap_ok = e->tmap_ok && ctd_make_weight_map(&e->tmap[l], sp[l], Ns[l], Ks[l]);
+      v.tmap_ok = v.tmap_ok && ctd_make_weight_map(&v.tmap[l], sp[l], Ns[l], Ks[l]);
     }
     CTD_CUDA(e, cudaGetLastError());
   }
   CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  v.ready = true;
   return CTD_OK;
 }
 
+ctd_status ctd_set_value_model(ctd_engine* e, const float* w1t, const float* b1, const float* w2t, const float* b2,
+                               const float* w3t, const float* b3, const float* w4t, const float* b4) {
+  return ctd_set_value_model_slot(e, 0, w1t, b1, w2t, b2, w3t, b3, w4t, b4);
+}
+
 ctd_status ctd_value_eval(ctd_engine* e, uint32_t n, const float* features, float weight, float* out6) {
-  if (!e || !features || !out6 || n > e->capacity || !e->d_model) return CTD_EARG;
+  if (!e || !features || !out6 || n > e->capacity || !e->vm[0].ready) return CTD_EARG;
   if (n == 0) return CTD_OK;
   CTD_CUDA(e, cudaSetDevice(e->device));
   ctd_status s = ctd_pred_buffers(e);
   if (s != CTD_OK) return s;
   CTD_CUDA(e, cudaMemcpyAsync(e->d_feat, features, (size_t)n * CTD_FEATURES_PAD * sizeof(float), cudaMemcpyHostToDevice, e->stream));
-  s = ctd_value_forward(e, n, nullptr, weight, 0, nullptr);
+  s = ctd_value_forward(e, e->vm[0], n, nullptr, weight, 0, nullptr);
   if (s != CTD_OK) return s;
   CTD_CUDA(e, cudaMemcpy2DAsync(out6, 6 * sizeof(float), e->d_pred, 8 * sizeof(float), 6 * sizeof(float), n, cudaMemcpyDeviceToHost, e->stream));
   CTD_CUDA(e, cudaStreamSynchronize(e->stream));
@@ -1722,9 +1741,9 @@ ctd_status ctd_encode(ctd_engine* e, uint32_t n, int cfr_role_pick, float* featu
 
 ctd_status ctd_mccfr_pred(ctd_engine* e, uint32_t n_roots, uint64_t seed, uint32_t iterations, uint32_t max_depth, int ruleset,
                           float reward_weight, ctd_mccfr_result* results, float* elapsed_ms, uint32_t* waves_out) {
-  if (!e || n_roots > e->capacity || !e->d_knows || !e->d_model || (ruleset < CTD_RULESET_PRESET || ruleset > CTD_RULESET_RANDOM)) return CTD_EARG;
+  if (!e || n_roots > e->capacity || !e->d_knows || !e->vm[0].ready || (ruleset < CTD_RULESET_PRESET || ruleset > CTD_RULESET_RANDOM)) return CTD_EARG;
   if (n_roots == 0) return CTD_OK;
-  CtdSearch sp{n_roots, seed, iterations, ruleset, true, max_depth, reward_weight, false};
+  CtdSearch sp{n_roots, seed, iterations, ruleset, true, max_depth, reward_weight, false, 0};
   return ctd_search(e, sp, results, elapsed_ms, waves_out);
 }
 
@@ -1745,21 +1764,25 @@ ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t fi
     return CTD_EARG;
   CtdArenaArgs a;
   memset(&a, 0, sizeof(a));
-  // seats with the same player share a search group: one batch of roots per group and decision round
+  // seats with the same player (kind, value-model slot included, and parameters) share a search group: one batch of roots per
+  // group and decision round
   CtdSearch groups[6];
   int n_groups = 0;
   for (int s = 0; s < 6; ++s) {
     const ctd_arena_seat& p = seats[s];
     a.seat_group[s] = -1;
-    if (p.kind == CTD_SEAT_RANDOM) continue;
-    if ((p.kind != CTD_SEAT_PURE && p.kind != CTD_SEAT_DEEP) || p.iterations == 0 || (p.kind == CTD_SEAT_DEEP && !e->d_model))
+    const uint32_t kind = (uint32_t)p.kind & 0xFFu, slot = ((uint32_t)p.kind >> 8) & 0xFFu;   // CTD_SEAT_DEEP_MODEL(slot)
+    if (((uint32_t)p.kind >> 16) != 0 || (slot != 0 && kind != CTD_SEAT_DEEP)) return CTD_EARG;
+    if (kind == CTD_SEAT_RANDOM) continue;
+    if ((kind != CTD_SEAT_PURE && kind != CTD_SEAT_DEEP) || p.iterations == 0 ||
+        (kind == CTD_SEAT_DEEP && (slot >= CTD_MAX_VALUE_MODELS || !e->vm[slot].ready)))
       return CTD_EARG;
     for (int t = 0; t < s && a.seat_group[s] < 0; ++t)
       if (a.seat_group[t] >= 0 && seats[t].kind == p.kind && seats[t].iterations == p.iterations && seats[t].max_depth == p.max_depth &&
           seats[t].reward_weight == p.reward_weight)
         a.seat_group[s] = a.seat_group[t];
     if (a.seat_group[s] < 0) {
-      groups[n_groups] = CtdSearch{0, seed, p.iterations, ruleset, p.kind == CTD_SEAT_DEEP, p.max_depth, p.reward_weight, false};
+      groups[n_groups] = CtdSearch{0, seed, p.iterations, ruleset, kind == CTD_SEAT_DEEP, p.max_depth, p.reward_weight, false, (int)slot};
       a.seat_group[s] = (int8_t)n_groups++;
     }
   }

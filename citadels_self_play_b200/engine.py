@@ -26,6 +26,7 @@ class Engine:
             raise EngineError("ctd_create: status %d (%s)" % (st, msg))
         self.capacity = int(capacity)
         self.device = int(device)
+        self._model_arrays = {}
 
     def close(self):
         if getattr(self, "_h", None):
@@ -121,7 +122,8 @@ class Engine:
 
     def arena(self, n_games, seats, seed=DEFAULT_SEED, first_gid=0, ruleset=RULESET_PRESET, max_steps=4096):
         """Games (seed, first_gid + i) played to the end on the device, one player per seat (ctd_arena).
-        seats: six (kind, iterations, max_depth, reward_weight) tuples, kind in layout.SEAT_RANDOM / SEAT_PURE / SEAT_DEEP.
+        seats: six (kind, iterations, max_depth, reward_weight) tuples, kind in layout.SEAT_RANDOM / SEAT_PURE / SEAT_DEEP, a deep
+        seat's value-model slot in bits 8..15 of kind (arena.deep(model=)).
         -> dict(winner[n] i8 (-1: error), points[n, 6] i8, steps[n] u16, searches[n] u32, stats, phase_ms)."""
         if len(seats) != 6:
             raise ValueError("ctd_arena takes one player per seat (6), got %d" % len(seats))
@@ -223,12 +225,13 @@ class Engine:
         self._check(self._lib.ctd_mccfr_root_set(self._h, len(r), r.shape[1], r.ctypes.data, c.ctypes.data, v.ctypes.data),
                     "ctd_mccfr_root_set")
 
-    def set_value_model(self, model):
-        """model: a ValueOnlyNN(418, 512) in eval mode (reference state_dict layout)."""
+    def set_value_model(self, model, slot=0):
+        """model: a ValueOnlyNN(418, 512) in eval mode (reference state_dict layout), loaded into value-model slot `slot` (0 ..
+        layout.MAX_VALUE_MODELS - 1).  mccfr_pred and value_eval use slot 0; an arena's deep seat uses the slot of arena.deep(model=)."""
         from .value_model import fold
         arrs = fold(model)
-        self._model_arrays = arrs   # keep alive during the copy
-        self._check(self._lib.ctd_set_value_model(self._h, *[a.ctypes.data for a in arrs]), "ctd_set_value_model")
+        self._check(self._lib.ctd_set_value_model_slot(self._h, int(slot), *[a.ctypes.data for a in arrs]), "ctd_set_value_model_slot")
+        self._model_arrays[int(slot)] = arrs   # the folded weights of every loaded slot
 
     def set_value_backend(self, backend):
         """'fp32' (CUDA cores, leaves batched in waves), 'tcgen05' (tensor cores, 3xTF32 split precision, waves) or 'fused' (the

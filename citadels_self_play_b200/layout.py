@@ -134,6 +134,9 @@ TREE_TERMINAL_ROOT, TREE_EPOOL, TREE_EENGINE, TREE_REF_RAISE = 1, 2, 4, 16
 # ctd_arena_seat.kind, and the Philox counter word 1 of the arena's random seats (draw s of game gid: block s >> 2, word s & 3)
 SEAT_RANDOM, SEAT_PURE, SEAT_DEEP = 0, 1, 2
 ARENA_STREAM = 4
+# value-model slots of an engine (CTD_MAX_VALUE_MODELS); a deep seat's slot sits in bits 8..15 of its kind (CTD_SEAT_DEEP_MODEL)
+MAX_VALUE_MODELS = 6
+SEAT_MODEL_SHIFT = 8
 
 
 def tree_bytes(n_nodes, child_used, arr_used):

@@ -33,6 +33,15 @@ def reduce_stats(stats, device="cpu", group=None):
     return tensor_to_stats(t)
 
 
+def reduce_sum(values, device="cpu", group=None):
+    """all_reduce(SUM) of integer counts over `group` (no-op for a single process)."""
+    import torch.distributed as dist
+    t = torch.tensor(list(values), dtype=torch.int64, device=device)
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
+    return [int(x) for x in t.tolist()]
+
+
 def reduce_max(values, device="cpu", group=None):
     import torch.distributed as dist
     t = torch.tensor(list(values), dtype=torch.float64, device=device)

@@ -285,9 +285,16 @@ ctd_status ctd_mccfr_root_set(ctd_engine* e, uint32_t n_roots, uint32_t stride, 
 /* ---- value model at depth-limited leaves (algorithms/models.py ValueOnlyNN(418, 512), eval mode) ----
  * Weights are passed BatchNorm-folded and transposed to [in][out]: w1t [448][512] (rows 418..447 zero), b1 [512],
  * w2t [512][256], b2 [256], w3t [256][128], b3 [128], w4t [128][6], b4 [6]  (value_model.fold() builds them from
- * the reference's state_dict, run_utils.py:11-18). */
+ * the reference's state_dict, run_utils.py:11-18).
+ * The engine holds CTD_MAX_VALUE_MODELS models, one slot per possible deep seat of an arena (CTD_SEAT_DEEP_MODEL); a slot
+ * allocates its device memory on first load, and loading one slot leaves the others untouched.  ctd_set_value_model loads
+ * slot 0, the model ctd_mccfr_pred and ctd_value_eval use. */
+#define CTD_MAX_VALUE_MODELS 6
 ctd_status ctd_set_value_model(ctd_engine* e, const float* w1t, const float* b1, const float* w2t, const float* b2,
                                const float* w3t, const float* b3, const float* w4t, const float* b4);
+/* the same for slot `slot` in [0, CTD_MAX_VALUE_MODELS) (anything else: CTD_EARG) */
+ctd_status ctd_set_value_model_slot(ctd_engine* e, int slot, const float* w1t, const float* b1, const float* w2t, const float* b2,
+                                    const float* w3t, const float* b3, const float* w4t, const float* b4);
 /* how leaf values are computed.
  *   0  batched, fp32 CUDA cores: ctd_mccfr_pred advances the trees in waves and evaluates all waiting leaves at once
  *   1  batched, tcgen05 tensor cores with 3xTF32 split precision (same waves)
@@ -356,9 +363,14 @@ void ctd_train_end(ctd_engine* e);
  * Launches grow with decision rounds, not with env steps. */
 #define CTD_SEAT_RANDOM 0  /* uniform over the legal options: Philox stream 4, draw (s >> 2, s & 3) for the record's steps s */
 #define CTD_SEAT_PURE 1    /* run_mccfr -> cfr_train(iterations) */
-#define CTD_SEAT_DEEP 2    /* run_mccfr -> cfr_pred(iterations, max_depth) with the engine's value model (ctd_set_value_model) */
+#define CTD_SEAT_DEEP 2    /* run_mccfr -> cfr_pred(iterations, max_depth) with the value model in slot 0 (ctd_set_value_model) */
+/* a deep seat on the value model in slot `slot` (ctd_set_value_model_slot): bits 8..15 of kind carry the slot, so CTD_SEAT_DEEP is
+ * CTD_SEAT_DEEP_MODEL(0).  ctd_arena returns CTD_EARG for a kind with bits above 15, with slot bits on a random or pure seat, or whose
+ * slot is >= CTD_MAX_VALUE_MODELS or holds no model.  Seats that differ only in their slot search in separate groups, each with
+ * its own weights. */
+#define CTD_SEAT_DEEP_MODEL(slot) (CTD_SEAT_DEEP | ((slot) << 8))
 typedef struct ctd_arena_seat {
-  int32_t kind;
+  int32_t kind;          /* CTD_SEAT_RANDOM, CTD_SEAT_PURE or CTD_SEAT_DEEP_MODEL(slot) */
   uint32_t iterations;
   uint32_t max_depth;    /* CTD_SEAT_DEEP only */
   float reward_weight;   /* CTD_SEAT_DEEP only: model_reward_weights */

@@ -11,7 +11,6 @@ Also times arena.play_games_batched (host-driven game steps, batched searches) a
 in the same process.  The GPU's name and power limit are read in the same run.  Writes one JSON file (rank 0)."""
 import argparse
 import json
-import math
 import os
 import subprocess
 import sys
@@ -28,16 +27,6 @@ CONFIGS = [
     dict(name="deep200_d10_vs_pure200", deep=(200, 10), pure=200, readme_counts=[35, 12, 14, 10, 12, 17]),
     dict(name="deep200_d10_vs_pure2000", deep=(200, 10), pure=2000, readme_counts=[34, 24, 7, 12, 9, 14]),
 ]
-Z99 = 2.5758293035489004
-
-
-def wilson(k, n, z=Z99):
-    if n == 0:
-        return [0.0, 1.0]
-    p = k / n
-    c = (p + z * z / (2 * n)) / (1 + z * z / n)
-    h = z * math.sqrt(p * (1 - p) / n + z * z / (4 * n * n)) / (1 + z * z / n)
-    return [max(0.0, c - h), min(1.0, c + h)]
 
 
 def readme_chi2(counts, rates):
@@ -88,6 +77,7 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     rank, world = (dist.get_rank(), dist.get_world_size()) if distributed else (0, 1)
     from citadels_self_play_b200 import Engine, arena, sharding
+    from citadels_self_play_b200.arena import wilson
     model = load_checkpoint()
     eng = Engine(capacity=args.capacity, device=local)
     eng.set_value_model(model)
