@@ -23,6 +23,11 @@ class ArenaSeat(ctypes.Structure):
                 ("reward_weight", ctypes.c_float)]
 
 
+class RecordOpts(ctypes.Structure):
+    """ctd_record_opts"""
+    _fields_ = [("seat_mask", ctypes.c_uint32), ("mode", ctypes.c_int32), ("threshold", ctypes.c_double)]
+
+
 # every symbol include/citadels_b200.h declares: name -> (restype, argtypes)
 _u32, _u64, _i = ctypes.c_uint32, ctypes.c_uint64, ctypes.c_int
 SIGNATURES = {
@@ -47,6 +52,14 @@ SIGNATURES = {
                              ctypes.POINTER(ctypes.c_float)]),
     "ctd_arena": (_i, [c_void, _u64, _u64, _u64, _i, ctypes.POINTER(ArenaSeat), _u32, c_void, c_void, c_void, c_void,
                        ctypes.POINTER(PlayoutStats), ctypes.POINTER(ctypes.c_float)]),
+    "ctd_arena_record": (_i, [c_void, _u64, _u64, _u64, _i, ctypes.POINTER(ArenaSeat), _u32, c_void, c_void, c_void, c_void,
+                              ctypes.POINTER(PlayoutStats), ctypes.POINTER(RecordOpts), ctypes.POINTER(ctypes.c_float)]),
+    "ctd_dataset_reserve": (_i, [c_void, _u32, _u32]),
+    "ctd_dataset_clear": (_i, [c_void]),
+    "ctd_dataset_info": (_i, [c_void, ctypes.POINTER(_u32), ctypes.POINTER(_u32), ctypes.POINTER(_u64), ctypes.POINTER(_u64)]),
+    "ctd_dataset_read": (_i, [c_void, _u32, _u32, c_void, c_void, c_void]),
+    "ctd_dataset_read_options": (_i, [c_void, _u32, _u32, c_void, c_void]),
+    "ctd_train_begin_dataset": (_i, [c_void, _u32, c_void, _u32, c_void, _i, _u32]),
     "ctd_launch_count": (_u64, [c_void]),
     "ctd_make_roots": (_i, [c_void, _u32, _u64, _u64, _i, _u32, _u32, _i, c_void]),
     "ctd_load_roots": (_i, [c_void, _u32, c_void, c_void, c_void, c_void]),

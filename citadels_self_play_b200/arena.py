@@ -169,20 +169,9 @@ def rank_block(n_games, rank, world):
     return first, min(int(n_games), first + per) - first
 
 
-def play_arena(n_games, seats=None, model=None, engine=None, seed=DEFAULT_SEED, first_gid=0, ruleset=RULESET_PRESET,
-               max_steps=4096, group=None, models=None):
-    """compare_to_random.play_games with a player per seat, every game on the device (Engine.arena).  Under torch.distributed
-    each rank plays its own block of game ids (sharding.first_gid over rank_block's split) and the statistics are summed.
-    Without `engine` the games run on torch's current CUDA device (under torchrun: the rank's own GPU after
-    torch.cuda.set_device(LOCAL_RANK)); the statistics are reduced on the engine's device.
-    models: value models loaded into slots 0 .. len(models) - 1, for the seats deep(..., model=slot); `model` is short for
-    models=[model].  Without `engine` every deep seat's slot must be among them.
-    -> dict(winners[6] and stats over all ranks; this rank's local_stats, first_gid of its games, their per-game arrays
-    winner / points / steps / searches and its phase_ms)."""
-    import torch
-    import torch.distributed as dist
-    from . import sharding
-    seats = default_seats() if seats is None else list(seats)
+def arena_models(seats, model, models, engine):
+    """The value models of play_arena's model= / models= as a list for slots 0, 1, ...; ValueError when both are given, when there are
+    more than an engine holds, or (without `engine`, whose slots may already be loaded) when a deep seat's slot is not among them."""
     if model is not None:
         if models is not None:
             raise ValueError("pass model= or models=, not both")
@@ -193,6 +182,25 @@ def play_arena(n_games, seats=None, model=None, engine=None, seed=DEFAULT_SEED, 
     missing = sorted({_seat_model(s[0]) for s in seats if _seat_kind(s[0]) == SEAT_DEEP} - set(range(len(models))))
     if missing and engine is None:
         raise ValueError("deep seats on value-model slots %s, but models= fills slots [0, %d)" % (missing, len(models)))
+    return models
+
+
+def play_arena(n_games, seats=None, model=None, engine=None, seed=DEFAULT_SEED, first_gid=0, ruleset=RULESET_PRESET,
+               max_steps=4096, group=None, models=None, record=None):
+    """compare_to_random.play_games with a player per seat, every game on the device (Engine.arena).  Under torch.distributed
+    each rank plays its own block of game ids (sharding.first_gid over rank_block's split) and the statistics are summed.
+    Without `engine` the games run on torch's current CUDA device (under torchrun: the rank's own GPU after
+    torch.cuda.set_device(LOCAL_RANK)); the statistics are reduced on the engine's device.
+    models: value models loaded into slots 0 .. len(models) - 1, for the seats deep(..., model=slot); `model` is short for
+    models=[model].  Without `engine` every deep seat's slot must be among them.
+    record: Engine.arena's recording spec, appending to `engine`'s dataset (selfplay.record_arena).
+    -> dict(winners[6] and stats over all ranks; this rank's local_stats, first_gid of its games, their per-game arrays
+    winner / points / steps / searches and its phase_ms)."""
+    import torch
+    import torch.distributed as dist
+    from . import sharding
+    seats = default_seats() if seats is None else list(seats)
+    models = arena_models(seats, model, models, engine)
     dist_on = dist.is_available() and dist.is_initialized()
     rank = dist.get_rank(group) if dist_on else 0
     world = dist.get_world_size(group) if dist_on else 1
@@ -203,7 +211,7 @@ def play_arena(n_games, seats=None, model=None, engine=None, seed=DEFAULT_SEED, 
     try:
         for slot, m in enumerate(models):
             eng.set_value_model(m, slot=slot)
-        out = eng.arena(count, seats, seed=seed, first_gid=first_gid + first, ruleset=ruleset, max_steps=max_steps)
+        out = eng.arena(count, seats, seed=seed, first_gid=first_gid + first, ruleset=ruleset, max_steps=max_steps, record=record)
     finally:
         if own:
             eng.close()

@@ -8,6 +8,7 @@
 
 #define CTD_ARENA_STREAM 4u   // Philox counter word 1 of the random seats' choices (0 game chance, 1 trees, 2 root draws, 3 targets)
 #define CTD_ARENA_GID_BITS 40 // facade.tree_gid: bits 40.. of a tree id carry the game's search number
+#define CTD_REC_NONE 0xFFFFFFFFu  // recording: rec_off of a tree the dataset does not take
 
 // what one game keeps between launches
 struct CtdArenaGame {
@@ -201,6 +202,72 @@ __global__ void __launch_bounds__(256) ctd_k_arena_finish(const CtdArenaGame* ga
     const int maxi = offsetof(ctd_playout_stats, max_steps) / 8;
     if ((int)threadIdx.x == maxi) atomicMax(&gs[maxi], bst[threadIdx.x]);
     else atomicAdd(&gs[threadIdx.x], bst[threadIdx.x]);
+  }
+}
+
+// ------------------------------------------------------------------------------------------ recording (ctd_arena_record)
+// The dataset's cursors and drop counts live on the device, so a search's trees claim their rows without the host waiting.
+struct CtdDatasetCtr {
+  unsigned long long n_records, n_slots, dropped_trees, dropped_records;
+  unsigned long long call_first;   // n_records when the current ctd_arena_record call began: its records are [call_first, n_records)
+};
+
+// Rows for the trees of one search: an exclusive scan of their record and option-slot counts in queue order, behind the dataset's
+// cursors.  A tree is kept when all of its records and slots fit.  The scan runs over every tree, kept or not, and the offsets only
+// grow, so the kept trees are the leading ones and their rows are consecutive.  rec_off[t] = CTD_REC_NONE for a tree not kept (or
+// without records).  One block; tiles of its width in order, so the result does not depend on scheduling.
+#define CTD_RESERVE_THREADS 1024
+__global__ void __launch_bounds__(CTD_RESERVE_THREADS) ctd_k_record_reserve(uint32_t n, const uint32_t* nrec, const uint32_t* nopt,
+                                                                           uint32_t* rec_off, uint32_t* opt_off, CtdDatasetCtr* ctr,
+                                                                           uint32_t max_records, uint32_t max_slots) {
+  __shared__ unsigned long long wr[32], wo[32];
+  __shared__ unsigned long long base_r, base_o, keep_r, keep_o, drop_t, drop_r;
+  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  if (tid == 0) { base_r = ctr->n_records; base_o = ctr->n_slots; keep_r = keep_o = drop_t = drop_r = 0; }
+  __syncthreads();
+  for (uint32_t first = 0; first < n; first += CTD_RESERVE_THREADS) {
+    const uint32_t t = first + tid;
+    const unsigned long long r = t < n ? nrec[t] : 0ull, o = t < n ? nopt[t] : 0ull;
+    unsigned long long sr = r, so = o;   // inclusive scan within the warp
+    for (int d = 1; d < 32; d <<= 1) {
+      const unsigned long long ur = __shfl_up_sync(0xFFFFFFFFu, sr, d), uo = __shfl_up_sync(0xFFFFFFFFu, so, d);
+      if (lane >= d) { sr += ur; so += uo; }
+    }
+    if (lane == 31) { wr[wid] = sr; wo[wid] = so; }
+    __syncthreads();
+    if (wid == 0) {   // exclusive scan of the 32 warp totals
+      const unsigned long long own_r = wr[lane], own_o = wo[lane];
+      unsigned long long xr = own_r, xo = own_o;
+      for (int d = 1; d < 32; d <<= 1) {
+        const unsigned long long ur = __shfl_up_sync(0xFFFFFFFFu, xr, d), uo = __shfl_up_sync(0xFFFFFFFFu, xo, d);
+        if (lane >= d) { xr += ur; xo += uo; }
+      }
+      wr[lane] = xr - own_r; wo[lane] = xo - own_o;
+    }
+    __syncthreads();
+    const unsigned long long off_r = base_r + wr[wid] + sr - r, off_o = base_o + wo[wid] + so - o;
+    const bool keep = r != 0 && off_r + r <= max_records && off_o + o <= max_slots;
+    if (t < n) { rec_off[t] = keep ? (uint32_t)off_r : CTD_REC_NONE; opt_off[t] = keep ? (uint32_t)off_o : 0u; }
+    if (keep) { atomicAdd(&keep_r, r); atomicAdd(&keep_o, o); }
+    else if (r != 0) { atomicAdd(&drop_t, 1ull); atomicAdd(&drop_r, r); }
+    __syncthreads();
+    if (tid == CTD_RESERVE_THREADS - 1) { base_r = off_r + r; base_o = off_o + o; }   // the tile's total, kept or not
+    __syncthreads();
+  }
+  if (tid == 0) {
+    ctr->n_records += keep_r; ctr->n_slots += keep_o;
+    ctr->dropped_trees += drop_t; ctr->dropped_records += drop_r;
+  }
+}
+
+// the outcome of every record of this call: its game's winner (-1 for an errored game) and points, once every game is over
+__global__ void __launch_bounds__(256) ctd_k_record_outcome(const CtdArenaGame* games, const ctd_target_meta* meta, ctd_record_origin* origin,
+                                                            const CtdDatasetCtr* ctr) {
+  const unsigned long long end = ctr->n_records;
+  for (unsigned long long r = ctr->call_first + blockIdx.x * blockDim.x + threadIdx.x; r < end; r += (unsigned long long)gridDim.x * blockDim.x) {
+    const ctd_state& s = games[meta[r].tree].rec;
+    origin[r].winner = s.err ? (int8_t)-1 : s.winner;
+    for (int p = 0; p < 6; ++p) origin[r].points[p] = s.points[p];
   }
 }
 #endif  // __CUDACC__

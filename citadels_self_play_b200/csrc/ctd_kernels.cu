@@ -239,22 +239,28 @@ struct CtdTargetArgs {
   ctd_target_meta* meta;    // [records]
   ctd_option* options;      // [option slots]
   double* regrets;          // [option slots]
+  // recording (ctd_arena_record) only: tree t is the search of game list[t]
+  const CtdArenaGame* games;
+  const uint32_t* list;
+  uint32_t seat_mask;       // trees whose mover (the searching seat) is not in the mask have no records
+  int root_only;            // CTD_RECORD_ROOT: node 0 alone, threshold not applied
+  ctd_record_origin* origin;   // [records]
 };
 
-__global__ void __launch_bounds__(CTD_BLOCK) ctd_k_targets(CtdTargetArgs a) {
-  __shared__ CtdWork works[CTD_WARPS_PER_BLOCK];
-  __shared__ CtdKnow knows[CTD_WARPS_PER_BLOCK];
-  __shared__ __align__(16) ctd_state tstage[CTD_WARPS_PER_BLOCK];
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  const uint32_t t = blockIdx.x * CTD_WARPS_PER_BLOCK + wib;
-  if (t >= a.n_roots || lane != 0) return;
+// Rec: the recording form -- trees of unrecorded seats count nothing, rec_off[t] == CTD_REC_NONE skips a tree, meta.tree is the
+// game index and every record also gets its origin.  Without Rec this is ctd_mccfr_targets' walk.
+template <bool Rec>
+__device__ __forceinline__ void ctd_targets_tree(const CtdTargetArgs& a, uint32_t t, CtdWork* work, CtdKnow* know, ctd_state* stage) {
   CtdTree T;
-  T.w = &works[wib]; T.kn = &knows[wib]; T.stage = &tstage[wib]; T.vnet = nullptr; T.act = nullptr;
+  T.w = work; T.kn = know; T.stage = stage; T.vnet = nullptr; T.act = nullptr;
   ctd_tree_attach(T, &a.hdrs[t], CtdArena{a.hdrs[t].arena, nullptr, 0});
   const CtdTreeHdr& h = *T.hdr;
   uint32_t nrec = 0, nopt = 0, rp_draws = 0;
+  const CtdArenaGame* G = Rec ? &a.games[a.list[t]] : nullptr;
+  bool take = true;
+  if (Rec) take = ((a.seat_mask >> G->rec.player) & 1) && (!a.fill || a.rec_off[t] != CTD_REC_NONE);
   // trees that stopped early (arena exhausted, engine limit, the reference raises) are not training data
-  if (h.n_nodes != 0 && h.status == CTD_TREE_OK) {
+  if (take && h.n_nodes != 0 && h.status == CTD_TREE_OK) {
     // Where node_value counts backpropagations (cfr_train, and cfr_pred in training mode: every backprop adds a reward that sums
     // to one to each node on its path) a child never has more than its parent, so nothing below a node under the threshold
     // qualifies and the walk does not go there: a 2000-iteration tree has ~3800 nodes and a handful over 200 backprops.
@@ -265,7 +271,7 @@ __global__ void __launch_bounds__(CTD_BLOCK) ctd_k_targets(CtdTargetArgs a) {
       const uint32_t K = n.n_children;
       double vs = 0.0;
       for (int i = 0; i < 6; ++i) vs += n.V[i];
-      if (K != 0 && vs >= a.threshold) {
+      if (K != 0 && (vs >= a.threshold || (Rec && a.root_only))) {
         const bool rp = n.flags & CTD_NF_ROLE_PICK;
         uint32_t seat = n.player;
         if (rp) {
@@ -279,8 +285,14 @@ __global__ void __launch_bounds__(CTD_BLOCK) ctd_k_targets(CtdTargetArgs a) {
           ctd_node_load(T, n);
           ctd_encode_game(*T.w, *T.kn, (int)seat, a.feat + (size_t)rec * CTD_FEATURES_PAD);
           ctd_target_meta& m = a.meta[rec];
-          m.tree = t; m.node = (uint32_t)cur; m.n_options = K; m.option_offset = ko; m.seat = seat; m.role_pick = rp ? 1 : 0;
+          m.tree = Rec ? a.list[t] : t; m.node = (uint32_t)cur; m.n_options = K; m.option_offset = ko; m.seat = seat; m.role_pick = rp ? 1 : 0;
           for (int i = 0; i < 6; ++i) m.node_value[i] = n.V[i];
+          if (Rec) {
+            ctd_record_origin& o = a.origin[rec];
+            o.gid = G->rec.gid; o.search = G->searches; o.step = G->rec.steps; o.mover = G->rec.player; o.winner = -1;
+            for (int i = 0; i < 6; ++i) o.points[i] = 0;
+            o.pad[0] = o.pad[1] = 0;
+          }
           const double* R = ctd_R(T, n) + (rp ? seat * 10 : 0);
           const CtdChild* kids = ctd_kids(T, n);
           double rs = 0.0;
@@ -293,6 +305,7 @@ __global__ void __launch_bounds__(CTD_BLOCK) ctd_k_targets(CtdTargetArgs a) {
         ++nrec;
         nopt += K;
       }
+      if (Rec && a.root_only) break;
       // pre-order successor: first child, else next sibling of the nearest ancestor that has one
       if (K != 0 && !(prune && vs < a.threshold)) { cur = (int)ctd_kids(T, n)[0].node; continue; }
       int c = cur;
@@ -312,6 +325,19 @@ __global__ void __launch_bounds__(CTD_BLOCK) ctd_k_targets(CtdTargetArgs a) {
   }
   if (!a.fill) { a.n_targets[t] = nrec; a.n_options[t] = nopt; }
 }
+
+template <bool Rec>
+__device__ __forceinline__ void ctd_targets_warp(const CtdTargetArgs& a) {
+  __shared__ CtdWork works[CTD_WARPS_PER_BLOCK];
+  __shared__ CtdKnow knows[CTD_WARPS_PER_BLOCK];
+  __shared__ __align__(16) ctd_state tstage[CTD_WARPS_PER_BLOCK];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const uint32_t t = blockIdx.x * CTD_WARPS_PER_BLOCK + wib;
+  if (t >= a.n_roots || lane != 0) return;
+  ctd_targets_tree<Rec>(a, t, &works[wib], &knows[wib], &tstage[wib]);
+}
+__global__ void __launch_bounds__(CTD_BLOCK) ctd_k_targets(CtdTargetArgs a) { ctd_targets_warp<false>(a); }
+__global__ void __launch_bounds__(CTD_BLOCK) ctd_k_record_targets(CtdTargetArgs a) { ctd_targets_warp<true>(a); }
 
 // ------------------------------------------------------------------------------------------ single-game entry points
 // The facade's Game object owns its record and the knowledge of all six observers on the host; these kernels run
@@ -652,6 +678,14 @@ struct ctd_engine {
   CtdBuf<uint8_t, true> h_pinned;        // pinned host staging for result copies
   std::unique_ptr<CtdTrainer> trainer;   // value-network training (ctd_train_*), created on first use
   CtdBuf<uint8_t> d_one;  // single-game staging: state | know6 | used_cards | count | winner | opts
+  // self-play dataset (ctd_dataset_*, ctd_arena_record): rows of CTD_FEATURES_PAD floats, metas and origins; option slots
+  uint32_t ds_max_records, ds_max_slots;   // 0: not reserved
+  CtdBuf<float> ds_feat;
+  CtdBuf<ctd_target_meta> ds_meta;
+  CtdBuf<ctd_record_origin> ds_origin;
+  CtdBuf<ctd_option> ds_opt;
+  CtdBuf<double> ds_reg;
+  CtdBuf<CtdDatasetCtr> ds_ctr;
   char err[256];
 };
 
@@ -739,7 +773,7 @@ void ctd_destroy(ctd_engine* e) {
 
 const char* ctd_last_error(const ctd_engine* e) { return e ? e->err : "null engine"; }
 // sizes of the records that cross the boundary (binding self-check): 0 ctd_state, 1 ctd_mccfr_result, 2 ctd_target_meta,
-// 3 knowledge block, 4 exported tree header, 5 exported node, 6 child entry, 7 ctd_playout_stats, 8 ctd_arena_seat
+// 3 knowledge block, 4 exported tree header, 5 exported node, 6 child entry, 7 ctd_playout_stats, 8 ctd_arena_seat, 9 ctd_record_origin
 uint32_t ctd_sizeof(int what) {
   switch (what) {
     case 0: return (uint32_t)sizeof(ctd_state);
@@ -751,6 +785,7 @@ uint32_t ctd_sizeof(int what) {
     case 6: return (uint32_t)sizeof(CtdChild);
     case 7: return (uint32_t)sizeof(ctd_playout_stats);
     case 8: return (uint32_t)sizeof(ctd_arena_seat);
+    case 9: return (uint32_t)sizeof(ctd_record_origin);
     default: return 0;
   }
 }
@@ -1748,17 +1783,41 @@ ctd_status ctd_mccfr_pred(ctd_engine* e, uint32_t n_roots, uint64_t seed, uint32
 }
 
 // ------------------------------------------------------------------------------------------ arena (ctd_arena.cuh)
-// the phase-timing events of one ctd_arena call, destroyed on every way out
+// Record the trees of one arena search (roots [0, cnt), game list[t]), still in e->d_hdrs -- ctd_search leaves every tree there
+// from its final pass, retried trees included.  Three launches between the event pair: count, reserve rows on the device, fill.
+// rcnt: 4 * capacity words.  Nothing is waited for.
+static ctd_status ctd_record_search(ctd_engine* e, const ctd_record_opts& rec, const CtdArenaGame* games, const uint32_t* list, uint32_t cnt,
+                                    uint64_t seed, uint32_t* rcnt, cudaEvent_t ev0, cudaEvent_t ev1) {
+  CtdTargetArgs a;
+  memset(&a, 0, sizeof(a));
+  a.n_roots = cnt; a.hdrs = e->d_hdrs; a.seed = seed; a.threshold = rec.threshold;
+  a.n_targets = rcnt; a.n_options = rcnt + e->capacity; a.rec_off = rcnt + 2 * e->capacity; a.opt_off = rcnt + 3 * e->capacity;
+  a.games = games; a.list = list; a.seat_mask = rec.seat_mask; a.root_only = rec.mode == CTD_RECORD_ROOT;
+  a.feat = e->ds_feat; a.meta = e->ds_meta; a.options = e->ds_opt; a.regrets = e->ds_reg; a.origin = e->ds_origin;
+  CTD_CUDA(e, cudaEventRecord(ev0, e->stream));
+  ctd_k_record_targets<<<ctd_blocks(cnt), CTD_BLOCK, 0, e->stream>>>(a);
+  ctd_k_record_reserve<<<1, CTD_RESERVE_THREADS, 0, e->stream>>>(cnt, a.n_targets, a.n_options, rcnt + 2 * e->capacity, rcnt + 3 * e->capacity,
+                                                                  e->ds_ctr, e->ds_max_records, e->ds_max_slots);
+  a.fill = 1;
+  ctd_k_record_targets<<<ctd_blocks(cnt), CTD_BLOCK, 0, e->stream>>>(a);
+  e->launches += 3;
+  CTD_CUDA(e, cudaGetLastError());
+  CTD_CUDA(e, cudaEventRecord(ev1, e->stream));
+  return CTD_OK;
+}
+
+// the phase-timing events of one ctd_arena call, destroyed on every way out (ev[4], ev[5]: recording only)
 struct CtdArenaEvents {
-  cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+  cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   ~CtdArenaEvents() {
     for (cudaEvent_t v : ev) if (v) cudaEventDestroy(v);
   }
 };
 
-ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t first_gid, int ruleset, const ctd_arena_seat seats[6],
-                     uint32_t max_steps, int8_t* winner, int8_t* points6, uint16_t* steps, uint32_t* searches,
-                     ctd_playout_stats* stats, float* elapsed_ms) {
+// ctd_arena, and with `rec` ctd_arena_record: elapsed_ms then takes a fourth time, the recording's
+static ctd_status ctd_arena_run(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t first_gid, int ruleset, const ctd_arena_seat seats[6],
+                                uint32_t max_steps, int8_t* winner, int8_t* points6, uint16_t* steps, uint32_t* searches,
+                                ctd_playout_stats* stats, const ctd_record_opts* rec, float* elapsed_ms) {
   // max_steps: the record's steps field saturates at 65535, a larger limit would never be reached
   if (!e || !seats || n_games > 0xFFFFFFFFull || max_steps > 65535u || (ruleset < CTD_RULESET_PRESET || ruleset > CTD_RULESET_RANDOM))
     return CTD_EARG;
@@ -1786,10 +1845,16 @@ ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t fi
       a.seat_group[s] = (int8_t)n_groups++;
     }
   }
-  float ms[3] = {0.f, 0.f, 0.f};
+  // a group is recorded when one of its seats is in the mask
+  bool recorded[6] = {false, false, false, false, false, false};
+  if (rec)
+    for (int s = 0; s < 6; ++s)
+      if (a.seat_group[s] >= 0 && ((rec->seat_mask >> s) & 1)) recorded[a.seat_group[s]] = true;
+  float ms[4] = {0.f, 0.f, 0.f, 0.f};
+  const size_t ms_bytes = (rec ? 4 : 3) * sizeof(float);
   if (n_games == 0) {
     if (stats) memset(stats, 0, sizeof(*stats));
-    if (elapsed_ms) memcpy(elapsed_ms, ms, sizeof(ms));
+    if (elapsed_ms) memcpy(elapsed_ms, ms, ms_bytes);
     return CTD_OK;
   }
   const uint32_t n = (uint32_t)n_games;
@@ -1805,7 +1870,9 @@ ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t fi
   CTD_CUDA(e, games.grow((size_t)n * sizeof(CtdArenaGame)));
   CTD_CUDA(e, queue.grow(256 + (size_t)n_groups * n * sizeof(uint32_t)));
   CTD_CUDA(e, out.grow(wb + pb + sb + ((cb + 255) & ~(size_t)255) + sizeof(ctd_playout_stats)));
-  for (cudaEvent_t& v : run.ev) CTD_CUDA(e, cudaEventCreate(&v));
+  for (int k = 0; k < (rec ? 6 : 4); ++k) CTD_CUDA(e, cudaEventCreate(&run.ev[k]));
+  CtdBuf<uint32_t> rcnt;   // recording: per tree of a search, records, option slots, first row, first slot
+  if (rec) CTD_CUDA(e, rcnt.grow((size_t)4 * e->capacity * sizeof(uint32_t)));
   int8_t* d_winner = out;
   int8_t* d_points = d_winner + wb;
   uint16_t* d_steps = (uint16_t*)(d_winner + wb + pb);
@@ -1818,7 +1885,8 @@ ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t fi
   e->slots_rs_n = 0;
   // Phase times.  The advance and the search phases end where the host waits anyway (the queue counts, the search's own
   // read-backs); an apply launch is not waited for: its event pair (ev[2], ev[3]) is read at the next of those waits.
-  bool apply_pending = false;
+  // The recording's pair (ev[4], ev[5]) is read the same way.
+  bool apply_pending = false, record_pending = false;
   auto timed = [&](int phase) -> ctd_status {
     CTD_CUDA(e, cudaEventRecord(run.ev[1], e->stream));
     CTD_CUDA(e, cudaEventSynchronize(run.ev[1]));
@@ -1830,12 +1898,20 @@ ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t fi
       ms[2] += t;
       apply_pending = false;
     }
+    if (record_pending) {
+      CTD_CUDA(e, cudaEventElapsedTime(&t, run.ev[4], run.ev[5]));
+      ms[3] += t;
+      record_pending = false;
+    }
     return CTD_OK;
   };
   CTD_CUDA(e, cudaEventRecord(run.ev[0], e->stream));
   ctd_k_arena_deal<<<ctd_blocks(n), CTD_BLOCK, 0, e->stream>>>(a);
   e->launches++;
   CTD_CUDA(e, cudaGetLastError());
+  if (rec)   // this call's records start where the dataset stands now
+    CTD_CUDA(e, cudaMemcpyAsync(&e->ds_ctr.get()->call_first, &e->ds_ctr.get()->n_records, sizeof(unsigned long long),
+                                cudaMemcpyDeviceToDevice, e->stream));
   uint32_t queued[6];
   for (;;) {   // one decision round: every live game plays on to its next search (or its end), then each group searches
     CTD_CUDA(e, cudaMemsetAsync(a.queued, 0, sizeof(queued), e->stream));
@@ -1859,6 +1935,10 @@ ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t fi
         sp.n_roots = cnt;
         if ((s = ctd_search(e, sp, nullptr, nullptr, nullptr)) != CTD_OK) return s;   // results stay in d_results
         if ((s = timed(1)) != CTD_OK) return s;
+        if (recorded[g]) {   // the trees of this search, before its decisions are applied (the games still stand at the roots)
+          if ((s = ctd_record_search(e, *rec, a.games, list, cnt, seed, rcnt, run.ev[4], run.ev[5])) != CTD_OK) return s;
+          record_pending = true;
+        }
         CTD_CUDA(e, cudaEventRecord(run.ev[2], e->stream));
         ctd_k_arena_apply<<<ctd_blocks(cnt), CTD_BLOCK, 0, e->stream>>>(a, list, cnt, e->d_results);
         e->launches++;
@@ -1875,6 +1955,13 @@ ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t fi
   e->launches++;
   CTD_CUDA(e, cudaGetLastError());
   CTD_CUDA(e, cudaEventRecord(run.ev[1], e->stream));
+  if (rec) {   // every game is over: the outcome of each record this call appended
+    CTD_CUDA(e, cudaEventRecord(run.ev[4], e->stream));
+    ctd_k_record_outcome<<<(unsigned)e->sm_count * 4, 256, 0, e->stream>>>(a.games, e->ds_meta, e->ds_origin, e->ds_ctr);
+    e->launches++;
+    CTD_CUDA(e, cudaGetLastError());
+    CTD_CUDA(e, cudaEventRecord(run.ev[5], e->stream));
+  }
   // the final records of the first games stay readable through ctd_store_states
   const uint32_t keep = n < e->capacity ? n : e->capacity;
   CTD_CUDA(e, cudaMemcpy2DAsync(e->d_slots, sizeof(ctd_state), &a.games[0].rec, sizeof(CtdArenaGame), sizeof(ctd_state), keep,
@@ -1888,7 +1975,97 @@ ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t fi
   float t = 0.f;
   CTD_CUDA(e, cudaEventElapsedTime(&t, run.ev[0], run.ev[1]));   // the final kernel
   ms[0] += t;
-  if (elapsed_ms) memcpy(elapsed_ms, ms, sizeof(ms));
+  if (rec) {
+    CTD_CUDA(e, cudaEventElapsedTime(&t, run.ev[4], run.ev[5]));
+    ms[3] += t;
+  }
+  if (elapsed_ms) memcpy(elapsed_ms, ms, ms_bytes);
+  return CTD_OK;
+}
+
+ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t first_gid, int ruleset, const ctd_arena_seat seats[6],
+                     uint32_t max_steps, int8_t* winner, int8_t* points6, uint16_t* steps, uint32_t* searches,
+                     ctd_playout_stats* stats, float* elapsed_ms) {
+  return ctd_arena_run(e, n_games, seed, first_gid, ruleset, seats, max_steps, winner, points6, steps, searches, stats, nullptr, elapsed_ms);
+}
+
+ctd_status ctd_arena_record(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t first_gid, int ruleset, const ctd_arena_seat seats[6],
+                            uint32_t max_steps, int8_t* winner, int8_t* points6, uint16_t* steps, uint32_t* searches,
+                            ctd_playout_stats* stats, const ctd_record_opts* rec, float* elapsed_ms) {
+  if (!e || !rec || (rec->seat_mask >> 6) != 0 || (rec->mode != CTD_RECORD_TREE && rec->mode != CTD_RECORD_ROOT) ||
+      !(rec->threshold >= 0.0) || e->ds_max_records == 0)
+    return CTD_EARG;
+  return ctd_arena_run(e, n_games, seed, first_gid, ruleset, seats, max_steps, winner, points6, steps, searches, stats, rec, elapsed_ms);
+}
+
+// ------------------------------------------------------------------------------------------ self-play dataset
+ctd_status ctd_dataset_reserve(ctd_engine* e, uint32_t max_records, uint32_t max_option_slots) {
+  if (!e || max_records == 0 || max_option_slots == 0) return CTD_EARG;
+  CTD_CUDA(e, cudaSetDevice(e->device));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));   // no recording may still write into the old buffers
+  e->ds_max_records = e->ds_max_slots = 0;         // not reserved until every buffer exists
+  CTD_CUDA(e, e->ds_feat.grow((size_t)max_records * CTD_FEATURES_PAD * sizeof(float)));
+  CTD_CUDA(e, e->ds_meta.grow((size_t)max_records * sizeof(ctd_target_meta)));
+  CTD_CUDA(e, e->ds_origin.grow((size_t)max_records * sizeof(ctd_record_origin)));
+  CTD_CUDA(e, e->ds_opt.grow((size_t)max_option_slots * sizeof(ctd_option)));
+  CTD_CUDA(e, e->ds_reg.grow((size_t)max_option_slots * sizeof(double)));
+  CTD_CUDA(e, e->ds_ctr.grow(sizeof(CtdDatasetCtr)));
+  CTD_CUDA(e, cudaMemsetAsync(e->ds_ctr, 0, sizeof(CtdDatasetCtr), e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  e->ds_max_records = max_records; e->ds_max_slots = max_option_slots;
+  return CTD_OK;
+}
+
+ctd_status ctd_dataset_clear(ctd_engine* e) {
+  if (!e || e->ds_max_records == 0) return CTD_EARG;
+  CTD_CUDA(e, cudaSetDevice(e->device));
+  CTD_CUDA(e, cudaMemsetAsync(e->ds_ctr, 0, sizeof(CtdDatasetCtr), e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  return CTD_OK;
+}
+
+static ctd_status ctd_dataset_counts(ctd_engine* e, CtdDatasetCtr* c) {
+  if (!e || e->ds_max_records == 0) return CTD_EARG;
+  CTD_CUDA(e, cudaSetDevice(e->device));
+  CTD_CUDA(e, cudaMemcpyAsync(c, e->ds_ctr, sizeof(CtdDatasetCtr), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  return CTD_OK;
+}
+
+ctd_status ctd_dataset_info(ctd_engine* e, uint32_t* n_records, uint32_t* n_option_slots, uint64_t* dropped_trees, uint64_t* dropped_records) {
+  CtdDatasetCtr c;
+  const ctd_status s = ctd_dataset_counts(e, &c);
+  if (s != CTD_OK) return s;
+  if (n_records) *n_records = (uint32_t)c.n_records;
+  if (n_option_slots) *n_option_slots = (uint32_t)c.n_slots;
+  if (dropped_trees) *dropped_trees = c.dropped_trees;
+  if (dropped_records) *dropped_records = c.dropped_records;
+  return CTD_OK;
+}
+
+ctd_status ctd_dataset_read(ctd_engine* e, uint32_t first, uint32_t n, float* features, ctd_target_meta* meta, ctd_record_origin* origin) {
+  CtdDatasetCtr c;
+  const ctd_status s = ctd_dataset_counts(e, &c);
+  if (s != CTD_OK) return s;
+  if ((uint64_t)first + n > c.n_records) return CTD_EARG;
+  if (n == 0) return CTD_OK;
+  if (features) CTD_CUDA(e, cudaMemcpyAsync(features, e->ds_feat + (size_t)first * CTD_FEATURES_PAD, (size_t)n * CTD_FEATURES_PAD * sizeof(float),
+                                            cudaMemcpyDeviceToHost, e->stream));
+  if (meta) CTD_CUDA(e, cudaMemcpyAsync(meta, e->ds_meta + first, (size_t)n * sizeof(ctd_target_meta), cudaMemcpyDeviceToHost, e->stream));
+  if (origin) CTD_CUDA(e, cudaMemcpyAsync(origin, e->ds_origin + first, (size_t)n * sizeof(ctd_record_origin), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  return CTD_OK;
+}
+
+ctd_status ctd_dataset_read_options(ctd_engine* e, uint32_t first_slot, uint32_t n, ctd_option* options, double* regrets) {
+  CtdDatasetCtr c;
+  const ctd_status s = ctd_dataset_counts(e, &c);
+  if (s != CTD_OK) return s;
+  if ((uint64_t)first_slot + n > c.n_slots) return CTD_EARG;
+  if (n == 0) return CTD_OK;
+  if (options) CTD_CUDA(e, cudaMemcpyAsync(options, e->ds_opt + first_slot, (size_t)n * sizeof(ctd_option), cudaMemcpyDeviceToHost, e->stream));
+  if (regrets) CTD_CUDA(e, cudaMemcpyAsync(regrets, e->ds_reg + first_slot, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
   return CTD_OK;
 }
 
@@ -1901,10 +2078,8 @@ void ctd_train_end(ctd_engine* e) {
   e->trainer.reset();
 }
 
-ctd_status ctd_train_begin(ctd_engine* e, uint32_t n_train, const float* features, const double* node_values, uint32_t n_val,
-                           const float* val_features, const double* val_node_values, uint32_t batch_size) {
-  if (!e || !features || !node_values || n_train == 0 || batch_size == 0 || batch_size > 65536 || (n_val != 0 && (!val_features || !val_node_values)))
-    return CTD_EARG;
+// a new trainer for n_train / n_val rows: every buffer allocated and zeroed (the previous trainer is gone)
+static ctd_status ctd_train_alloc(ctd_engine* e, uint32_t n_train, uint32_t n_val, uint32_t batch_size, std::unique_ptr<CtdTrainer>& out) {
   CTD_CUDA(e, cudaSetDevice(e->device));
   ctd_train_end(e);
   std::unique_ptr<CtdTrainer> t(new (std::nothrow) CtdTrainer());
@@ -1931,12 +2106,12 @@ ctd_status ctd_train_begin(ctd_engine* e, uint32_t n_train, const float* feature
   zeroed(t->inv1, CTD_TR_H1); zeroed(t->inv2, CTD_TR_H2); zeroed(t->zero, 512);
   zeroed(t->T, bp * 6); zeroed(t->loss, 2);
   if (c != cudaSuccess) return ctd_fail(e, c, "training buffers");
-  CTD_CUDA(e, cudaMemcpyAsync(t->feat_tr, features, (size_t)n_train * 418 * sizeof(float), cudaMemcpyHostToDevice, e->stream));
-  CTD_CUDA(e, cudaMemcpyAsync(t->val_tr, node_values, (size_t)n_train * 6 * sizeof(double), cudaMemcpyHostToDevice, e->stream));
-  if (n_val) {
-    CTD_CUDA(e, cudaMemcpyAsync(t->feat_va, val_features, (size_t)n_val * 418 * sizeof(float), cudaMemcpyHostToDevice, e->stream));
-    CTD_CUDA(e, cudaMemcpyAsync(t->val_va, val_node_values, (size_t)n_val * 6 * sizeof(double), cudaMemcpyHostToDevice, e->stream));
-  }
+  out = std::move(t);
+  return CTD_OK;
+}
+
+// the rows are in place: the GEMM's set-up, then the trainer becomes the engine's
+static ctd_status ctd_train_install(ctd_engine* e, std::unique_ptr<CtdTrainer>& t) {
   CTD_CUDA(e, cudaFuncSetAttribute(ctd_k_linear_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CTD_TC_SMEM));
   if (!e->d_tc_err) {
     CTD_CUDA(e, e->d_tc_err.grow(sizeof(int)));
@@ -1945,6 +2120,80 @@ ctd_status ctd_train_begin(ctd_engine* e, uint32_t n_train, const float* feature
   CTD_CUDA(e, cudaStreamSynchronize(e->stream));
   e->trainer = std::move(t);
   return CTD_OK;
+}
+
+ctd_status ctd_train_begin(ctd_engine* e, uint32_t n_train, const float* features, const double* node_values, uint32_t n_val,
+                           const float* val_features, const double* val_node_values, uint32_t batch_size) {
+  if (!e || !features || !node_values || n_train == 0 || batch_size == 0 || batch_size > 65536 || (n_val != 0 && (!val_features || !val_node_values)))
+    return CTD_EARG;
+  std::unique_ptr<CtdTrainer> t;
+  ctd_status s = ctd_train_alloc(e, n_train, n_val, batch_size, t);
+  if (s != CTD_OK) return s;
+  CTD_CUDA(e, cudaMemcpyAsync(t->feat_tr, features, (size_t)n_train * 418 * sizeof(float), cudaMemcpyHostToDevice, e->stream));
+  CTD_CUDA(e, cudaMemcpyAsync(t->val_tr, node_values, (size_t)n_train * 6 * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+  if (n_val) {
+    CTD_CUDA(e, cudaMemcpyAsync(t->feat_va, val_features, (size_t)n_val * 418 * sizeof(float), cudaMemcpyHostToDevice, e->stream));
+    CTD_CUDA(e, cudaMemcpyAsync(t->val_va, val_node_values, (size_t)n_val * 6 * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+  }
+  return ctd_train_install(e, t);
+}
+
+// rows idx[0, n) of the dataset -> X [n][418] and labels V [n][6]; bad |= 1 for an index past the records, 2 for a winner label on
+// an errored game.  One block per row.
+__global__ void __launch_bounds__(128) ctd_k_dataset_rows(const float* feat, const ctd_target_meta* meta, const ctd_record_origin* origin,
+                                                          const CtdDatasetCtr* ctr, const uint32_t* idx, uint32_t n, int label, float* X,
+                                                          double* V, int* bad) {
+  const uint32_t r = blockIdx.x;
+  if (r >= n) return;
+  const uint32_t i = idx[r];
+  if (i >= ctr->n_records) {
+    if (threadIdx.x == 0) atomicOr(bad, 1);
+    return;
+  }
+  for (int c = threadIdx.x; c < 418; c += blockDim.x) X[(size_t)r * 418 + c] = feat[(size_t)i * CTD_FEATURES_PAD + c];
+  if (threadIdx.x < 6) {
+    double v = meta[i].node_value[threadIdx.x];
+    if (label == CTD_LABEL_WINNER) {
+      const int w = origin[i].winner;
+      if (w < 0 && threadIdx.x == 0) atomicOr(bad, 2);
+      v = (int)threadIdx.x == w ? 1.0 : 0.0;
+    }
+    V[(size_t)r * 6 + threadIdx.x] = v;
+  }
+}
+
+ctd_status ctd_train_begin_dataset(ctd_engine* e, uint32_t n_train, const uint32_t* train_idx, uint32_t n_val, const uint32_t* val_idx,
+                                   int label, uint32_t batch_size) {
+  if (!e || !train_idx || n_train == 0 || batch_size == 0 || batch_size > 65536 || (n_val != 0 && !val_idx) || e->ds_max_records == 0 ||
+      (label != CTD_LABEL_NODE_VALUE && label != CTD_LABEL_WINNER))
+    return CTD_EARG;
+  std::unique_ptr<CtdTrainer> t;
+  ctd_status s = ctd_train_alloc(e, n_train, n_val, batch_size, t);
+  if (s != CTD_OK) return s;
+  CtdBuf<uint32_t> d_idx;
+  CtdBuf<int> d_bad;
+  CTD_CUDA(e, d_idx.grow(((size_t)n_train + n_val) * sizeof(uint32_t)));
+  CTD_CUDA(e, d_bad.grow(sizeof(int)));
+  CTD_CUDA(e, cudaMemsetAsync(d_bad, 0, sizeof(int), e->stream));
+  CTD_CUDA(e, cudaMemcpyAsync(d_idx, train_idx, (size_t)n_train * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
+  if (n_val) CTD_CUDA(e, cudaMemcpyAsync(d_idx + n_train, val_idx, (size_t)n_val * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
+  ctd_k_dataset_rows<<<n_train, 128, 0, e->stream>>>(e->ds_feat, e->ds_meta, e->ds_origin, e->ds_ctr, d_idx, n_train, label, t->feat_tr,
+                                                      t->val_tr, d_bad);
+  e->launches++;
+  if (n_val) {
+    ctd_k_dataset_rows<<<n_val, 128, 0, e->stream>>>(e->ds_feat, e->ds_meta, e->ds_origin, e->ds_ctr, d_idx + n_train, n_val, label,
+                                                      t->feat_va, t->val_va, d_bad);
+    e->launches++;
+  }
+  CTD_CUDA(e, cudaGetLastError());
+  int bad = 0;
+  CTD_CUDA(e, cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  if (bad) {
+    snprintf(e->err, sizeof(e->err), "ctd_train_begin_dataset: %s", bad & 1 ? "an index past the dataset's records" : "a winner label on an errored game");
+    return CTD_EARG;
+  }
+  return ctd_train_install(e, t);
 }
 
 // the 16 tensors of ValueOnlyNN(418, 512).state_dict() in its own order (num_batches_tracked aside):

@@ -4,7 +4,7 @@ import ctypes
 import numpy as np
 
 from . import _lib
-from .layout import STATE_BYTES, KNOW_BYTES, MCCFR_RESULT_DTYPE, TARGET_META_DTYPE, TreeView, encode_options
+from .layout import STATE_BYTES, KNOW_BYTES, MCCFR_RESULT_DTYPE, TARGET_META_DTYPE, ORIGIN_DTYPE, TreeView, encode_options
 
 RULESET_PRESET, RULESET_CLASSIC, RULESET_RANDOM = 0, 1, 2
 ROOTS_CLOSE_TO_FINISHED, ROOTS_RANDOM_GAME = 0, 1
@@ -120,11 +120,14 @@ class Engine:
         d["kernel_ms"] = ms.value
         return dict(stats=d)
 
-    def arena(self, n_games, seats, seed=DEFAULT_SEED, first_gid=0, ruleset=RULESET_PRESET, max_steps=4096):
+    def arena(self, n_games, seats, seed=DEFAULT_SEED, first_gid=0, ruleset=RULESET_PRESET, max_steps=4096, record=None):
         """Games (seed, first_gid + i) played to the end on the device, one player per seat (ctd_arena).
         seats: six (kind, iterations, max_depth, reward_weight) tuples, kind in layout.SEAT_RANDOM / SEAT_PURE / SEAT_DEEP, a deep
         seat's value-model slot in bits 8..15 of kind (arena.deep(model=)).
-        -> dict(winner[n] i8 (-1: error), points[n, 6] i8, steps[n] u16, searches[n] u32, stats, phase_ms)."""
+        record: None, or (seats, mode, threshold) to append the targets of those seats' searches to the engine's dataset
+        (ctd_arena_record; dataset_reserve first): mode layout.RECORD_TREE (CFRNode.get_all_targets(threshold) of every tree) or
+        RECORD_ROOT (the position played, threshold not applied).  The games are the same either way.
+        -> dict(winner[n] i8 (-1: error), points[n, 6] i8, steps[n] u16, searches[n] u32, stats, phase_ms (with record: + "record"))."""
         if len(seats) != 6:
             raise ValueError("ctd_arena takes one player per seat (6), got %d" % len(seats))
         arr = (_lib.ArenaSeat * 6)(*[_lib.ArenaSeat(int(k), int(it), int(d), float(wt)) for k, it, d, wt in seats])
@@ -133,12 +136,55 @@ class Engine:
         steps = np.empty(n_games, dtype=np.uint16)
         searches = np.empty(n_games, dtype=np.uint32)
         stats = _lib.PlayoutStats()
-        ms = (ctypes.c_float * 3)()
-        self._check(self._lib.ctd_arena(self._h, n_games, seed, first_gid, ruleset, arr, max_steps, winner.ctypes.data,
-                                        points.ctypes.data, steps.ctypes.data, searches.ctypes.data, ctypes.byref(stats), ms),
-                    "ctd_arena")
-        return dict(winner=winner, points=points, steps=steps, searches=searches, stats=stats_dict(stats),
-                    phase_ms=dict(advance=ms[0], search=ms[1], apply=ms[2]))
+        ms = (ctypes.c_float * 4)()
+        args = (self._h, n_games, seed, first_gid, ruleset, arr, max_steps, winner.ctypes.data, points.ctypes.data, steps.ctypes.data,
+                searches.ctypes.data, ctypes.byref(stats))
+        if record is None:
+            self._check(self._lib.ctd_arena(*args, ms), "ctd_arena")
+        else:
+            rec_seats, mode, threshold = record
+            mask = 0
+            for s in rec_seats:
+                mask |= 1 << int(s)
+            opts = _lib.RecordOpts(mask, int(mode), float(threshold))
+            self._check(self._lib.ctd_arena_record(*args, ctypes.byref(opts), ms), "ctd_arena_record")
+        phase_ms = dict(advance=ms[0], search=ms[1], apply=ms[2])
+        if record is not None:
+            phase_ms["record"] = ms[3]
+        return dict(winner=winner, points=points, steps=steps, searches=searches, stats=stats_dict(stats), phase_ms=phase_ms)
+
+    # ---- self-play dataset (filled by arena(record=...)) ----
+    def dataset_reserve(self, max_records, max_option_slots):
+        """Allocate the engine's dataset in HBM (max_records rows of 448 floats; max_option_slots options / regrets) and clear it."""
+        self._check(self._lib.ctd_dataset_reserve(self._h, int(max_records), int(max_option_slots)), "ctd_dataset_reserve")
+
+    def dataset_clear(self):
+        self._check(self._lib.ctd_dataset_clear(self._h), "ctd_dataset_clear")
+
+    def dataset_info(self):
+        """-> dict(records, option_slots, dropped_trees, dropped_records): trees that did not fit are dropped whole."""
+        nr, ns, dt, dr = ctypes.c_uint32(), ctypes.c_uint32(), ctypes.c_uint64(), ctypes.c_uint64()
+        self._check(self._lib.ctd_dataset_info(self._h, ctypes.byref(nr), ctypes.byref(ns), ctypes.byref(dt), ctypes.byref(dr)),
+                    "ctd_dataset_info")
+        return dict(records=nr.value, option_slots=ns.value, dropped_trees=dt.value, dropped_records=dr.value)
+
+    def dataset_read(self):
+        """Every record of the dataset in canonical order (origin gid, search, then pre-order within the tree): features[R, 418] f32,
+        meta[R] (tree: the game's index in its arena call; option_offset into options / regrets), origin[R] (layout.ORIGIN_DTYPE),
+        row[R] (the record's physical row, what train_on_dataset's indices name), and every option slot: options[S] u64, regrets[S]
+        f64.  Engine.targets_as_tuples accepts the result as it is."""
+        info = self.dataset_info()
+        n, ns = info["records"], info["option_slots"]
+        feats = np.zeros((n, 448), dtype=np.float32)
+        meta = np.zeros(n, dtype=TARGET_META_DTYPE)
+        origin = np.zeros(n, dtype=ORIGIN_DTYPE)
+        opts = np.zeros(ns, dtype=np.uint64)
+        regs = np.zeros(ns, dtype=np.float64)
+        self._check(self._lib.ctd_dataset_read(self._h, 0, n, feats.ctypes.data, meta.ctypes.data, origin.ctypes.data), "ctd_dataset_read")
+        self._check(self._lib.ctd_dataset_read_options(self._h, 0, ns, opts.ctypes.data, regs.ctypes.data), "ctd_dataset_read_options")
+        # a tree's records are consecutive in pre-order, so the physical row orders them within (gid, search)
+        row = np.lexsort((np.arange(n), origin["search"], origin["gid"])).astype(np.int64)
+        return dict(features=feats[row, :418], meta=meta[row], origin=origin[row], row=row, options=opts, regrets=regs)
 
     def playout_slots(self, n, max_steps=4096):
         winner = np.empty(n, dtype=np.int8)

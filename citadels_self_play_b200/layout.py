@@ -184,6 +184,14 @@ TARGET_META_DTYPE = np.dtype([("tree", np.uint32), ("node", np.uint32), ("n_opti
                               ("seat", np.uint32), ("role_pick", np.uint32), ("node_value", np.float64, 6)])
 assert TARGET_META_DTYPE.itemsize == 72
 
+# ctd_record_origin (ctd_sizeof(9)): where a self-play record came from and how its game ended (winner -1: errored or max_steps)
+ORIGIN_DTYPE = np.dtype([("gid", np.uint64), ("search", np.uint32), ("step", np.uint16), ("mover", np.uint8), ("winner", np.int8),
+                         ("points", np.int8, 6), ("pad", np.uint8, 2)])
+assert ORIGIN_DTYPE.itemsize == 24
+# ctd_record_opts.mode and the labels of ctd_train_begin_dataset
+RECORD_TREE, RECORD_ROOT = 0, 1
+LABEL_NODE_VALUE, LABEL_WINNER = 0, 1
+
 
 def encode_options(descs):
     """option.encode_option (game/option.py:52-115) for a list of descriptors -> float32[K, 131].

@@ -75,6 +75,20 @@ class Trainer:
         engine._check(self.lib.ctd_train_begin(self.h, len(f), f.ctypes.data, v.ctypes.data, len(vf), vf.ctypes.data if len(vf) else None,
                                                vv.ctypes.data if len(vf) else None, int(batch_size)), "ctd_train_begin")
 
+    @classmethod
+    def from_dataset(cls, engine, train_idx, val_idx, label, batch_size):
+        """ctd_train_begin_dataset: the rows are records train_idx / val_idx (physical rows) of the engine's dataset, gathered on the
+        device; label layout.LABEL_NODE_VALUE or LABEL_WINNER."""
+        self = cls.__new__(cls)
+        self.e = engine
+        self.lib, self.h = engine._lib, engine._h
+        ti = np.ascontiguousarray(train_idx, dtype=np.uint32).reshape(-1)
+        vi = np.ascontiguousarray(val_idx, dtype=np.uint32).reshape(-1)
+        self.n_train, self.n_val = len(ti), len(vi)
+        engine._check(self.lib.ctd_train_begin_dataset(self.h, len(ti), ti.ctypes.data, len(vi), vi.ctypes.data if len(vi) else None,
+                                                       int(label), int(batch_size)), "ctd_train_begin_dataset")
+        return self
+
     def _ptrs(self, arrs):
         return (ctypes.c_void_p * 16)(*[a.ctypes.data for a in arrs])
 
@@ -120,7 +134,6 @@ def train_node_value_only(train_data, val_data, epochs, lr, hidden_size=512, gam
     """algorithms/train.py:13-86.  -> best evaluation loss; writes <parent_folder>/best_model.pt.
     `model` (optional): a ValueOnlyNN(418, 512) whose weights are the starting point (default: a freshly initialised one, as in
     the reference); `history` (optional dict) receives the per-epoch train / eval losses, learning rates and the final state."""
-    import torch
     from .value_model import ValueOnlyNN
     if hidden_size != 512:
         raise ValueError("the training kernels are built for ValueOnlyNN(418, 512)")
@@ -130,30 +143,37 @@ def train_node_value_only(train_data, val_data, epochs, lr, hidden_size=512, gam
     eng = engine or Engine(capacity=8, device=0 if device in (None, "cuda", "cuda:0") else int(str(device).split(":")[-1]))
     tr = Trainer(eng, _stack(train_data, 0, np.float32), _stack(train_data, 2, np.float64), _stack(val_data, 0, np.float32),
                  _stack(val_data, 2, np.float64), batch_size)
-    train_losses, eval_losses, lrs = [], [], []
-    best = float("inf")
     try:
-        tr.set_state(model.state_dict())
-        steps_per_epoch = (tr.n_train + batch_size - 1) // batch_size
-        for epoch in range(epochs):
-            cur_lr = lr * gamma ** (epoch // 300)                         # StepLR(step_size=300, gamma), stepped once per epoch
-            tl, el = tr.epoch(seed, cur_lr, epoch_permutation(seed, epoch, tr.n_train))
-            train_losses.append(tl)
-            eval_losses.append(el)
-            lrs.append(lr * gamma ** ((epoch + 1) // 300))                # scheduler.get_last_lr() after scheduler.step()
-            if el < best:
-                best = el
-                sd = {k: torch.from_numpy(v.copy()) for k, v in tr.get_state().items()}
-                for bn in ("bn1", "bn2"):
-                    sd[bn + ".num_batches_tracked"] = torch.tensor((epoch + 1) * steps_per_epoch, dtype=torch.long)
-                ordered = {k: sd[k] for k in model.state_dict().keys()}
-                torch.save(ordered, os.path.join(parent_folder, "best_model.pt"))
-            if verbose:
-                print("Epoch %d/%d - Train Loss: %.4f - Eval Loss: %.4f" % (epoch + 1, epochs, tl, el))
-        if history is not None:
-            history.update(train_losses=train_losses, eval_losses=eval_losses, learning_rates=lrs, final_state=tr.get_state())
+        return _epochs(tr, model, epochs, lr, gamma, batch_size, seed, parent_folder, verbose, history)
     finally:
         tr.close()
         if own:
             eng.close()
+
+
+def _epochs(tr, model, epochs, lr, gamma, batch_size, seed, parent_folder, verbose, history):
+    """The epoch loop of train_node_value_only on a trainer that holds its rows: start from `model`'s weights, StepLR(300, gamma),
+    <parent_folder>/best_model.pt at every new best evaluation loss.  -> best evaluation loss."""
+    import torch
+    train_losses, eval_losses, lrs = [], [], []
+    best = float("inf")
+    tr.set_state(model.state_dict())
+    steps_per_epoch = (tr.n_train + batch_size - 1) // batch_size
+    for epoch in range(epochs):
+        cur_lr = lr * gamma ** (epoch // 300)                         # StepLR(step_size=300, gamma), stepped once per epoch
+        tl, el = tr.epoch(seed, cur_lr, epoch_permutation(seed, epoch, tr.n_train))
+        train_losses.append(tl)
+        eval_losses.append(el)
+        lrs.append(lr * gamma ** ((epoch + 1) // 300))                # scheduler.get_last_lr() after scheduler.step()
+        if el < best:
+            best = el
+            sd = {k: torch.from_numpy(v.copy()) for k, v in tr.get_state().items()}
+            for bn in ("bn1", "bn2"):
+                sd[bn + ".num_batches_tracked"] = torch.tensor((epoch + 1) * steps_per_epoch, dtype=torch.long)
+            ordered = {k: sd[k] for k in model.state_dict().keys()}
+            torch.save(ordered, os.path.join(parent_folder, "best_model.pt"))
+        if verbose:
+            print("Epoch %d/%d - Train Loss: %.4f - Eval Loss: %.4f" % (epoch + 1, epochs, tl, el))
+    if history is not None:
+        history.update(train_losses=train_losses, eval_losses=eval_losses, learning_rates=lrs, final_state=tr.get_state())
     return best

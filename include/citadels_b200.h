@@ -131,7 +131,7 @@ void ctd_destroy(ctd_engine* e);
 const char* ctd_last_error(const ctd_engine* e);
 /* sizeof of the records that cross this boundary, for a binding to check its own layouts against: 0 ctd_state, 1 ctd_mccfr_result,
  * 2 ctd_target_meta, 3 knowledge block, 4 exported tree header, 5 exported node, 6 exported child entry, 7 ctd_playout_stats,
- * 8 ctd_arena_seat */
+ * 8 ctd_arena_seat, 9 ctd_record_origin */
 uint32_t ctd_sizeof(int what);
 ctd_status ctd_sync(ctd_engine* e);
 /* use an existing CUDA stream (cudaStream_t as void*); default is a stream the engine owns */
@@ -386,6 +386,63 @@ typedef struct ctd_arena_seat {
 ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t first_gid, int ruleset,
                      const ctd_arena_seat seats[6], uint32_t max_steps, int8_t* winner, int8_t* points6,
                      uint16_t* steps, uint32_t* searches, ctd_playout_stats* stats, float* elapsed_ms);
+
+/* ---- self-play training data: the arena records its searches' targets into a dataset the engine keeps in HBM ----
+ * ctd_arena_record is ctd_arena plus recording: after each search of a group holding a recorded seat, the targets of its trees are
+ * appended to the dataset (features, ctd_target_meta, options / regrets as ctd_mccfr_targets writes them, and a ctd_record_origin
+ * per record).  The games, their outcomes, the final records and the statistics are those of ctd_arena with the same arguments:
+ * recording only reads the trees, and the role-pick seat of a record is drawn from the targets' own stream (3) of its tree.
+ * In the dataset, ctd_target_meta.tree is the game's index in its ctd_arena_record call and option_offset indexes the dataset's
+ * option slots.  Records of one tree are consecutive in pre-order; trees are appended in no fixed order (the arena queues its games
+ * with atomics), so the canonical order is (origin.gid, origin.search, row).
+ * Capacity is enforced on the device: the trees of a search are kept in queue order while all their records and option slots fit;
+ * a tree that does not fit is dropped whole and counted. */
+typedef struct ctd_record_origin {
+  uint64_t gid;          /* the game: ctd_game_new(seed, gid, ruleset) */
+  uint32_t search;       /* the game's search number t: the tree id is (gid & (2^40 - 1)) | t << 40 */
+  uint16_t step;         /* the record's steps at that search */
+  uint8_t mover;         /* the seat whose search made the tree */
+  int8_t winner;         /* the game's winner, filled in when the call ends; -1 for an errored game or one stopped at max_steps */
+  int8_t points[6];      /* the game's points, filled in with the winner */
+  uint8_t pad[2];
+} ctd_record_origin;
+#define CTD_RECORD_TREE 0  /* every target of the tree: CFRNode.get_all_targets(threshold) */
+#define CTD_RECORD_ROOT 1  /* node 0 only, the position the game played, whenever it has children (threshold not applied) */
+typedef struct ctd_record_opts {
+  uint32_t seat_mask;    /* bit s: record the trees of seat s's searches (bits above 5: CTD_EARG) */
+  int32_t mode;          /* CTD_RECORD_TREE or CTD_RECORD_ROOT */
+  double threshold;      /* CTD_RECORD_TREE: node_value.sum() >= threshold (the reference uses 15); >= 0 */
+} ctd_record_opts;
+/* Note: a deep seat's tree in eval mode writes node_value only on a node's first backprop, so it sums to reward_weight (or 1 at a
+ * terminal) and never reaches the reference's threshold of 15: record deep seats with CTD_RECORD_ROOT and train on
+ * CTD_LABEL_WINNER, not on the model's own values. */
+/* allocate the dataset (max_records rows of 448 floats, metas and origins; max_option_slots options and regrets) and clear it;
+ * both sizes >= 1 */
+ctd_status ctd_dataset_reserve(ctd_engine* e, uint32_t max_records, uint32_t max_option_slots);
+/* empty the dataset (keeps its allocation) */
+ctd_status ctd_dataset_clear(ctd_engine* e);
+/* records and option slots held, trees and records dropped for want of room since the last reserve / clear (outputs may be NULL) */
+ctd_status ctd_dataset_info(ctd_engine* e, uint32_t* n_records, uint32_t* n_option_slots, uint64_t* dropped_trees,
+                            uint64_t* dropped_records);
+/* records [first, first + n): features [n][448] f32, meta, origin (outputs may be NULL); first + n > n_records: CTD_EARG */
+ctd_status ctd_dataset_read(ctd_engine* e, uint32_t first, uint32_t n, float* features, ctd_target_meta* meta,
+                            ctd_record_origin* origin);
+/* option slots [first_slot, first_slot + n): descriptors and regrets (outputs may be NULL); beyond n_option_slots: CTD_EARG */
+ctd_status ctd_dataset_read_options(ctd_engine* e, uint32_t first_slot, uint32_t n, ctd_option* options, double* regrets);
+/* ctd_arena with recording.  rec: which seats, which mode, which threshold; CTD_EARG for a NULL rec, seat-mask bits above 5, an
+ * unknown mode, a negative or NaN threshold, or no dataset reserved.  elapsed_ms (may be NULL) receives four CUDA-event times: the
+ * three of ctd_arena and the recording (count, reserve and fill kernels per search, the outcome kernel at the end). */
+ctd_status ctd_arena_record(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t first_gid, int ruleset,
+                            const ctd_arena_seat seats[6], uint32_t max_steps, int8_t* winner, int8_t* points6, uint16_t* steps,
+                            uint32_t* searches, ctd_playout_stats* stats, const ctd_record_opts* rec, float* elapsed_ms);
+/* ctd_train_begin with its rows gathered on the device from the dataset: records train_idx[n_train] and val_idx[n_val] (physical
+ * rows).  label: CTD_LABEL_NODE_VALUE = meta.node_value (the reference's target), CTD_LABEL_WINNER = one-hot of origin.winner (a
+ * single sample of what a pure tree's node_value estimates).  CTD_EARG for an index >= n_records, a winner label on a record whose
+ * winner is -1, an unknown label, or whatever ctd_train_begin rejects. */
+#define CTD_LABEL_NODE_VALUE 0
+#define CTD_LABEL_WINNER 1
+ctd_status ctd_train_begin_dataset(ctd_engine* e, uint32_t n_train, const uint32_t* train_idx, uint32_t n_val, const uint32_t* val_idx,
+                                   int label, uint32_t batch_size);
 
 /* number of kernels this engine has launched so far */
 uint64_t ctd_launch_count(const ctd_engine* e);
