@@ -59,6 +59,7 @@ SIGNATURES = {
     "ctd_dataset_info": (_i, [c_void, ctypes.POINTER(_u32), ctypes.POINTER(_u32), ctypes.POINTER(_u64), ctypes.POINTER(_u64)]),
     "ctd_dataset_read": (_i, [c_void, _u32, _u32, c_void, c_void, c_void]),
     "ctd_dataset_read_options": (_i, [c_void, _u32, _u32, c_void, c_void]),
+    "ctd_dataset_append": (_i, [c_void, _u32, _u32, c_void, c_void, c_void, c_void, c_void]),
     "ctd_train_begin_dataset": (_i, [c_void, _u32, c_void, _u32, c_void, _i, _u32]),
     "ctd_launch_count": (_u64, [c_void]),
     "ctd_make_roots": (_i, [c_void, _u32, _u64, _u64, _i, _u32, _u32, _i, c_void]),

@@ -270,4 +270,31 @@ __global__ void __launch_bounds__(256) ctd_k_record_outcome(const CtdArenaGame* 
     for (int p = 0; p < 6; ++p) origin[r].points[p] = s.points[p];
   }
 }
+
+// ctd_dataset_append: n records and n_slots option slots were copied in past the cursors, where no read reaches.  Rebase their
+// option_offset by the slot cursor, OR every malformed record into *bad (1 option span, 2 mover, 4 winner), and advance the
+// cursors only when none is.  One block, so the commit comes after every check.
+#define CTD_APPEND_THREADS 1024
+__global__ void __launch_bounds__(CTD_APPEND_THREADS) ctd_k_dataset_append(ctd_target_meta* meta, const ctd_record_origin* origin,
+                                                                           CtdDatasetCtr* ctr, uint32_t n, uint32_t n_slots, int* bad) {
+  __shared__ int sbad;
+  if (threadIdx.x == 0) sbad = 0;
+  __syncthreads();
+  const unsigned long long base = ctr->n_records, slots = ctr->n_slots;
+  int b = 0;
+  for (uint32_t i = threadIdx.x; i < n; i += CTD_APPEND_THREADS) {
+    ctd_target_meta& m = meta[base + i];
+    const ctd_record_origin& o = origin[base + i];
+    if (m.n_options == 0 || (unsigned long long)m.option_offset + m.n_options > n_slots) b |= 1;
+    if (o.mover > 5) b |= 2;
+    if (o.winner < -1 || o.winner > 5) b |= 4;
+    m.option_offset += (uint32_t)slots;
+  }
+  if (b) atomicOr(&sbad, b);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    if (sbad == 0) { ctr->n_records = base + n; ctr->n_slots = slots + n_slots; }
+    *bad = sbad;
+  }
+}
 #endif  // __CUDACC__

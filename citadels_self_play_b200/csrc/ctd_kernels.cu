@@ -2049,10 +2049,11 @@ ctd_status ctd_dataset_read(ctd_engine* e, uint32_t first, uint32_t n, float* fe
   if (s != CTD_OK) return s;
   if ((uint64_t)first + n > c.n_records) return CTD_EARG;
   if (n == 0) return CTD_OK;
+  // cudaMemcpyDefault: the outputs may be host memory or device memory on any GPU
   if (features) CTD_CUDA(e, cudaMemcpyAsync(features, e->ds_feat + (size_t)first * CTD_FEATURES_PAD, (size_t)n * CTD_FEATURES_PAD * sizeof(float),
-                                            cudaMemcpyDeviceToHost, e->stream));
-  if (meta) CTD_CUDA(e, cudaMemcpyAsync(meta, e->ds_meta + first, (size_t)n * sizeof(ctd_target_meta), cudaMemcpyDeviceToHost, e->stream));
-  if (origin) CTD_CUDA(e, cudaMemcpyAsync(origin, e->ds_origin + first, (size_t)n * sizeof(ctd_record_origin), cudaMemcpyDeviceToHost, e->stream));
+                                            cudaMemcpyDefault, e->stream));
+  if (meta) CTD_CUDA(e, cudaMemcpyAsync(meta, e->ds_meta + first, (size_t)n * sizeof(ctd_target_meta), cudaMemcpyDefault, e->stream));
+  if (origin) CTD_CUDA(e, cudaMemcpyAsync(origin, e->ds_origin + first, (size_t)n * sizeof(ctd_record_origin), cudaMemcpyDefault, e->stream));
   CTD_CUDA(e, cudaStreamSynchronize(e->stream));
   return CTD_OK;
 }
@@ -2063,9 +2064,50 @@ ctd_status ctd_dataset_read_options(ctd_engine* e, uint32_t first_slot, uint32_t
   if (s != CTD_OK) return s;
   if ((uint64_t)first_slot + n > c.n_slots) return CTD_EARG;
   if (n == 0) return CTD_OK;
-  if (options) CTD_CUDA(e, cudaMemcpyAsync(options, e->ds_opt + first_slot, (size_t)n * sizeof(ctd_option), cudaMemcpyDeviceToHost, e->stream));
-  if (regrets) CTD_CUDA(e, cudaMemcpyAsync(regrets, e->ds_reg + first_slot, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+  if (options) CTD_CUDA(e, cudaMemcpyAsync(options, e->ds_opt + first_slot, (size_t)n * sizeof(ctd_option), cudaMemcpyDefault, e->stream));
+  if (regrets) CTD_CUDA(e, cudaMemcpyAsync(regrets, e->ds_reg + first_slot, (size_t)n * sizeof(double), cudaMemcpyDefault, e->stream));
   CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  return CTD_OK;
+}
+
+// The incoming records are copied past the cursors, where no read reaches them, and ctd_k_dataset_append checks them, rebases their
+// option offsets and only then moves the cursors: a rejected append leaves the dataset as it was.
+ctd_status ctd_dataset_append(ctd_engine* e, uint32_t n_records, uint32_t n_option_slots, const float* features, const ctd_target_meta* meta,
+                              const ctd_record_origin* origin, const ctd_option* options, const double* regrets) {
+  if (!e || e->ds_max_records == 0 || (n_records && (!features || !meta || !origin)) || (n_option_slots && (!options || !regrets)))
+    return CTD_EARG;
+  if (n_records == 0 && n_option_slots == 0) return CTD_OK;
+  CtdDatasetCtr c;
+  ctd_status s = ctd_dataset_counts(e, &c);   // waits for every recording in flight
+  if (s != CTD_OK) return s;
+  if (c.n_records + n_records > e->ds_max_records || c.n_slots + n_option_slots > e->ds_max_slots) {
+    snprintf(e->err, sizeof(e->err), "ctd_dataset_append: %llu + %u records / %llu + %u option slots exceed the reservation (%u / %u)",
+             c.n_records, n_records, c.n_slots, n_option_slots, e->ds_max_records, e->ds_max_slots);
+    return CTD_ECAP;
+  }
+  CtdBuf<int> d_bad;
+  CTD_CUDA(e, d_bad.grow(sizeof(int)));
+  if (n_records) {
+    CTD_CUDA(e, cudaMemcpyAsync(e->ds_feat + (size_t)c.n_records * CTD_FEATURES_PAD, features, (size_t)n_records * CTD_FEATURES_PAD * sizeof(float),
+                                cudaMemcpyDefault, e->stream));
+    CTD_CUDA(e, cudaMemcpyAsync(e->ds_meta + c.n_records, meta, (size_t)n_records * sizeof(ctd_target_meta), cudaMemcpyDefault, e->stream));
+    CTD_CUDA(e, cudaMemcpyAsync(e->ds_origin + c.n_records, origin, (size_t)n_records * sizeof(ctd_record_origin), cudaMemcpyDefault, e->stream));
+  }
+  if (n_option_slots) {
+    CTD_CUDA(e, cudaMemcpyAsync(e->ds_opt + c.n_slots, options, (size_t)n_option_slots * sizeof(ctd_option), cudaMemcpyDefault, e->stream));
+    CTD_CUDA(e, cudaMemcpyAsync(e->ds_reg + c.n_slots, regrets, (size_t)n_option_slots * sizeof(double), cudaMemcpyDefault, e->stream));
+  }
+  ctd_k_dataset_append<<<1, CTD_APPEND_THREADS, 0, e->stream>>>(e->ds_meta, e->ds_origin, e->ds_ctr, n_records, n_option_slots, d_bad);
+  e->launches++;
+  CTD_CUDA(e, cudaGetLastError());
+  int bad = 0;
+  CTD_CUDA(e, cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, e->stream));
+  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
+  if (bad) {
+    snprintf(e->err, sizeof(e->err), "ctd_dataset_append: %s", bad & 1 ? "a record's option span is empty or outside the incoming slots"
+                                                                : bad & 2 ? "an origin's mover is not a seat" : "an origin's winner is not -1 or a seat");
+    return CTD_EARG;
+  }
   return CTD_OK;
 }
 

@@ -27,6 +27,7 @@ class Engine:
         self.capacity = int(capacity)
         self.device = int(device)
         self._model_arrays = {}
+        self._ds_cap = None   # (max_records, max_option_slots) of the dataset's reservation
 
     def close(self):
         if getattr(self, "_h", None):
@@ -156,35 +157,80 @@ class Engine:
     # ---- self-play dataset (filled by arena(record=...)) ----
     def dataset_reserve(self, max_records, max_option_slots):
         """Allocate the engine's dataset in HBM (max_records rows of 448 floats; max_option_slots options / regrets) and clear it."""
+        self._ds_cap = None
         self._check(self._lib.ctd_dataset_reserve(self._h, int(max_records), int(max_option_slots)), "ctd_dataset_reserve")
+        self._ds_cap = (int(max_records), int(max_option_slots))
 
     def dataset_clear(self):
         self._check(self._lib.ctd_dataset_clear(self._h), "ctd_dataset_clear")
 
     def dataset_info(self):
-        """-> dict(records, option_slots, dropped_trees, dropped_records): trees that did not fit are dropped whole."""
+        """-> dict(records, option_slots, dropped_trees, dropped_records, max_records, max_option_slots): trees that did not fit are
+        dropped whole; the last two are the reservation's."""
         nr, ns, dt, dr = ctypes.c_uint32(), ctypes.c_uint32(), ctypes.c_uint64(), ctypes.c_uint64()
         self._check(self._lib.ctd_dataset_info(self._h, ctypes.byref(nr), ctypes.byref(ns), ctypes.byref(dt), ctypes.byref(dr)),
                     "ctd_dataset_info")
-        return dict(records=nr.value, option_slots=ns.value, dropped_trees=dt.value, dropped_records=dr.value)
+        return dict(records=nr.value, option_slots=ns.value, dropped_trees=dt.value, dropped_records=dr.value,
+                    max_records=self._ds_cap[0], max_option_slots=self._ds_cap[1])
+
+    def _dataset_fill(self, n, ns, feats, meta, origin, opts, regs):
+        self._check(self._lib.ctd_dataset_read(self._h, 0, n, feats, meta, origin), "ctd_dataset_read")
+        self._check(self._lib.ctd_dataset_read_options(self._h, 0, ns, opts, regs), "ctd_dataset_read_options")
+
+    def dataset_arrays(self):
+        """The whole dataset in physical order, as dataset_append takes it: features[R, 448] f32, meta[R] (layout.TARGET_META_DTYPE),
+        origin[R] (layout.ORIGIN_DTYPE), options[S] u64, regrets[S] f64."""
+        info = self.dataset_info()
+        n, ns = info["records"], info["option_slots"]
+        a = dict(features=np.zeros((n, 448), dtype=np.float32), meta=np.zeros(n, dtype=TARGET_META_DTYPE),
+                 origin=np.zeros(n, dtype=ORIGIN_DTYPE), options=np.zeros(ns, dtype=np.uint64), regrets=np.zeros(ns, dtype=np.float64))
+        self._dataset_fill(n, ns, *(a[k].ctypes.data for k in DATASET_KEYS))
+        return a
+
+    def dataset_tensors(self, device):
+        """dataset_arrays as torch tensors on CUDA device `device`, copied device to device: features[R, 448] f32, meta[R, 72] and
+        origin[R, 24] u8 (the bytes of the two records), options[S] u64, regrets[S] f64."""
+        import torch
+        dev = torch.device(device)
+        if dev.type != "cuda":
+            raise ValueError("dataset_tensors fills CUDA tensors, got device %r" % (device,))
+        info = self.dataset_info()
+        n, ns = info["records"], info["option_slots"]
+        t = dict(features=torch.empty((n, 448), dtype=torch.float32, device=dev),
+                 meta=torch.empty((n, TARGET_META_DTYPE.itemsize), dtype=torch.uint8, device=dev),
+                 origin=torch.empty((n, ORIGIN_DTYPE.itemsize), dtype=torch.uint8, device=dev),
+                 options=torch.empty(ns, dtype=torch.uint64, device=dev), regrets=torch.empty(ns, dtype=torch.float64, device=dev))
+        torch.cuda.current_stream(dev).synchronize()   # the engine writes on its own stream: nothing of torch's may still use the memory
+        self._dataset_fill(n, ns, *(t[k].data_ptr() for k in DATASET_KEYS))
+        return t
+
+    def dataset_append(self, features, meta, origin, options, regrets):
+        """Append records after the dataset's own (ctd_dataset_append), from numpy arrays or torch CUDA tensors on any device, laid
+        out as dataset_arrays / dataset_tensors return them (features with 418 columns are zero-padded to 448; meta and origin may
+        also be their raw bytes).  option_offset indexes `options` and is rebased; tree and origin are kept.  All or nothing:
+        EngineError with status 3 when the reservation is too small, 1 for a malformed record, and the dataset is unchanged."""
+        arrs = [_append_input(x, k) for x, k in zip((features, meta, origin, options, regrets), DATASET_KEYS)]
+        (f, nf), (m, n), (o, no), (x, ns), (r, nr) = arrs
+        if nf != n or no != n or nr != ns:
+            raise ValueError("dataset_append: %d feature rows, %d metas, %d origins, %d options, %d regrets" % (nf, n, no, ns, nr))
+        tensors = [a for a, _ in arrs if not isinstance(a, np.ndarray)]
+        for d in {t.device for t in tensors}:
+            import torch
+            torch.cuda.current_stream(d).synchronize()   # the producing work must be complete: the engine copies on its own stream
+        ptr = [a.ctypes.data if isinstance(a, np.ndarray) else a.data_ptr() for a in (f, m, o, x, r)]
+        self._check(self._lib.ctd_dataset_append(self._h, n, ns, *ptr), "ctd_dataset_append")
 
     def dataset_read(self):
         """Every record of the dataset in canonical order (origin gid, search, then pre-order within the tree): features[R, 418] f32,
         meta[R] (tree: the game's index in its arena call; option_offset into options / regrets), origin[R] (layout.ORIGIN_DTYPE),
         row[R] (the record's physical row, what train_on_dataset's indices name), and every option slot: options[S] u64, regrets[S]
         f64.  Engine.targets_as_tuples accepts the result as it is."""
-        info = self.dataset_info()
-        n, ns = info["records"], info["option_slots"]
-        feats = np.zeros((n, 448), dtype=np.float32)
-        meta = np.zeros(n, dtype=TARGET_META_DTYPE)
-        origin = np.zeros(n, dtype=ORIGIN_DTYPE)
-        opts = np.zeros(ns, dtype=np.uint64)
-        regs = np.zeros(ns, dtype=np.float64)
-        self._check(self._lib.ctd_dataset_read(self._h, 0, n, feats.ctypes.data, meta.ctypes.data, origin.ctypes.data), "ctd_dataset_read")
-        self._check(self._lib.ctd_dataset_read_options(self._h, 0, ns, opts.ctypes.data, regs.ctypes.data), "ctd_dataset_read_options")
+        a = self.dataset_arrays()
+        origin = a["origin"]
         # a tree's records are consecutive in pre-order, so the physical row orders them within (gid, search)
-        row = np.lexsort((np.arange(n), origin["search"], origin["gid"])).astype(np.int64)
-        return dict(features=feats[row, :418], meta=meta[row], origin=origin[row], row=row, options=opts, regrets=regs)
+        row = np.lexsort((np.arange(len(origin)), origin["search"], origin["gid"])).astype(np.int64)
+        return dict(features=a["features"][row, :418], meta=a["meta"][row], origin=origin[row], row=row, options=a["options"],
+                    regrets=a["regrets"])
 
     def playout_slots(self, n, max_steps=4096):
         winner = np.empty(n, dtype=np.int8)
@@ -342,6 +388,39 @@ class Engine:
     @property
     def launches(self):
         return int(self._lib.ctd_launch_count(self._h))
+
+
+DATASET_KEYS = ("features", "meta", "origin", "options", "regrets")
+# per input of dataset_append: (numpy dtypes, torch dtype names, bytes per item)
+_APPEND_TYPES = dict(features=((np.float32,), ("float32",), 4 * 448),
+                     meta=((TARGET_META_DTYPE, np.uint8), ("uint8",), TARGET_META_DTYPE.itemsize),
+                     origin=((ORIGIN_DTYPE, np.uint8), ("uint8",), ORIGIN_DTYPE.itemsize),
+                     options=((np.uint64, np.int64), ("uint64", "int64"), 8),
+                     regrets=((np.float64,), ("float64",), 8))
+
+
+def _append_input(a, key):
+    """One input of Engine.dataset_append -> (contiguous numpy array or CUDA tensor, item count); features of 418 columns padded."""
+    np_types, t_types, item = _APPEND_TYPES[key]
+    if isinstance(a, np.ndarray) or not hasattr(a, "data_ptr"):
+        a = np.ascontiguousarray(a)
+        if key == "features" and a.ndim == 2 and a.shape[1] == 418:
+            a = np.pad(a, ((0, 0), (0, 448 - 418)))
+        ok, nbytes = any(a.dtype == np.dtype(t) for t in np_types), a.nbytes
+    else:
+        if not a.is_cuda:
+            raise ValueError("dataset_append takes numpy arrays or CUDA tensors, got a tensor on %s" % a.device)
+        if key == "features" and a.dim() == 2 and a.shape[1] == 418:
+            import torch
+            a = torch.nn.functional.pad(a, (0, 448 - 418))
+        a = a.contiguous()
+        ok, nbytes = str(a.dtype).replace("torch.", "") in t_types, a.numel() * a.element_size()
+    if key == "features" and (len(a.shape) != 2 or a.shape[1] != 448):
+        ok = False
+    if not ok or nbytes % item:
+        raise ValueError("dataset_append: %s of dtype %s and shape %s is not what dataset_arrays returns"
+                         % (key, a.dtype, tuple(a.shape)))
+    return a, nbytes // item
 
 
 def stats_dict(s):

@@ -10,6 +10,12 @@ The arena records the targets of its searches into a dataset the engine keeps in
 trees are counted, given rows on the device and written out, and each record's game outcome is filled in when the call ends.
 Training gathers its rows from that dataset on the device (ctd_train_begin_dataset); only the index lists cross to the device.
 
+On several GPUs (torchrun, one rank per GPU) every rank records its own block of games into its own engine, gather_dataset
+appends all of them to one rank's dataset (NCCL: device to device, the records never touch the host) and that rank trains as
+above.  The training step is bound by launch latency, so one GPU training on everything is as fast as several sharing the work,
+and the semantics stay those of one engine.  save_dataset / load_dataset keep a dataset in an .npz beyond its engine, so a round
+can be trained again or appended to a later round's records.
+
 Which records, which labels.  The reference trains on CFRNode.get_all_targets(15) of pure-MCCFR trees, labelled with node_value.
 A deep seat's tree is different: in eval mode a node's node_value is written only on its first backprop, so it sums to the reward
 weight (5) or to 1 at a terminal and never reaches 15 -- tree mode at the reference's threshold records nothing from it -- and what
@@ -22,11 +28,13 @@ import math
 
 import numpy as np
 
-from .engine import Engine, DEFAULT_SEED, RULESET_PRESET
-from .layout import RECORD_TREE, RECORD_ROOT, LABEL_NODE_VALUE, LABEL_WINNER
+from .engine import Engine, DEFAULT_SEED, RULESET_PRESET, DATASET_KEYS
+from .layout import RECORD_TREE, RECORD_ROOT, LABEL_NODE_VALUE, LABEL_WINNER, TARGET_META_DTYPE, ORIGIN_DTYPE
 
 MODES = {"tree": RECORD_TREE, "root": RECORD_ROOT}
 LABELS = {"node_value": LABEL_NODE_VALUE, "winner": LABEL_WINNER}
+DATASET_FORMAT = 1   # save_dataset's .npz layout
+COUNT_KEYS = ("records", "option_slots", "dropped_trees", "dropped_records")
 
 
 def _code(value, names, what):
@@ -79,6 +87,109 @@ def record_arena(n_games, seats, record_seats, models=None, mode="root", thresho
         if own:
             eng.close()
     return out
+
+
+def _item_bytes(key, n_records, n_slots):
+    return {"features": 448 * 4 * n_records, "meta": TARGET_META_DTYPE.itemsize * n_records,
+            "origin": ORIGIN_DTYPE.itemsize * n_records, "options": 8 * n_slots, "regrets": 8 * n_slots}[key]
+
+
+def _from_bytes(key, b, n_records):
+    """A received byte buffer (torch CUDA tensor or numpy array) -> the layout dataset_append takes."""
+    if isinstance(b, np.ndarray):
+        dt = {"features": np.float32, "meta": TARGET_META_DTYPE, "origin": ORIGIN_DTYPE, "options": np.uint64, "regrets": np.float64}
+        a = b.view(dt[key])
+        return a.reshape(n_records, 448) if key == "features" else a
+    import torch
+    if key == "features":
+        return b.view(torch.float32).view(n_records, 448)
+    if key in ("meta", "origin"):
+        return b.view(n_records, -1)
+    return b.view(torch.int64 if key == "options" else torch.float64)
+
+
+def gather_dataset(engine, dst=0, group=None):
+    """Collective over `group` (default: the default process group): every rank calls it with its own engine.  The datasets of all
+    ranks but `dst` are appended to `dst`'s (Engine.dataset_append), in rank order, so that dst holds its own records followed by
+    those of the other ranks; their datasets are left as they are.  The ranks' counts and dst's reservation are all_gathered first,
+    so every rank reaches the same verdict: when the records or option slots do not fit dst's reservation, every rank raises the
+    same ValueError and nothing is appended.  Then one rank at a time sends its physical-order dataset to dst (point to point,
+    which bounds dst's staging memory to one rank's records): with NCCL as CUDA tensors (Engine.dataset_tensors), so the records
+    never touch the host; with gloo as host arrays (Engine.dataset_arrays).  Game ids of different ranks are disjoint (play_arena's
+    rank blocks), so dataset_read's canonical order and split_by_game work on the merged dataset as they are.  A single process:
+    nothing to do.  -> dict(records, option_slots, dropped_trees, dropped_records): one entry per rank, as the datasets stood
+    before the gather."""
+    import torch
+    import torch.distributed as dist
+    info = engine.dataset_info()
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return {k: [info[k]] for k in COUNT_KEYS}
+    rank, world = dist.get_rank(group), dist.get_world_size(group)
+    if not 0 <= int(dst) < world:
+        raise ValueError("dst must be a rank of the group (0 .. %d), got %r" % (world - 1, dst))
+    dst = int(dst)
+    nccl = dist.get_backend(group) == "nccl"
+    dev = torch.device("cuda", engine.device) if nccl else torch.device("cpu")
+    mine = torch.tensor([info[k] for k in COUNT_KEYS + ("max_records", "max_option_slots")], dtype=torch.int64, device=dev)
+    every = [torch.empty_like(mine) for _ in range(world)]
+    dist.all_gather(every, mine, group=group)
+    every = [[int(x) for x in t.tolist()] for t in every]
+    counts = {k: [c[i] for c in every] for i, k in enumerate(COUNT_KEYS)}
+    recs, slots = counts["records"], counts["option_slots"]
+    cap_r, cap_s = every[dst][4], every[dst][5]
+    if sum(recs) > cap_r or sum(slots) > cap_s:
+        raise ValueError("gather_dataset: %d records and %d option slots over %d ranks do not fit rank %d's reservation of %d and %d"
+                         % (sum(recs), sum(slots), world, dst, cap_r, cap_s))
+    for src in range(world):
+        if src == dst or (recs[src] == 0 and slots[src] == 0) or rank not in (src, dst):
+            continue
+        sizes = {k: _item_bytes(k, recs[src], slots[src]) for k in DATASET_KEYS}
+        if rank == src:
+            parts = engine.dataset_tensors(dev) if nccl else engine.dataset_arrays()
+            for k in DATASET_KEYS:
+                if sizes[k]:
+                    p = parts[k]
+                    b = p.view(torch.uint8).reshape(-1) if nccl else torch.from_numpy(np.ascontiguousarray(p).view(np.uint8).reshape(-1))
+                    dist.send(b, group=group, group_dst=dst)
+            if nccl:
+                torch.cuda.current_stream(dev).synchronize()   # the sends have read the tensors before they are freed
+        else:
+            got = {}
+            for k in DATASET_KEYS:
+                b = torch.empty(sizes[k], dtype=torch.uint8, device=dev)
+                if sizes[k]:
+                    dist.recv(b, group=group, group_src=src)
+                got[k] = _from_bytes(k, b if nccl else b.numpy(), recs[src])
+            engine.dataset_append(*(got[k] for k in DATASET_KEYS))
+    return counts
+
+
+def save_dataset(engine, path):
+    """The engine's dataset, in physical order, to an .npz (np.savez: `path` gains .npz unless it has it) with its format version:
+    features [R, 448] f32, meta [R, 72] and origin [R, 24] as bytes, options [S] u64, regrets [S] f64.  -> dict(records, option_slots)"""
+    a = engine.dataset_arrays()
+    n = len(a["meta"])
+    np.savez(path, format_version=np.int64(DATASET_FORMAT), features=a["features"], meta=a["meta"].view(np.uint8).reshape(n, -1),
+             origin=a["origin"].view(np.uint8).reshape(n, -1), options=a["options"], regrets=a["regrets"])
+    return dict(records=n, option_slots=len(a["options"]))
+
+
+def load_dataset(engine, path):
+    """Append the records of a save_dataset file to the engine's reserved dataset (Engine.dataset_append: their option offsets are
+    rebased, trees and origins kept).  ValueError when the file is not of this format or does not fit the reservation (nothing is
+    appended); EngineError when no dataset is reserved.  -> dict(records, option_slots) appended."""
+    with np.load(path, allow_pickle=False) as z:
+        if "format_version" not in z.files or int(z["format_version"]) != DATASET_FORMAT:
+            raise ValueError("%s is not a dataset of format %d (save_dataset)" % (path, DATASET_FORMAT))
+        a = {k: z[k] for k in DATASET_KEYS}
+    meta, origin = a["meta"].reshape(-1).view(TARGET_META_DTYPE), a["origin"].reshape(-1).view(ORIGIN_DTYPE)
+    n, ns = len(meta), len(a["options"])
+    info = engine.dataset_info()
+    if info["records"] + n > info["max_records"] or info["option_slots"] + ns > info["max_option_slots"]:
+        raise ValueError("%s: %d records and %d option slots do not fit the dataset (%d + %d of %d, %d + %d of %d)"
+                         % (path, n, ns, info["records"], n, info["max_records"], info["option_slots"], ns, info["max_option_slots"]))
+    engine.dataset_append(a["features"], meta, origin, a["options"], a["regrets"])
+    return dict(records=n, option_slots=ns)
 
 
 def split_by_game(origin, val_fraction, seed, rows=None):

@@ -396,7 +396,10 @@ ctd_status ctd_arena(ctd_engine* e, uint64_t n_games, uint64_t seed, uint64_t fi
  * option slots.  Records of one tree are consecutive in pre-order; trees are appended in no fixed order (the arena queues its games
  * with atomics), so the canonical order is (origin.gid, origin.search, row).
  * Capacity is enforced on the device: the trees of a search are kept in queue order while all their records and option slots fit;
- * a tree that does not fit is dropped whole and counted. */
+ * a tree that does not fit is dropped whole and counted.
+ * Records added by ctd_dataset_append (another engine's, or a saved dataset's) follow the ones already held.  Their tree stays
+ * what it was in the call that recorded them, their origin is kept as given, and their option_offset is rebased to index this
+ * dataset's option slots. */
 typedef struct ctd_record_origin {
   uint64_t gid;          /* the game: ctd_game_new(seed, gid, ruleset) */
   uint32_t search;       /* the game's search number t: the tree id is (gid & (2^40 - 1)) | t << 40 */
@@ -424,11 +427,25 @@ ctd_status ctd_dataset_clear(ctd_engine* e);
 /* records and option slots held, trees and records dropped for want of room since the last reserve / clear (outputs may be NULL) */
 ctd_status ctd_dataset_info(ctd_engine* e, uint32_t* n_records, uint32_t* n_option_slots, uint64_t* dropped_trees,
                             uint64_t* dropped_records);
-/* records [first, first + n): features [n][448] f32, meta, origin (outputs may be NULL); first + n > n_records: CTD_EARG */
+/* records [first, first + n): features [n][448] f32, meta, origin (outputs may be NULL); first + n > n_records: CTD_EARG.
+ * The outputs may be host memory or device memory on any GPU (the copies use cudaMemcpyDefault); the call returns once they are
+ * written. */
 ctd_status ctd_dataset_read(ctd_engine* e, uint32_t first, uint32_t n, float* features, ctd_target_meta* meta,
                             ctd_record_origin* origin);
-/* option slots [first_slot, first_slot + n): descriptors and regrets (outputs may be NULL); beyond n_option_slots: CTD_EARG */
+/* option slots [first_slot, first_slot + n): descriptors and regrets (outputs may be NULL, host or device memory as for
+ * ctd_dataset_read); beyond n_option_slots: CTD_EARG */
 ctd_status ctd_dataset_read_options(ctd_engine* e, uint32_t first_slot, uint32_t n, ctd_option* options, double* regrets);
+/* Append n_records records and n_option_slots option slots after the dataset's own: features [n_records][448] f32, meta, origin,
+ * options and regrets [n_option_slots], laid out as ctd_dataset_read / ctd_dataset_read_options return them.  Every input may be
+ * host memory or device memory on any GPU (cudaMemcpyDefault); device inputs must be complete when the call is made.  Each
+ * meta.option_offset indexes the incoming options and is rebased by the dataset's n_option_slots; meta.tree and origin are kept
+ * as given; the drop counts are not changed.  All or nothing: on any error the dataset is left as it was.
+ * CTD_ECAP: the records or the slots do not fit the reservation.  CTD_EARG: no dataset reserved, a NULL input with n_records > 0
+ * (options / regrets: with n_option_slots > 0), a meta with n_options == 0 or option_offset + n_options > n_option_slots, an origin
+ * with mover > 5 or winner outside [-1, 5].  n_records == n_option_slots == 0 on a reserved dataset does nothing. */
+ctd_status ctd_dataset_append(ctd_engine* e, uint32_t n_records, uint32_t n_option_slots, const float* features,
+                              const ctd_target_meta* meta, const ctd_record_origin* origin, const ctd_option* options,
+                              const double* regrets);
 /* ctd_arena with recording.  rec: which seats, which mode, which threshold; CTD_EARG for a NULL rec, seat-mask bits above 5, an
  * unknown mode, a negative or NaN threshold, or no dataset reserved.  elapsed_ms (may be NULL) receives four CUDA-event times: the
  * three of ctd_arena and the recording (count, reserve and fill kernels per search, the outcome kernel at the end). */
