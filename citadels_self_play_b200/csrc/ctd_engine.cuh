@@ -22,8 +22,6 @@
 #define CTD_NI __noinline__
 #define CTD_LOOP _Pragma("unroll 1")
 #define CTD_UNROLL _Pragma("unroll")
-#define CTD_LOOP_HOT4 _Pragma("unroll 1")
-#define CTD_LOOP_HOTFULL _Pragma("unroll 1")
 #elif defined(__CUDACC__)
 #define CTD_HD __host__ __device__
 // out-of-line on the device: the playout kernel's warps sit at unrelated points of the rules code, so the
@@ -31,25 +29,16 @@
 #define CTD_NI __noinline__
 #define CTD_LOOP _Pragma("unroll 1")
 #define CTD_UNROLL _Pragma("unroll")
-#ifdef CTD_HOT_UNROLL   /* experiment: fewer taken branches in the hottest tiny loops */
-#define CTD_LOOP_HOT4 _Pragma("unroll 4")
-#define CTD_LOOP_HOTFULL _Pragma("unroll")
-#else
-#define CTD_LOOP_HOT4 _Pragma("unroll 1")
-#define CTD_LOOP_HOTFULL _Pragma("unroll 1")
-#endif
 #else
 #define CTD_HD
 #define CTD_NI
 #define CTD_LOOP
 #define CTD_UNROLL
-#define CTD_LOOP_HOT4
-#define CTD_LOOP_HOTFULL
 #endif
 // On the device every CtdWork / CtdKnow lives in shared memory (all kernels declare them __shared__).  Telling the
 // compiler turns the generic LD.E / ST.E (+ descriptor moves and 64-bit address arithmetic) of the out-of-line rules code
 // into LDS / STS with immediate offsets.
-#if defined(__CUDA_ARCH__) && !defined(CTD_NO_ASSUME_SHARED)
+#if defined(__CUDA_ARCH__)
 #define CTD_ASSUME_SHARED(p) __builtin_assume(__isShared(p))
 #define CTD_ASSUME_GLOBAL(p) __builtin_assume(__isGlobal(p))
 #else
@@ -75,12 +64,6 @@
 #define CTD_NOT_CLASSIC() __builtin_unreachable()
 #else
 #define CTD_NOT_CLASSIC() ((void)0)
-#endif
-#ifndef CTD_PLAYOUT_RING
-/* 1 = the fused playout computes 32 Philox blocks at a time, one per lane (ctd_warp.cuh ctd_ring_refill): 40 fewer warp
- * instructions per env step (7 %) and bit-identical results, but no faster on B200 -- the kernel is bound by instruction
- * fetch, not by issue slots (profiles/README.md, round-1 A/B table) -- so the simpler lane-0 stream is the default. */
-#define CTD_PLAYOUT_RING 0
 #endif
 // Container capacities.  The fused playout units (ctd_*_playout.cu) define CTD_SMALL_CAPS: real games of the fixed rulesets
 // stay far below them (hand 25, city 9, museum 14, just_drawn 33 over 5e5 games) and the working record is what occupies
@@ -214,9 +197,7 @@ struct alignas(16) CtdWork {
   uint32_t draws;
   uint32_t buf[4];
   uint32_t buf_blk;
-  // playout kernel only: 32 Philox blocks computed one per lane (ctd_ring_refill in ctd_warp.cuh); ring[(b & 31) * 4 ..] holds
-  // block b for b in [ring_hi - 32, ring_hi).  ring == nullptr everywhere else (lane 0 computes blocks one at a time).
-  uint32_t* ring;
+  uint32_t* ring;     // unused; kept so that the kernels' shared-memory layout and code stay unchanged
   uint32_t ring_hi;
   const uint8_t* tape;
   uint32_t tape_pos, tape_len;
@@ -229,7 +210,7 @@ static_assert(offsetof(CtdWork, scratch) == CTD_SNAP_BYTES && CTD_SNAP_BYTES % 1
 // ------------------------------------------------------------------------------------------ chance
 CTD_HD CTD_NI inline void ctd_philox(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1,
                               uint32_t out[4]) {
-  CTD_LOOP_HOTFULL for (int i = 0; i < 10; ++i) {
+  CTD_LOOP for (int i = 0; i < 10; ++i) {
     uint64_t p0 = (uint64_t)0xD2511F53u * c0;
     uint64_t p1 = (uint64_t)0xCD9E8D57u * c2;
     uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ k0;
@@ -251,21 +232,11 @@ CTD_HD inline void ctd_chance_init(CtdWork& w, uint64_t seed, uint64_t gid, uint
   w.stream = 0;
   w.buf_blk = 0xFFFFFFFFu;
   w.tape = nullptr; w.tape_pos = 0; w.tape_len = 0;
-  w.ring = nullptr; w.ring_hi = 0;
+  w.ring = nullptr; w.ring_hi = 0;   // kept so that the kernels' code stays unchanged
 }
 
-#ifndef CTD_U32_ATTR
-#if CTD_PLAYOUT_RING
-#define CTD_U32_ATTR CTD_NI /* one copy of the ring test + block refill */
-#else
-#define CTD_U32_ATTR
-#endif
-#endif
-CTD_HD CTD_U32_ATTR inline uint32_t ctd_u32(CtdWork& w) {
+CTD_HD inline uint32_t ctd_u32(CtdWork& w) {
   uint32_t blk = w.draws >> 2;
-#if CTD_PLAYOUT_RING
-  if (w.ring != nullptr && w.ring_hi - 1u - blk < 32u) return w.ring[((blk & 31u) << 2) | (w.draws++ & 3u)];
-#endif
   if (blk != w.buf_blk) {
     ctd_philox(blk, w.stream, w.g0, w.g1, w.k0, w.k1, w.buf);
     w.buf_blk = blk;
@@ -300,35 +271,6 @@ CTD_HD inline void ctd_shuffle(CtdWork& w, int n, At at) {
     w.tape_pos += n;
     return;
   }
-#if defined(__CUDA_ARCH__) && defined(CTD_COOP_SHUFFLE)
-  // Search kernels: the whole warp runs this code converged.  The draws of a shuffle are known in advance (draw k bounds
-  // i = n-1-k), so 32 of them are produced at once -- every lane runs Philox for the block holding its draw and reduces it to a
-  // swap index -- and only the swaps themselves stay sequential.  Same draws, same order, same result as the loop below.
-  if (n >= 12 && __activemask() == 0xFFFFFFFFu) {
-    const int lane = threadIdx.x & 31;
-    int i = n - 1;
-    CTD_LOOP while (i > 0) {
-      const int cnt = i < 32 ? i : 32;               // swaps of this batch: i, i-1, ..., i-cnt+1
-      __syncwarp();
-      if (lane < cnt) {
-        const uint32_t dr = w.draws + (uint32_t)lane;
-        uint32_t r[4];
-        ctd_philox(dr >> 2, w.stream, w.g0, w.g1, w.k0, w.k1, r);
-        w.scratch[lane] = (uint8_t)(((uint64_t)r[dr & 3u] * (uint32_t)(i - lane + 1)) >> 32);
-      }
-      __syncwarp();
-      CTD_LOOP for (int k = 0; k < cnt; ++k) {
-        const int j = w.scratch[k];
-        const uint8_t a = at(i - k), b = at(j);
-        at(i - k) = b; at(j) = a;
-      }
-      __syncwarp();
-      w.draws += (uint32_t)cnt;
-      i -= cnt;
-    }
-    return;
-  }
-#endif
   CTD_LOOP for (int i = n - 1; i > 0; --i) {
     int j = (int)ctd_randbelow(w, (uint32_t)(i + 1));
     uint8_t a = at(i), b = at(j);
@@ -450,29 +392,29 @@ CTD_HD inline void ctd_kn_confirm(CtdKnowSet ks, int seat, int role) {
 
 // ------------------------------------------------------------------------------------------ list helpers
 CTD_HD CTD_NI inline bool ctd_has(const uint8_t* a, int n, int t) {
-  CTD_LOOP_HOT4 for (int i = 0; i < n; ++i) if (ctd_ctype(a[i]) == t) return true;
+  CTD_LOOP for (int i = 0; i < n; ++i) if (ctd_ctype(a[i]) == t) return true;
   return false;
 }
 CTD_HD CTD_NI inline int ctd_count_type(const uint8_t* a, int n, int t) {
   int k = 0;
-  CTD_LOOP_HOT4 for (int i = 0; i < n; ++i) k += ctd_ctype(a[i]) == t;
+  CTD_LOOP for (int i = 0; i < n; ++i) k += ctd_ctype(a[i]) == t;
   return k;
 }
 CTD_HD CTD_NI inline int ctd_count_suit(const uint8_t* a, int n, int s) {
   int k = 0;
-  CTD_LOOP_HOT4 for (int i = 0; i < n; ++i) k += ctd_csuit(a[i]) == s;
+  CTD_LOOP for (int i = 0; i < n; ++i) k += ctd_csuit(a[i]) == s;
   return k;
 }
 CTD_HD inline int ctd_remove_at(uint8_t* a, uint8_t& n, int i) {
   int c = a[i];
-  CTD_LOOP_HOT4 for (int k = i; k + 1 < n; ++k) a[k] = a[k + 1];
+  CTD_LOOP for (int k = i; k + 1 < n; ++k) a[k] = a[k + 1];
   --n;
   return c;
 }
 // Deck.get_a_card_like_it (game/deck.py:49-55): first card of that type; the requested card is fabricated
 // when none matches.
 CTD_HD CTD_NI inline int ctd_take_like(uint8_t* a, uint8_t& n, int t) {
-  CTD_LOOP_HOT4 for (int i = 0; i < n; ++i)
+  CTD_LOOP for (int i = 0; i < n; ++i)
     if (ctd_ctype(a[i]) == t) return ctd_remove_at(a, n, i);
   return t;
 }
@@ -1918,6 +1860,6 @@ CTD_HD CTD_NI inline void ctd_unpack(const ctd_state* s, CtdWork& w) {
   w.seer_mask = s->seer_mask; w.n_seven = s->seven_n > 7 ? 7 : s->seven_n;
   CTD_LOOP for (int i = 0; i < 7; ++i) w.seven[i] = s->seven[i];
   w.draws = s->rng_draws; w.buf_blk = 0xFFFFFFFFu; w.tape_pos = s->tape_pos; w.steps = s->steps;
-  w.ring = nullptr; w.ring_hi = 0;
+  w.ring = nullptr; w.ring_hi = 0;   // kept so that the kernels' code stays unchanged
   w.g0 = (uint32_t)s->gid; w.g1 = (uint32_t)(s->gid >> 32);
 }

@@ -610,17 +610,14 @@ struct CtdTrainer {
 };
 
 // one value model as the engine holds it (ctd_set_value_model_slot): the fused search and the fp32 kernel read the BN-folded
-// [in][out] weights, the tcgen05 kernels their [out][in] copy or, by TMA, its split TF32 terms
+// [in][out] weights, the tcgen05 kernels, by TMA, their split TF32 terms
 struct CtdValueSlot {
   bool ready;              // the last load completed
   CtdBuf<float> d_model;   // BN folded, transposed
   CtdValueModel model;
-  CtdBuf<float> d_model_tc;
-  const float *tc_w1, *tc_w2, *tc_w3;
   // the weights pre-split into their three TF32 terms, [3][N][K] per layer, and their tensor maps (TMA loads of the B operand)
   CtdBuf<float> d_wsplit;
   CUtensorMap tmap[3];
-  bool tmap_ok;
 };
 
 #define CTD_MAX_ARENAS 6
@@ -673,7 +670,7 @@ struct ctd_engine {
   // tensor-core path of the value model: activations between layers, error flag
   CtdBuf<float> d_h1, d_h2, d_h3;
   CtdBuf<int> d_tc_err;
-  int value_backend;  // batched evaluations: 0 = fp32 CUDA cores (ctd_k_value_mlp), 1 = tcgen05 split-TF32 (ctd_k_linear_tc)
+  int value_backend;  // batched evaluations: 0 = fp32 CUDA cores (ctd_k_value_mlp), 1 = tcgen05 split-TF32 (ctd_k_linear_tc_tma)
   int fused;          // deep MCCFR: 1 = one launch, every warp evaluates its own leaves (ctd_value_inline); 0 = waves + batched evaluation
   CtdBuf<uint8_t, true> h_pinned;        // pinned host staging for result copies
   std::unique_ptr<CtdTrainer> trainer;   // value-network training (ctd_train_*), created on first use
@@ -1181,11 +1178,9 @@ static ctd_status ctd_deep_pass(ctd_engine* e, const CtdSearch& sp, const uint32
   a.roots = e->d_slots; a.knows = e->d_knows; a.used_cards = e->d_used_cards; a.gids = e->d_gids;
   a.seed = sp.seed; a.iterations = sp.iterations; a.n0_log2 = ctd_n0_log2(sp.iterations); a.hdrs = e->d_hdrs; a.arena = ctd_arena_of(e, ai);
   a.results = e->d_results; a.n_epool = e->d_n_epool;
-  {  // wave budget: trees that never reach the depth limit would otherwise walk all their iterations in the first wave
-    const char* env = getenv("CTD_PRED_BUDGET");
-    p.budget = env ? (uint32_t)strtoul(env, nullptr, 10) : 20u;   // measured best at 4096 roots x 200 iterations (8: 8.4e6, 20: 1.12e7, 64: 8.9e6, unbounded: 7.3e6 it/s)
-    if (p.budget == 0) p.budget = 0xFFFFFFFFu;
-  }
+  // wave budget: trees that never reach the depth limit would otherwise walk all their iterations in the first wave
+  const uint32_t wave_budget = 20;   // measured best at 4096 roots x 200 iterations (8: 8.4e6, 20: 1.12e7, 64: 8.9e6, unbounded: 7.3e6 it/s)
+  p.budget = wave_budget;
   p.max_depth = sp.max_depth; p.feat = e->d_feat; p.pred = e->d_pred; p.pending = e->d_pending;
   CtdPersistent<CtdPredArgs> k{e->sm_count, 0, nullptr};
   CTD_CUDA(e, ctd_pred_kernel(sp.ruleset, e->fused, k));
@@ -1209,8 +1204,7 @@ static ctd_status ctd_deep_pass(ctd_engine* e, const CtdSearch& sp, const uint32
   // Two groups of trees take turns: each group's waves (walk kernel -> batched leaf evaluation -> walk kernel ...) run on
   // their own stream, so the tail of one group's wave -- a few trees with expensive expansions -- overlaps with the other
   // group's kernel instead of idling the GPU.  Trees are independent, results do not depend on the grouping.
-  const char* genv = getenv("CTD_PRED_GROUPS");
-  const int G = (genv ? atoi(genv) : 2) >= 2 && n >= 1024 ? 2 : 1;
+  const int G = n >= 1024 ? 2 : 1;
   if (G == 2 && !e->ev_join) {   // the join event comes last: a failure part way is completed by the next call
     if (!e->stream2) CTD_CUDA(e, cudaStreamCreateWithFlags(&e->stream2, cudaStreamNonBlocking));
     CTD_CUDA(e, e->d_counter2.grow(sizeof(unsigned long long)));
@@ -1611,7 +1605,6 @@ static ctd_status ctd_pred_buffers(ctd_engine* e) {
   CTD_CUDA(e, cudaMemsetAsync(e->d_pred, 0, n * 8 * sizeof(float), e->stream));
   CTD_CUDA(e, cudaMemsetAsync(e->d_pending, 0, n, e->stream));
   CTD_CUDA(e, cudaFuncSetAttribute(ctd_k_value_mlp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CTD_MLP_SMEM));
-  CTD_CUDA(e, cudaFuncSetAttribute(ctd_k_linear_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CTD_TC_SMEM));
   CTD_CUDA(e, cudaFuncSetAttribute(ctd_k_linear_tc_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CTD_TC_SMEM));
   CTD_CUDA(e, e->d_h1.grow(n * 512 * sizeof(float)));
   CTD_CUDA(e, e->d_h2.grow(n * 256 * sizeof(float)));
@@ -1638,19 +1631,10 @@ static ctd_status ctd_value_forward(ctd_engine* e, const CtdValueSlot& vm, uint3
   }
   float *h1 = e->d_h1 + (size_t)row0 * 512, *h2 = e->d_h2 + (size_t)row0 * 256, *h3 = e->d_h3 + (size_t)row0 * 128;
   const int M = (int)n, gm = (M + CTD_TC_BM - 1) / CTD_TC_BM;
-  if (vm.tmap_ok) {   // weight operand by TMA from the pre-split terms
-    ctd_k_linear_tc_tma<<<dim3(gm, 512 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(feat, CTD_FEATURES_PAD, vm.tmap[0], m.b1, h1, 512, M, CTD_FEATURES_PAD, 1, e->d_tc_err);
-    ctd_k_linear_tc_tma<<<dim3(gm, 256 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h1, 512, vm.tmap[1], m.b2, h2, 256, M, 512, 1, e->d_tc_err);
-    ctd_k_linear_tc_tma<<<dim3(gm, 128 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h2, 256, vm.tmap[2], m.b3, h3, 128, M, 256, 1, e->d_tc_err);
-    ctd_k_value_head<<<(n + 127) / 128, 128, 0, st>>>(h3, m.w4t, m.b4, pending, n, pred, weight);
-    e->launches += 4;
-    CTD_CUDA(e, cudaGetLastError());
-    return CTD_OK;
-  }
-  ctd_k_linear_tc<<<dim3(gm, 512 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(feat, CTD_FEATURES_PAD, vm.tc_w1, CTD_FEATURES_PAD, m.b1, h1, 512,
-                                                                       M, CTD_FEATURES_PAD, 1, e->d_tc_err);
-  ctd_k_linear_tc<<<dim3(gm, 256 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h1, 512, vm.tc_w2, 512, m.b2, h2, 256, M, 512, 1, e->d_tc_err);
-  ctd_k_linear_tc<<<dim3(gm, 128 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h2, 256, vm.tc_w3, 256, m.b3, h3, 128, M, 256, 1, e->d_tc_err);
+  // weight operand by TMA from the pre-split terms
+  ctd_k_linear_tc_tma<<<dim3(gm, 512 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(feat, CTD_FEATURES_PAD, vm.tmap[0], m.b1, h1, 512, M, CTD_FEATURES_PAD, 1, e->d_tc_err);
+  ctd_k_linear_tc_tma<<<dim3(gm, 256 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h1, 512, vm.tmap[1], m.b2, h2, 256, M, 512, 1, e->d_tc_err);
+  ctd_k_linear_tc_tma<<<dim3(gm, 128 / CTD_TC_BN), 128, CTD_TC_SMEM, st>>>(h2, 256, vm.tmap[2], m.b3, h3, 128, M, 256, 1, e->d_tc_err);
   ctd_k_value_head<<<(n + 127) / 128, 128, 0, st>>>(h3, m.w4t, m.b4, pending, n, pred, weight);
   e->launches += 4;
   CTD_CUDA(e, cudaGetLastError());
@@ -1707,31 +1691,34 @@ ctd_status ctd_set_value_model_slot(ctd_engine* e, int slot, const float* w1t, c
     *dst[i] = p;
     p += pad[i];
   }
-  {  // tensor-core layout: [out][in] (the reference's own nn.Linear layout), BN already folded
+  {  // tensor-core layout: the static weights split into their TF32 terms once, and described to the TMA engine
     const size_t t1 = (size_t)512 * CTD_FEATURES_PAD, t2 = (size_t)256 * 512, t3 = (size_t)128 * 256;
+    CTD_CUDA(e, v.d_wsplit.grow(3 * (t1 + t2 + t3) * sizeof(float)));
+    float* sp[3] = {v.d_wsplit, v.d_wsplit + 3 * t1, v.d_wsplit + 3 * (t1 + t2)};
+    const size_t cnt[3] = {t1, t2, t3};
+    const int Ns[3] = {512, 256, 128}, Ks[3] = {CTD_FEATURES_PAD, 512, 256};
+    for (int l = 0; l < 3; ++l)
+      if (!ctd_make_weight_map(&v.tmap[l], sp[l], Ns[l], Ks[l])) {
+        snprintf(e->err, sizeof(e->err), "ctd_set_value_model: cannot build the TMA tensor maps of the weights (cuTensorMapEncodeTiled)");
+        return CTD_ECUDA;
+      }
+    // the split's source: [out][in] (the reference's own nn.Linear layout), BN already folded
     std::unique_ptr<float[]> h(new (std::nothrow) float[t1 + t2 + t3]);
     if (!h) return CTD_ENOMEM;
     for (int o = 0; o < 512; ++o) for (int k = 0; k < CTD_FEATURES_PAD; ++k) h[(size_t)o * CTD_FEATURES_PAD + k] = w1t[(size_t)k * 512 + o];
     for (int o = 0; o < 256; ++o) for (int k = 0; k < 512; ++k) h[t1 + (size_t)o * 512 + k] = w2t[(size_t)k * 256 + o];
     for (int o = 0; o < 128; ++o) for (int k = 0; k < 256; ++k) h[t1 + t2 + (size_t)o * 256 + k] = w3t[(size_t)k * 128 + o];
-    CTD_CUDA(e, v.d_model_tc.grow((t1 + t2 + t3) * sizeof(float)));
-    CTD_CUDA(e, cudaMemcpy(v.d_model_tc, h.get(), (t1 + t2 + t3) * sizeof(float), cudaMemcpyHostToDevice));
-    v.tc_w1 = v.d_model_tc; v.tc_w2 = v.d_model_tc + t1; v.tc_w3 = v.d_model_tc + t1 + t2;
-    // split the static weights into their TF32 terms once and describe them to the TMA engine
-    CTD_CUDA(e, v.d_wsplit.grow(3 * (t1 + t2 + t3) * sizeof(float)));
-    float* sp[3] = {v.d_wsplit, v.d_wsplit + 3 * t1, v.d_wsplit + 3 * (t1 + t2)};
-    const size_t cnt[3] = {t1, t2, t3};
-    const float* src[3] = {v.tc_w1, v.tc_w2, v.tc_w3};
-    const int Ns[3] = {512, 256, 128}, Ks[3] = {CTD_FEATURES_PAD, 512, 256};
-    v.tmap_ok = getenv("CTD_TC_NO_TMA") == nullptr;
+    CtdBuf<float> d_oi;
+    CTD_CUDA(e, d_oi.grow((t1 + t2 + t3) * sizeof(float)));
+    CTD_CUDA(e, cudaMemcpy(d_oi, h.get(), (t1 + t2 + t3) * sizeof(float), cudaMemcpyHostToDevice));
+    const float* src[3] = {d_oi, d_oi + t1, d_oi + t1 + t2};
     for (int l = 0; l < 3; ++l) {
       ctd_k_split3<<<(unsigned)((cnt[l] + 255) / 256), 256, 0, e->stream>>>(src[l], sp[l], cnt[l]);
       e->launches++;
-      v.tmap_ok = v.tmap_ok && ctd_make_weight_map(&v.tmap[l], sp[l], Ns[l], Ks[l]);
     }
     CTD_CUDA(e, cudaGetLastError());
+    CTD_CUDA(e, cudaStreamSynchronize(e->stream));   // the split has read d_oi before it is freed
   }
-  CTD_CUDA(e, cudaStreamSynchronize(e->stream));
   v.ready = true;
   return CTD_OK;
 }

@@ -10,9 +10,7 @@
 #define CTD_WARPS_PER_BLOCK 8
 #define CTD_BLOCK (CTD_WARPS_PER_BLOCK * 32)
 #endif
-#ifndef CTD_PLAYOUT_MIN_BLOCKS
 #define CTD_PLAYOUT_MIN_BLOCKS 8
-#endif
 #ifndef CTD_FULL
 #define CTD_FULL 0xFFFFFFFFu
 #endif
@@ -51,16 +49,9 @@ __global__ void __launch_bounds__(CTD_BLOCK, CTD_PLAYOUT_MIN_BLOCKS) CTD_PLAYOUT
   // shared memory is kept small because what is left of the 256 KB is the L1 that holds lane 0's stack
   __shared__ __align__(16) uint64_t scratch_u64[CTD_WARPS_PER_BLOCK][CTD_CHOOSE_BUF];
   static_assert(sizeof(ctd_state) <= CTD_CHOOSE_BUF * 8, "stage aliases the option buffer");
-#if CTD_PLAYOUT_RING
-  __shared__ __align__(16) uint32_t rings[CTD_WARPS_PER_BLOCK][128];
-#endif
   __shared__ unsigned long long bst[sizeof(ctd_playout_stats) / 8];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-#ifdef CTD_NO_STAGE_ALIAS
-  __shared__ ctd_state stage[CTD_WARPS_PER_BLOCK];
-#else
   ctd_state* const stage = reinterpret_cast<ctd_state*>(scratch_u64[0]);   // stage[wib] == scratch_u64[wib]
-#endif
   uint64_t (*choose_buf)[CTD_CHOOSE_BUF] = scratch_u64;
   CtdWork& w = works[wib];
   if (threadIdx.x < sizeof(ctd_playout_stats) / 8) bst[threadIdx.x] = 0;
@@ -78,26 +69,13 @@ __global__ void __launch_bounds__(CTD_BLOCK, CTD_PLAYOUT_MIN_BLOCKS) CTD_PLAYOUT
         w.k0 = (uint32_t)a.seed; w.k1 = (uint32_t)(a.seed >> 32);
         w.stream = 0;
         w.tape = nullptr; w.tape_len = 0;
-#if CTD_PLAYOUT_RING
-        w.ring = rings[wib]; w.ring_hi = 0;
-#endif
       }
       __syncwarp();
     } else {
       if (lane == 0) {
-#ifdef CTD_EXPERIMENT_GID_MASK   /* developer experiment: many warps play the SAME game (upper bound of what instruction-stream alignment could give) */
-        ctd_chance_init(w, a.seed, a.first_gid + (g & CTD_EXPERIMENT_GID_MASK), 0);
-#else
         ctd_chance_init(w, a.seed, a.first_gid + g, 0);
-#endif
-#if CTD_PLAYOUT_RING
-        w.ring = rings[wib];
-#endif
       }
       __syncwarp();
-#if CTD_PLAYOUT_RING
-      ctd_ring_refill(w, lane);   // the deal's 76-card shuffle and the first round's role shuffle come out of one refill
-#endif
       if (lane == 0) {
         ctd_deal_preset(w, a.ruleset);
         ctd_setup_round<false>(w);
@@ -109,25 +87,12 @@ __global__ void __launch_bounds__(CTD_BLOCK, CTD_PLAYOUT_MIN_BLOCKS) CTD_PLAYOUT
     for (;;) {
       bool stop = (w.gflags & 2) || w.err || (w.steps - steps0) >= a.max_steps;
       if (stop) break;
-#if CTD_PLAYOUT_RING
-      ctd_ring_refill(w, lane);
-#endif
-#if CTD_PLAYOUT_RING
-      uint64_t d = ctd_warp_choose(w, lane, choose_buf[wib], nullptr, -1, rings[wib]);
-#else
       uint64_t d = ctd_warp_choose(w, lane, choose_buf[wib]);
-#endif
-#ifdef CTD_PLAYOUT_ALL_LANES   /* experiment: every lane runs the transition (identical values), no divergence around it */
-      if (d == 0) w.err |= CTD_ERR_REF_RAISE;
-      else ctd_apply<false>(w, d);
-      __syncwarp();
-#else
       if (lane == 0) {
         if (d == 0) w.err |= CTD_ERR_REF_RAISE;
         else ctd_apply<false>(w, d);
       }
       __syncwarp();
-#endif
     }
     if (lane == 0 && !(w.gflags & 2) && !w.err) w.err |= CTD_ERR_MAXSTEPS;
     __syncwarp();

@@ -15,10 +15,8 @@
 #ifndef CTD_LAYOUT_HEADER
 #define CTD_LAYOUT_HEADER "ctd_layout_preset.h"
 #endif
-#ifndef CTD_NO_LAYOUT
 #define CTD_CHOOSE_LINKAGE inline   /* external name: takes part in the ordering */
 #include CTD_LAYOUT_HEADER
-#endif
 #include "ctd_playout.cuh"
 
 cudaError_t ctd_playout_preset_launch(const CtdPlayoutArgs& a, int grid, cudaStream_t stream) {

@@ -10,14 +10,9 @@
 // measured (round 2 A/B, 4096 roots): node moves, fp64 division / exp and the byte shuffle inlined at their uses are 10 % faster
 // than one out-of-line copy of each -- calls cost the search more (callee-saved registers through local memory on 32 lanes) than
 // the extra 30 KB of image
-#ifndef CTD_NODE_MOVE_ATTR
 #define CTD_NODE_MOVE_ATTR
 #define CTD_MATH_ATTR
 #define CTD_SHUFFLE_ATTR
-#endif
-#ifdef CTD_WANT_COOP_SHUFFLE   /* measured 6 % slower than the scalar loop (round 2 A/B): off */
-#define CTD_COOP_SHUFFLE 1   /* the warp runs the search converged: shuffles draw 32 swap indices at a time (ctd_engine.cuh) */
-#endif
 #define CTD_FIXED_PRESET 1
 #define CTD_NO_PLAYOUT_KERNEL 1
 #define CTD_NO_PRED_KERNEL 1

@@ -49,12 +49,7 @@ static __device__ void ctd_write_result(CtdTree& T, ctd_mccfr_result* r) {
   for (uint32_t i = 0; i < na; ++i) { r->cumulative_regrets[i] = R[i]; r->strategy[i] = S[i]; r->cumulative_strategy[i] = C[i]; }
 }
 
-#ifndef CTD_MCCFR_ALL_LANES
-#define CTD_MCCFR_ALL_LANES 1
-#endif
-#ifndef CTD_MCCFR_MIN_BLOCKS
 #define CTD_MCCFR_MIN_BLOCKS 3 /* 80 registers: fewer spills on the single active lane; 24 trees per SM resident (measured best at the 4096-root configuration) */
-#endif
 #ifndef CTD_NO_TRAIN_KERNEL
 __global__ void __launch_bounds__(CTD_BLOCK, CTD_MCCFR_MIN_BLOCKS) CTD_MCCFR_KERNEL_NAME(CtdMccfrArgs a) {
   __shared__ CtdWork works[CTD_WARPS_PER_BLOCK];
@@ -72,8 +67,8 @@ __global__ void __launch_bounds__(CTD_BLOCK, CTD_MCCFR_MIN_BLOCKS) CTD_MCCFR_KER
     // Every lane runs the same scalar search on the same data (identical values to identical addresses, control flow
     // uniform, the warp stays converged): no lane does anything the others do not, but leaf operations that are
     // lane-parallel by nature -- moving a 1.8 KB node between HBM and the working set -- can split their work over the
-    // lanes without restructuring the walk (CTD_MCCFR_ALL_LANES=0 restores the one-lane form).
-    if (CTD_MCCFR_ALL_LANES || lane == 0) {
+    // lanes without restructuring the walk.
+    {
       CtdTree T;
       T.w = &works[wib]; T.kn = &knows[wib]; T.opts = opts; T.scratch = scratch[wib]; T.stage = &tstage[wib];
       T.vnet = nullptr; T.act = nullptr;
@@ -147,7 +142,7 @@ __global__ void __launch_bounds__(CTD_BLOCK, CTD_MCCFR_MIN_BLOCKS) CTD_MCCFR_PRE
     t = __shfl_sync(CTD_FULL, t, 0);
     if (t >= a.n_roots) break;
     t = a.tree_list ? a.tree_list[t] : t + a.first_root;
-    if (CTD_MCCFR_ALL_LANES || lane == 0) {   // all lanes on the same scalar walk, see ctd_k_mccfr
+    {   // all lanes on the same scalar walk, see ctd_k_mccfr
       CtdTree T;
       T.w = &works[wib]; T.kn = &knows[wib]; T.opts = opts; T.scratch = scratch[wib]; T.stage = &tstage[wib];
       CtdTreeHdr* hdr = &a.hdrs[t];

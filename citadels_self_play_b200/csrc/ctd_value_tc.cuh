@@ -36,14 +36,8 @@
 #define CTD_TC_TERMS 3
 #define CTD_TC_TILE_BYTES (128 * CTD_TC_BK * 4)                   /* 16 KB: one operand tile, one split term */
 #define CTD_TC_STAGE_BYTES (2 * CTD_TC_TERMS * CTD_TC_TILE_BYTES) /* A0 A1 A2 B0 B1 B2 */
-#ifndef CTD_TC_HALF_K
-#define CTD_TC_HALF_K 0 /* experiment (1): every instruction carries four real products and four zeros -- twice the instructions, and the error DOUBLES (6.8e-5 vs 1.8e-5): the rounding happens once per instruction when the accumulator is updated */
-#endif
-#ifndef CTD_TC_ACCS
 #define CTD_TC_ACCS 4 /* TMEM accumulators the K slices are dealt over (each rounds once per instruction at its own, smaller, magnitude); summed in fp32 registers in the epilogue */
-#endif
-#define CTD_TC_ZERO_BYTES (CTD_TC_HALF_K ? CTD_TC_TILE_BYTES : 0)   /* a tile of zeros the padded K half is read from */
-#define CTD_TC_SMEM (2 * CTD_TC_STAGE_BYTES + CTD_TC_ZERO_BYTES + 1024)      /* two stages + zero tile + alignment slack */
+#define CTD_TC_SMEM (2 * CTD_TC_STAGE_BYTES + 1024)               /* two stages + alignment slack */
 #define CTD_TC_SPIN_LIMIT (1u << 24)
 
 __device__ __forceinline__ uint32_t ctd_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -141,15 +135,6 @@ __global__ void __launch_bounds__(128) ctd_k_linear_tc(const float* __restrict__
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_d = tmem_base_slot;
 
-#if CTD_TC_HALF_K
-  // The residual error of this path is made inside the instruction, when it sums its eight products
-  // (profiles/r01_value_tc_accuracy.md).  Halve it: an instruction's second K core column is read from a tile of zeros (the
-  // descriptor's leading-dimension offset points there), so it sums four real products; the other column gets its own
-  // instruction.  Twice the MMAs, which these tiny layers do not notice.
-  uint8_t* zero_tile = smem + 2 * CTD_TC_STAGE_BYTES;
-  for (int i = tid * 16; i < CTD_TC_TILE_BYTES; i += 128 * 16) *reinterpret_cast<float4*>(zero_tile + i) = make_float4(0.f, 0.f, 0.f, 0.f);
-  const uint32_t zero_addr = ctd_smem_u32(zero_tile);
-#endif
   const int stages = K / CTD_TC_BK;
   bool ok = true;
   for (int s = 0; s < stages; ++s) {
@@ -175,26 +160,16 @@ __global__ void __launch_bounds__(128) ctd_k_linear_tc(const float* __restrict__
       for (int kk = 0; kk < CTD_TC_BK / 8; ++kk) {  // K = 8 per instruction = two 16-byte core columns
         const uint32_t ko = (uint32_t)kk * 256;
         const uint32_t tmem_acc = tmem_d + (uint32_t)((kk % CTD_TC_ACCS) * 128);   // K slice kk of every stage -> accumulator kk
-        uint32_t acc = CTD_TC_ACCS == 1 ? (uint32_t)((s | kk) != 0) : (uint32_t)(s != 0 || kk >= CTD_TC_ACCS);
+        uint32_t acc = (uint32_t)(s != 0 || kk >= CTD_TC_ACCS);
         // smallest products first: (i, j) with i + j = 2, then 1, then 0
 #pragma unroll
         for (int sum = CTD_TC_TERMS - 1; sum >= 0; --sum)
 #pragma unroll
           for (int i = 0; i <= sum; ++i) {
             const int j = sum - i;
-#if CTD_TC_HALF_K
-#pragma unroll
-            for (int half = 0; half < 2; ++half) {   // core column `half` of this K = 8 slice, padded with a column of zeros
-              const uint32_t aa = a0 + i * CTD_TC_TILE_BYTES + ko + half * 128;
-              const uint32_t bb = b0 + j * CTD_TC_TILE_BYTES + ko + half * 128;
-              ctd_umma_tf32(tmem_acc, ctd_umma_desc(aa, zero_addr - aa, 1024), ctd_umma_desc(bb, zero_addr - bb, 1024), acc);
-              acc = 1;
-            }
-#else
             ctd_umma_tf32(tmem_acc, ctd_umma_desc(a0 + i * CTD_TC_TILE_BYTES + ko, 128, 1024),
                           ctd_umma_desc(b0 + j * CTD_TC_TILE_BYTES + ko, 128, 1024), acc);
             acc = 1;
-#endif
           }
       }
       // arrives on the stage barrier when every MMA issued so far has completed (implies fence::before_thread_sync)
@@ -327,7 +302,7 @@ __global__ void __launch_bounds__(128) ctd_k_linear_tc_tma(const float* __restri
 #pragma unroll
       for (int kk = 0; kk < CTD_TC_BK / 8; ++kk) {
         const uint32_t tmem_acc = tmem_d + (uint32_t)((kk % CTD_TC_ACCS) * 128);
-        uint32_t acc = CTD_TC_ACCS == 1 ? (uint32_t)((s | kk) != 0) : (uint32_t)(s != 0 || kk >= CTD_TC_ACCS);
+        uint32_t acc = (uint32_t)(s != 0 || kk >= CTD_TC_ACCS);
 #pragma unroll
         for (int sum = CTD_TC_TERMS - 1; sum >= 0; --sum)
 #pragma unroll

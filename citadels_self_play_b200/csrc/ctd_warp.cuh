@@ -14,31 +14,15 @@
 #pragma once
 #include "ctd_engine.cuh"
 
-#ifndef CTD_CHOOSE_BUF
 #define CTD_CHOOSE_BUF 32
-#endif
 /* descriptors kept by the scalar fallback (256 B = one packed record); longer lists are selected by a second enumeration pass */
 
 #ifdef __CUDACC__
 #define CTD_ALL 0xFFFFFFFFu
 
-// Chance for the fused playout: the Philox stream is counter-based, so the warp computes 32 blocks (128 draws) at once,
-// one block per lane, into a ring in shared memory; lane 0's scalar rules code then reads draws from the ring
-// (ctd_u32 in ctd_engine.cuh).  Called with all lanes converged whenever fewer than 16 blocks are left ahead of the
-// cursor; a step that needs more than that (a 76-card shuffle after the ring ran low) falls back to lane-0 blocks.
-__device__ __forceinline__ void ctd_ring_refill(CtdWork& w, int lane) {
-  const uint32_t blk = w.draws >> 2, hi = w.ring_hi;
-  if ((int32_t)(hi - blk) >= 16) return;
-  const uint32_t b = blk + (uint32_t)lane;
-  if ((int32_t)(b - hi) >= 0) ctd_philox(b, w.stream, w.g0, w.g1, w.k0, w.k1, &w.ring[(b & 31u) << 2]);
-  __syncwarp();
-  if (lane == 0) w.ring_hi = blk + 32u;
-  __syncwarp();
-}
-
 // scalar fallback: lane 0 materialises the list, draws k, picks
 // CHECK: the checker's form (ctd_k_choose_check: report the count, take a given k).  The playout kernels instantiate CHECK = false,
-// where count_out / want / ring are dead on entry and cost neither registers nor code.
+// where count_out / want are dead on entry and cost neither registers nor code.
 template <bool CHECK>
 static __device__ __noinline__ uint64_t ctd_choose_scalar(CtdWork& w, int lane, uint64_t* buf, uint32_t* count_out_, int want_) {
   uint32_t* const count_out = CHECK ? count_out_ : nullptr;
@@ -104,24 +88,16 @@ __device__ __forceinline__ int ctd_cost_w(int t) {
 // Structure: (A) classify the state and count -- all ballots happen here; (B) ONE draw; (C) select.
 enum { CTD_PM_ROLE_PICK, CTD_PM_GOLD_OR_CARD, CTD_PM_SINGLE, CTD_PM_KEEP, CTD_PM_KEEP_LIBRARY, CTD_PM_WITCH, CTD_PM_MAIN };
 
-#ifndef CTD_CHOOSE_ATTR
-#define CTD_CHOOSE_ATTR __noinline__
-#endif
-// `ring` (playout kernel): the warp's Philox ring, refilled at the top of the step, so the one draw of the cooperative
-// path is a broadcast read by every lane instead of lane-0 code followed by a shuffle.
 #ifndef CTD_CHOOSE_LINKAGE
 #define CTD_CHOOSE_LINKAGE static
 #endif
+// `ring_`, `ring` and the `ring != nullptr` draw below are unused; kept so that the callers' code stays unchanged
 template <bool CHECK = false>
-CTD_CHOOSE_LINKAGE __device__ CTD_CHOOSE_ATTR uint64_t ctd_warp_choose(CtdWork& w, int lane, uint64_t* buf, uint32_t* count_out_ = nullptr,
+CTD_CHOOSE_LINKAGE __device__ __noinline__ uint64_t ctd_warp_choose(CtdWork& w, int lane, uint64_t* buf, uint32_t* count_out_ = nullptr,
                                                  int want_ = -1, const uint32_t* ring_ = nullptr) {
   uint32_t* const count_out = CHECK ? count_out_ : nullptr;
   const int want = CHECK ? want_ : -1;
-#if CTD_PLAYOUT_RING
-  const uint32_t* const ring = ring_;
-#else
   const uint32_t* const ring = nullptr;
-#endif
   const int p = w.player, st = w.state;
   if ((w.gflags & 2) || p >= 6) return ctd_choose_scalar<CHECK>(w, lane, buf, count_out, want);
   const uint64_t me = (uint64_t)p << 6;
@@ -250,8 +226,8 @@ CTD_CHOOSE_LINKAGE __device__ CTD_CHOOSE_ATTR uint64_t ctd_warp_choose(CtdWork& 
   uint32_t k;
   if (want >= 0) {
     k = (uint32_t)want;
-  } else if (ring != nullptr) {
-    const uint32_t dr = w.draws;                    // draw number dr lives at ring[dr & 127] (block dr >> 2 in slot (dr >> 2) & 31)
+  } else if (ring != nullptr) {                     // never taken (see `ring` above)
+    const uint32_t dr = w.draws;
     k = (uint32_t)(((uint64_t)ring[dr & 127u] * total) >> 32);
     __syncwarp();
     if (lane == 0) w.draws = dr + 1;
