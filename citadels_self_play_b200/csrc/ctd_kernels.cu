@@ -1204,7 +1204,8 @@ static ctd_status ctd_deep_pass(ctd_engine* e, const CtdSearch& sp, const uint32
   // Two groups of trees take turns: each group's waves (walk kernel -> batched leaf evaluation -> walk kernel ...) run on
   // their own stream, so the tail of one group's wave -- a few trees with expensive expansions -- overlaps with the other
   // group's kernel instead of idling the GPU.  Trees are independent, results do not depend on the grouping.
-  const int G = n >= 1024 ? 2 : 1;
+  // A retry pass (d_list) runs as one group: its rows are indexed by root, so two groups would evaluate each other's rows.
+  const int G = n >= 1024 && !d_list ? 2 : 1;
   if (G == 2 && !e->ev_join) {   // the join event comes last: a failure part way is completed by the next call
     if (!e->stream2) CTD_CUDA(e, cudaStreamCreateWithFlags(&e->stream2, cudaStreamNonBlocking));
     CTD_CUDA(e, e->d_counter2.grow(sizeof(unsigned long long)));
@@ -1289,6 +1290,8 @@ static ctd_status ctd_deep_pass(ctd_engine* e, const CtdSearch& sp, const uint32
 static ctd_status ctd_search(ctd_engine* e, const CtdSearch& sp, ctd_mccfr_result* results, float* elapsed_ms, uint32_t* waves_out) {
   CTD_CUDA(e, cudaSetDevice(e->device));
   CTD_CUDA(e, e->d_results.grow((size_t)sp.n_roots * sizeof(ctd_mccfr_result)));
+  // a record's arrays are written up to the root's children only: the rest of the record must not keep an earlier call's tree
+  CTD_CUDA(e, cudaMemsetAsync(e->d_results, 0, (size_t)sp.n_roots * sizeof(ctd_mccfr_result), e->stream));
   ctd_status s = CTD_OK;
   if (sp.deep) { s = ctd_pred_buffers(e); if (s != CTD_OK) return s; }
   if (sp.resume) {   // the trees stay where they are (arena 0 keeps its bump pointer); trees that run out of arena now keep status 2

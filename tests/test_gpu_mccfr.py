@@ -161,16 +161,48 @@ def test_exhausted_arena_is_retried(engine, monkeypatch):
     assert (got["status"] <= 1).all()
     for f in ("status", "n_nodes", "rng_draws", "n_children", "cumulative_regrets", "cumulative_strategy", "node_value"):
         assert np.array_equal(got[f], want[f]), f
+
+
+def test_result_records_keep_nothing_of_an_earlier_call(engine):
+    """A record's arrays hold the root's first children only (all 60 entries at a role pick); everything after them, and every
+    array of a root without children, is zero, whatever the same slots held in the previous call."""
+    n = 64
+    engine.make_roots(n, seed=808, first_gid=3000, back_lo=0, back_hi=300, flavour=1)
+    before = engine.mccfr(n, iterations=50, seed=808)["results"]
+    engine.make_roots(n, seed=909, first_gid=4000, back_lo=0, back_hi=20)
+    res = engine.mccfr(n, iterations=50, seed=909)["results"]
+
+    def used(r):
+        k = min(int(r["n_children"]), 128)
+        return k, (60 if r["role_pick"] else k) if k else 0
+    assert any(used(a)[1] > used(b)[1] for a, b in zip(before, res))   # the earlier call left longer arrays in some slots
+    for i, r in enumerate(res):
+        k, na = used(r)
+        assert not r["options"][k:].any(), (i, "options")
+        for f in ("cumulative_regrets", "strategy", "cumulative_strategy"):
+            assert not r[f][na:].any(), (i, f)
+
+
+@pytest.mark.parametrize("backend", ["fused", "fp32", "tcgen05"])
+def test_exhausted_arena_is_retried_deep(engine, monkeypatch, backend):
+    """The same for deep MCCFR on each backend: a retry pass of fewer than 1024 trees runs as one group, its model evaluated over
+    every root's row with the pending mask picking the retried trees' leaves (tests/test_gpu_value_waves.py: more than 1024)."""
     from citadels_self_play_b200.value_model import ValueOnlyNN
     import torch
+    n = 96
+    engine.make_roots(n, seed=99, first_gid=7000, back_lo=0, back_hi=20)
     torch.manual_seed(0)
     engine.set_value_model(ValueOnlyNN(418, 512).eval())
-    want = engine.mccfr_pred(n, iterations=200, max_depth=10, seed=99)["results"]
-    monkeypatch.setenv("CTD_ARENA0_BYTES", str(24 << 20))
-    got = engine.mccfr_pred(n, iterations=200, max_depth=10, seed=99)["results"]
-    monkeypatch.delenv("CTD_ARENA0_BYTES")
+    engine.set_value_backend(backend)
+    try:
+        want = engine.mccfr_pred(n, iterations=200, max_depth=10, seed=99)["results"]
+        monkeypatch.setenv("CTD_ARENA0_BYTES", str(24 << 20))
+        got = engine.mccfr_pred(n, iterations=200, max_depth=10, seed=99)["results"]
+        monkeypatch.delenv("CTD_ARENA0_BYTES")
+    finally:
+        engine.set_value_backend("fused")      # back to the default
     assert (got["status"] <= 1).all()
-    for f in ("n_nodes", "rng_draws", "cumulative_regrets", "node_value"):
+    for f in ("status", "n_nodes", "rng_draws", "n_children", "live_option", "cumulative_regrets", "cumulative_strategy", "node_value"):
         assert np.array_equal(got[f], want[f]), f
 
 
