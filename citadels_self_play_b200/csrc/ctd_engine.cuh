@@ -1,14 +1,15 @@
 // ctd_engine.cuh -- the Citadels rules engine: on-chip working state, legal-option enumeration and
 // state transition.  Written from the behaviour of the reference (paths below are relative to the
 // reference repository root), not from its code structure: the reference walks Python object graphs
-// (Card/Deck/Agent/option); this engine works on a flat working record that lives in shared memory for
+// (Card/Deck/Agent/option); this engine works on a flat working record that lives in shared memory (in the fused playout: thread-local memory) for
 // the whole life of a game and is only packed to the 256-byte HBM record (ctd_state) at the API boundary.
 //
-// Execution model on the device: one warp owns one game.  The working record sits in that warp's slice
-// of shared memory.  The transition (`ctd_apply`) is a scalar, order-sensitive list manipulation and runs
-// on lane 0; enumeration is read-only and has both a scalar form (`ctd_enumerate`, used for materialised
-// option lists and as the definition of option order) and a warp-cooperative count/select form in
-// ctd_warp.cuh used by the fused playout kernel.
+// Execution model on the device.  The fused random playout (ctd_playout.cuh) gives every thread a game of its own: the
+// working record sits in that thread's local memory, and the thread chooses with the scalar enumerator (count, draw,
+// select) and applies with `ctd_apply`.  The other kernels (MCCFR, arena, step-wise API) give one warp one game: the
+// record sits in the warp's slice of shared memory and the transition (`ctd_apply`), a scalar, order-sensitive list
+// manipulation, runs on lane 0.  Enumeration (`ctd_enumerate`) is one scalar visitor walk that defines the option order:
+// it materialises option lists (CtdEmit) or counts and selects the k-th option (CtdPick, ctd_playout.cuh).
 //
 // The same source compiles for the host (tests/hostsim) so the rules can be replayed against the golden
 // traces without a GPU; that build is a test vehicle, never a fallback of the product.
@@ -35,15 +36,22 @@
 #define CTD_LOOP
 #define CTD_UNROLL
 #endif
-// On the device every CtdWork / CtdKnow lives in shared memory (all kernels declare them __shared__).  Telling the
-// compiler turns the generic LD.E / ST.E (+ descriptor moves and 64-bit address arithmetic) of the out-of-line rules code
-// into LDS / STS with immediate offsets.
+// On the device every CtdKnow, and every CtdWork of the warp-per-game kernels, lives in shared memory (they declare them
+// __shared__).  Telling the compiler turns the generic LD.E / ST.E (+ descriptor moves and 64-bit address arithmetic) of the
+// out-of-line rules code into LDS / STS with immediate offsets.  The fused playout units define CTD_WORK_LOCAL: there each
+// thread plays its own game in a CtdWork of its own local memory (ctd_playout.cuh), and the same hint gives LDL / STL.
 #if defined(__CUDA_ARCH__)
 #define CTD_ASSUME_SHARED(p) __builtin_assume(__isShared(p))
 #define CTD_ASSUME_GLOBAL(p) __builtin_assume(__isGlobal(p))
+#ifdef CTD_WORK_LOCAL
+#define CTD_ASSUME_WORK(p) __builtin_assume(__isLocal(p))
+#else
+#define CTD_ASSUME_WORK(p) CTD_ASSUME_SHARED(p)
+#endif
 #else
 #define CTD_ASSUME_SHARED(p)
 #define CTD_ASSUME_GLOBAL(p)
+#define CTD_ASSUME_WORK(p)
 #endif
 #define CTD_ASSUME_SHARED_K(p) CTD_ASSUME_SHARED(p)
 // (Only references to whole records carry the hint.  Hinting the raw list pointers of ctd_take_like & co. as well made
@@ -419,7 +427,7 @@ CTD_HD CTD_NI inline int ctd_take_like(uint8_t* a, uint8_t& n, int t) {
   return t;
 }
 CTD_HD CTD_NI inline void ctd_append(CtdWork& w, uint8_t* a, uint8_t& n, int cap, int c) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   if (n >= cap) {
 #ifdef CTD_HOST_DEBUG
     fprintf(stderr, "overflow cap %d list-offset %ld state %d\n", cap, (long)(a - (uint8_t*)&w), w.state);
@@ -441,7 +449,7 @@ CTD_HD inline void ctd_disc_push(CtdWork& w, int c) { ctd_append(w, w.disc, w.n_
 
 // reshuffle_deck_if_empty (game/option_functions.py:564-570)
 CTD_HD CTD_NI inline void ctd_reshuffle_if_empty(CtdWork& w) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   if (w.n_deck == 0 && w.n_disc != 0) {
     uint8_t* d = w.disc;
     ctd_shuffle_bytes(w, d, w.n_disc);
@@ -453,7 +461,7 @@ CTD_HD CTD_NI inline void ctd_reshuffle_if_empty(CtdWork& w) {
 }
 // reshuffle + draw_card; returns -1 for "Deck Empty" (game/deck.py:57-60), which add_card drops (:62-70)
 CTD_HD CTD_NI inline int ctd_draw(CtdWork& w) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   ctd_reshuffle_if_empty(w);
   if (w.n_deck == 0) return -1;
   int c = w.deck[w.deck_head];
@@ -477,7 +485,7 @@ CTD_HD inline int ctd_name(const CtdWork& w, int p) {
 }
 // Game.get_player_from_role_id (game/game.py:403-412); -1 when nobody holds it
 CTD_HD CTD_NI inline int ctd_player_from_rank(const CtdWork& w, int rank) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   int want = rank < 0 ? CTD_ROLE_BEWITCHED : rank;
   CTD_LOOP for (int p = 0; p < 6; ++p) if (w.role[p] == want) return p;
   return -1;
@@ -489,7 +497,7 @@ CTD_HD inline void ctd_clear_done(CtdWork& w) { w.done = 0; w.n_trade = 0; w.n_n
 // Game.setup_round (game/game.py:144-171)
 template <bool KN = true>
 CTD_HD CTD_NI inline void ctd_setup_round(CtdWork& w, CtdKnowSet ks = CtdKnowSet{nullptr, 0}) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   CTD_LOOP for (int r = 0; r < 8; ++r) w.rprops[r] = 0;
   w.used_len = 0;
   CTD_LOOP for (int i = 0; i < 6; ++i) w.used_roles[i] = 0;
@@ -514,7 +522,7 @@ CTD_HD CTD_NI inline void ctd_setup_round(CtdWork& w, CtdKnowSet ks = CtdKnowSet
 
 // Game.refresh_used_roles (game/game.py:349-357); value+1 encoding keeps Bewitched (-1) sortable as 0
 CTD_HD CTD_NI inline bool ctd_refresh_used_roles(CtdWork& w) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   uint8_t v[6];
   CTD_LOOP for (int p = 0; p < 6; ++p) {
     int r = w.role[p];
@@ -534,7 +542,7 @@ CTD_HD CTD_NI inline bool ctd_refresh_used_roles(CtdWork& w) {
 
 // Game.setup_next_player (game/game.py:391-401); current < 0 == None
 CTD_HD CTD_NI inline void ctd_setup_next_player(CtdWork& w, int current) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   int nxt;
   if (w.state == 0) {
     if (!ctd_refresh_used_roles(w)) return;
@@ -560,7 +568,7 @@ CTD_HD CTD_NI inline void ctd_setup_next_player(CtdWork& w, int current) {
 
 // Agent.count_points (game/agent.py:116-143)
 CTD_HD CTD_NI inline int ctd_count_points(const CtdWork& w, int p) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   int pts = 0;
   const uint8_t* b = w.bld[p];
   int n = w.n_bld[p];
@@ -581,7 +589,7 @@ CTD_HD CTD_NI inline int ctd_count_points(const CtdWork& w, int p) {
 
 // Game.check_game_ending (game/game.py:359-368): first arg-max wins
 CTD_HD CTD_NI inline bool ctd_check_game_ending(CtdWork& w) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   if (!(w.gflags & 1)) return false;
   int best = -1000, bi = 0;
   CTD_LOOP for (int p = 0; p < 6; ++p) {
@@ -596,7 +604,7 @@ CTD_HD CTD_NI inline bool ctd_check_game_ending(CtdWork& w) {
 
 // move_crown + troneroom_owner_gold (game/option_functions.py:625-631, :588-595)
 CTD_HD CTD_NI inline void ctd_move_crown(CtdWork& w, int target) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   w.crown = (uint8_t)target;
   CTD_LOOP for (int p = 0; p < 6; ++p)
     if (ctd_owns(w, p, 32)) { w.gold[p] += 1; break; }
@@ -615,7 +623,7 @@ CTD_HD inline void ctd_is_last_round(CtdWork& w) {
 
 // Game.set_preset (game/game.py:420-489): Deck() shuffles the 76 cards, fixed hands are pulled by type
 CTD_HD CTD_NI inline void ctd_deal_preset(CtdWork& w, int ruleset, uint8_t* used_cards_out = nullptr) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   CTD_LOOP for (int p = 0; p < 6; ++p) {
     w.n_hand[p] = w.n_bld[p] = w.n_mus[p] = w.n_jd[p] = 0;
     w.gold[p] = 2; w.role[p] = CTD_ROLE_NONE; w.replicas[p] = 0; w.pflags[p] = 0;
@@ -745,7 +753,7 @@ CTD_HD CTD_NI inline uint32_t ctd_magician_count(int n, int r) {
 // emperor_options (game/agent_functions.py:368-382)
 template <class E>
 CTD_HD CTD_NI inline void ctd_emperor_options(const CtdWork& w, int p, bool dead, E& e) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   CTD_LOOP for (int q = 0; q < 6; ++q) {
     if (q == p) continue;
     const uint64_t base = ctd_opt(CTD_K_GIVE_CROWN, p) | ctd_f_target(q);
@@ -759,7 +767,7 @@ CTD_HD CTD_NI inline void ctd_emperor_options(const CtdWork& w, int p, bool dead
 // "afford", the combinations of (gold - cost) other cards to hand over, thinned to about a hundred per card
 template <class E>
 CTD_HD CTD_NI inline void ctd_cardinal_options(const CtdWork& w, int p, E& e) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   const uint8_t* hand = w.hand[p];
   const int nh = w.n_hand[p];
   uint64_t own = 0;
@@ -790,7 +798,7 @@ CTD_HD CTD_NI inline void ctd_cardinal_options(const CtdWork& w, int p, E& e) {
 // every hand card and three times over it shuffles the other cards (cumulatively) and takes the first k-1.
 template <class E>
 CTD_HD CTD_NI inline void ctd_seer_give_back_options(CtdWork& w, int p, E& e) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   int k = 0;
   CTD_LOOP for (int q = 0; q < 6; ++q) k += (w.seer_mask >> q) & 1;
   const int n = w.n_hand[p];
@@ -822,7 +830,7 @@ CTD_HD CTD_NI inline void ctd_seer_give_back_options(CtdWork& w, int p, E& e) {
 // very list it iterates: every call shrinks seven_drawn_cards, and every option shares what is left.
 template <class E>
 CTD_HD CTD_NI inline void ctd_scholar_give_back_options(CtdWork& w, int p, E& e) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   int i = 0;
   while (i < w.n_seven) {
     const int t = ctd_ctype(w.seven[i]);
@@ -835,7 +843,7 @@ CTD_HD CTD_NI inline void ctd_scholar_give_back_options(CtdWork& w, int p, E& e)
 // character_options (game/agent_functions.py:156-209) and the per-role enumerators it dispatches to
 template <class E>
 CTD_HD CTD_NI inline void ctd_character_options(const CtdWork& w, int p, int nm, E& e) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   if (!(w.done & CTD_DM_CHARACTER)) {
     switch (nm) {
       case CTD_ASSASSIN: CTD_NOT_PRESET();  // :213-218
@@ -956,7 +964,7 @@ CTD_HD CTD_NI inline void ctd_character_options(const CtdWork& w, int p, int nm,
 // main_round_options (game/agent_functions.py:133-147); concatenation order is observable
 template <class E>
 CTD_HD CTD_NI inline void ctd_main_round_options(const CtdWork& w, int p, int nm, E& e) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   const uint8_t* bld = w.bld[p];
   const int nb = w.n_bld[p];
   const uint8_t* hand = w.hand[p];
@@ -1012,7 +1020,7 @@ CTD_HD CTD_NI inline void ctd_main_round_options(const CtdWork& w, int p, int nm
 // (HandKnowledge.hand); in a playout it equals the target's current hand.  `replica` leaks across iterations.
 template <class E>
 CTD_HD CTD_NI inline void ctd_wizard_take_options(const CtdWork& w, int p, const uint8_t* cards, int n, E& e) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   int q = w.wiz_target;
   uint64_t own = 0;
   CTD_LOOP for (int i = 0; i < w.n_bld[p]; ++i) own |= 1ull << ctd_ctype(w.bld[p][i]);
@@ -1039,7 +1047,7 @@ CTD_HD CTD_NI inline void ctd_wizard_take_options(const CtdWork& w, int p, const
 // Agent.get_options (game/agent.py:50-83).  An empty result with err set means the reference would raise.
 template <class E>
 CTD_HD CTD_NI inline void ctd_enumerate(CtdWork& w, E& e, const CtdKnow* kn = nullptr) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   if (w.gflags & 2) return;  // terminal: the reference's loops stop here
   const int p = w.player;
   const int st = w.state;
@@ -1145,7 +1153,7 @@ CTD_HD inline void ctd_restore_next(CtdWork& w) {
 
 // carry_out_building (game/option_functions.py:102-127)
 CTD_HD CTD_NI inline void ctd_apply_build(CtdWork& w, int p, int t, int replica) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   int c = ctd_take_like(w.hand[p], w.n_hand[p], t);
   ctd_append(w, w.bld[p], w.n_bld[p], CTD_BLD_CAP, c);
   if (ctd_name(w, p) != CTD_ALCHEMIST) w.gold[p] -= (int32_t)ctd_ccost(c);
@@ -1171,7 +1179,7 @@ CTD_HD CTD_NI inline void ctd_apply_build(CtdWork& w, int p, int t, int replica)
 // finish_main_sequnce_actions (game/option_functions.py:189-243).  Returns true when the game ended.
 template <bool KN>
 CTD_HD CTD_NI inline bool ctd_apply_finish(CtdWork& w, uint64_t d, CtdKnowSet ks) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   const int p = CTD_OPT_PERP(d);
   const int pr = w.role[p];
   if (pr >= 8) { w.err |= CTD_ERR_REF_RAISE; return false; }
@@ -1214,7 +1222,7 @@ CTD_HD CTD_NI inline bool ctd_apply_finish(CtdWork& w, uint64_t d, CtdKnowSet ks
 // KN = false instantiates the transition without the knowledge bookkeeping (the playout kernel: smaller image).
 template <bool KN = true>
 CTD_HD CTD_NI inline bool ctd_apply(CtdWork& w, uint64_t d, CtdKnowSet ks = CtdKnowSet{nullptr, 0}) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   const int k = CTD_OPT_KIND(d);
   const int p = CTD_OPT_PERP(d);
   bool won = false;
@@ -1733,16 +1741,16 @@ CTD_HD CTD_NI inline bool ctd_apply(CtdWork& w, uint64_t d, CtdKnowSet ks = CtdK
 
 // run_utils.create_game (run_utils.py:20-27)
 CTD_HD CTD_NI inline void ctd_new_game(CtdWork& w, uint64_t seed, uint64_t gid, int ruleset) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   ctd_chance_init(w, seed, gid, 0);
   ctd_deal_preset(w, ruleset);
   ctd_setup_round(w);
 }
 
 // ------------------------------------------------------------------------------------------ pack / unpack
-// Scalar forms (definition of the layout); ctd_warp.cuh has the lane-parallel device forms.
+// Scalar forms (definition of the layout).
 CTD_HD CTD_NI inline void ctd_pack(const CtdWork& w, ctd_state* s) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   {  // zero the record with eight-byte stores (ctd_state is 8-byte aligned)
     uint64_t* z = (uint64_t*)s;
     CTD_LOOP for (int i = 0; i < CTD_STATE_BYTES / 8; ++i) z[i] = 0;
@@ -1807,7 +1815,7 @@ CTD_HD CTD_NI inline void ctd_pack(const CtdWork& w, ctd_state* s) {
 }
 
 CTD_HD CTD_NI inline void ctd_unpack(const ctd_state* s, CtdWork& w) {
-  CTD_ASSUME_SHARED(&w);
+  CTD_ASSUME_WORK(&w);
   w.err = s->err;
   const uint8_t* arena = s->arena;
   int c = 0;

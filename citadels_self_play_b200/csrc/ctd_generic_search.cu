@@ -15,7 +15,7 @@
 #define CTD_NO_PRED_KERNEL 1
 #define CTD_MCCFR_KERNEL_NAME ctd_k_mccfr
 #define CTD_MCCFR_PRED_KERNEL_NAME ctd_k_mccfr_pred_unused
-#ifdef CTD_LAYOUT_HEADER   /* placement of the device functions by name order, see ctd_layout_preset.h / tools/layout_search.py */
+#ifdef CTD_LAYOUT_HEADER   /* placement of the device functions by name order, see ctd_layout_classic.h / tools/layout_search.py */
 #include CTD_LAYOUT_HEADER
 #endif
 #include "ctd_search.cuh"

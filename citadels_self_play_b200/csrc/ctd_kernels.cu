@@ -3,10 +3,11 @@
 // Layout of the data path:
 //   HBM     ctd_state slots[capacity]          256 B records, 2 x 128 B lines each, one warp moves one
 //                                              record as 32 x 8 B (coalesced)
-//   smem    CtdWork per warp (1.3 KB)          the game lives here for its whole fused playout (~420 steps)
-//   regs    option count / selection           warp-cooperative enumeration (ctd_warp.cuh)
-// One warp owns one game.  The playout kernel is persistent: warps pull game ids from a global counter so
-// that the 244..632-step spread of game lengths does not leave SMs idle at the tail.
+//   smem    CtdWork per warp (1.3 KB)          the game of a step-wise / search / arena kernel
+//   local   CtdWork per thread (1.5 KB)        the game of a fused playout for its whole life (~420 steps)
+// One warp owns one game, except in the fused playout, where one thread owns one game (ctd_playout.cuh).  The playout
+// kernel is persistent: threads pull game ids from a global counter so that the 244..632-step spread of game lengths
+// does not leave SMs idle at the tail.
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -22,7 +23,6 @@
 #define CTD_NO_TRAIN_KERNEL 1
 #define CTD_NO_PRED_KERNEL 1
 #include "ctd_engine.cuh"
-#include "ctd_warp.cuh"
 #include "ctd_playout.cuh"
 #include "ctd_mccfr.cuh"
 #include "ctd_search.cuh"
@@ -123,42 +123,36 @@ __global__ void __launch_bounds__(CTD_BLOCK) ctd_k_step(ctd_state* slots, uint32
   ctd_record_store(&slots[slot], &stage[wib], lane);
 }
 
-// Checker for the warp-cooperative chooser: for every slot, the cooperative count and the cooperative k-th option for
-// every k must equal the scalar enumerator's list.  mismatches[slot] = number of differing entries (+1e6 if the counts differ).
+// Checker for the fused playout's choice (ctd_playout.cuh): for every slot, the counting pass (ctd_lane_count) and the
+// selecting pass (ctd_lane_select) for every k must equal the scalar enumerator's materialised list.
+// mismatches[slot] = number of differing entries (+1e6 if the counts differ).  Lane 0 of each warp checks its slot.
 __global__ void __launch_bounds__(CTD_BLOCK) ctd_k_choose_check(const ctd_state* slots, uint32_t n, uint32_t* mismatches,
                                                                 uint64_t* scratch_opts, uint32_t cap) {
   __shared__ CtdWork works[CTD_WARPS_PER_BLOCK];
   __shared__ ctd_state stage[CTD_WARPS_PER_BLOCK];
-  __shared__ uint64_t choose_buf[CTD_WARPS_PER_BLOCK][CTD_CHOOSE_BUF];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const uint32_t slot = blockIdx.x * CTD_WARPS_PER_BLOCK + wib;
   if (slot >= n) return;
   CtdWork& w = works[wib];
   ctd_record_load(&slots[slot], &stage[wib], lane);
+  if (lane != 0) return;
+  ctd_unpack(&stage[wib], w);
   uint64_t* ref = scratch_opts + (size_t)slot * cap;
-  uint32_t nref = 0;
-  if (lane == 0) {
-    ctd_unpack(&stage[wib], w);
-    CtdEmit e{ref, cap, 0, 0xFFFFFFFFu, 0};
-    ctd_enumerate(w, e);
-    nref = e.n;
+  CtdEmit e{ref, cap, 0, 0xFFFFFFFFu, 0};
+  ctd_enumerate(w, e);
+  const uint32_t nref = e.n;
+  uint32_t bad = 0;
+  // impure enumerations (the Seer's and the Scholar's) change the record: ctd_lane_choose restores it around its passes
+  if (nref != 0 && w.state != 8 && w.state != 9) {
+    if (ctd_lane_count(w) != nref) {
+      bad = 1000000;
+    } else {
+      // discard_and_draw ordinals are reproduced too, so compare everything
+      for (uint32_t k = 0; k < nref && k < cap; ++k)
+        if (ctd_lane_select(w, k) != ref[k]) ++bad;
+    }
   }
-  nref = __shfl_sync(CTD_FULL, nref, 0);
-  __syncwarp();
-  uint32_t bad = 0, cnt = 0;
-  if (nref == 0 || w.state == 8 || w.state == 9) {  // impure enumerations: both paths are the scalar enumerator anyway
-    if (lane == 0) mismatches[slot] = 0;
-    return;
-  }
-  for (uint32_t k = 0; k < nref && k < cap; ++k) {
-    uint64_t d = ctd_warp_choose<true>(w, lane, choose_buf[wib], &cnt, (int)k);
-    __syncwarp();
-    if (cnt != nref) { bad += 1000000; break; }
-    uint64_t want = ref[k];
-    // discard_and_draw ordinals are reproduced too, so compare everything
-    if (d != want) ++bad;
-  }
-  if (lane == 0) mismatches[slot] = bad;
+  mismatches[slot] = bad;
 }
 
 // the same kernel specialised for the preset eight, compiled in ctd_preset_playout.cu
@@ -705,14 +699,16 @@ struct CtdPersistent {
   int sm_count;
   int per_sm;
   cudaError_t (*launch)(const Args&, int grid, cudaStream_t);
-  // enough blocks to fill every SM at the kernel's occupancy, fewer when the warps of `n` items need fewer (at least one)
+  int per_block = CTD_WARPS_PER_BLOCK;   // items one block works on at once: one per warp, or one per thread (the playouts)
+  // enough blocks to fill every SM at the kernel's occupancy, fewer when `n` items need fewer (at least one)
   int grid(uint64_t n) const {
-    const uint64_t want = (uint64_t)sm_count * (per_sm < 1 ? 1 : per_sm), need = (n + CTD_WARPS_PER_BLOCK - 1) / CTD_WARPS_PER_BLOCK;
+    const uint64_t want = (uint64_t)sm_count * (per_sm < 1 ? 1 : per_sm), need = (n + per_block - 1) / per_block;
     return need == 0 ? 1 : (int)(need < want ? need : want);
   }
 };
 // the specialised kernel of each family for games of ruleset `rs` (any other value: the generic one)
 static cudaError_t ctd_playout_kernel(int rs, CtdPersistent<CtdPlayoutArgs>& k) {
+  k.per_block = CTD_BLOCK;   // one game per thread (ctd_playout.cuh)
   if (rs == CTD_RULESET_PRESET) { k.launch = ctd_playout_preset_launch; return ctd_playout_preset_blocks_per_sm(&k.per_sm); }
   if (rs == CTD_RULESET_CLASSIC) { k.launch = ctd_playout_classic_launch; return ctd_playout_classic_blocks_per_sm(&k.per_sm); }
   k.launch = ctd_playout_generic_launch;

@@ -4,6 +4,9 @@
 // timed 230 orders (random, then hill-climbing on the best) of the 19 functions the loop runs every step (renamed here to equally long names with an order prefix, so that
 // they sit in one block in exactly this order, apart from the once-per-game code); this is the best one found for this unit
 // (classic 1.006e9 with the functions where their own names put them -> 1.141e9 env steps/s).  Regenerate with the tool after changing the rules code.
+// The order was found for the warp-per-game kernel, which also ran the warp chooser (slot 18, since removed).  On the
+// per-thread kernel (ctd_playout.cuh) this order still beats the functions' own names by 9.7 % (1.718e9 against 1.567e9
+// env steps/s, profiles/README.md, round 3).
 #pragma once
 #define ctd_count_suit ctd_h00_count_suit________________
 #define ctd_philox ctd_h01_philox____________________
@@ -23,4 +26,3 @@
 #define ctd_shuffle_bytes ctd_h15_shuffle_bytes_____________
 #define ctd_setup_round ctd_h16_setup_round_______________
 #define ctd_apply ctd_h17_apply_____________________
-#define ctd_warp_choose ctd_h18_warp_choose_______________

@@ -1,21 +1,28 @@
-// ctd_playout.cuh -- the fused random-playout kernel (run_utils.py:37-41 for a batch of games), shared by two translation
-// units: ctd_kernels.cu instantiates it for any ruleset (ctd_k_playout), ctd_preset_playout.cu with CTD_FIXED_PRESET, where
-// every option kind and character outside the preset eight (game/game.py:479-486) is marked unreachable
-// (ctd_k_playout_preset: 7.9 k instead of 10.6 k instructions, +5 % env steps/s -- the kernel is instruction-fetch bound).
+// ctd_playout.cuh -- the fused random-playout kernel (run_utils.py:37-41 for a batch of games), one translation unit per
+// ruleset family: ctd_generic_playout.cu (any ruleset, ctd_k_playout), ctd_preset_playout.cu with CTD_FIXED_PRESET and
+// ctd_classic_playout.cu with CTD_FIXED_CLASSIC, where every option kind and character outside the ruleset's eight is
+// marked unreachable.  ctd_kernels.cu includes the header for the argument block, the record movers and the two passes
+// of the choice (for its checker).
+//
+// One thread owns one game.  Its working record (CtdWork, 1.5 KB) is a local variable: local memory interleaves the
+// lanes of a warp word by word, so the same field of the warp's 32 games is one 128-byte line, and one warp instruction
+// advances every lane whose game is on that code path (DESIGN.md 3, 4).  A step is the scalar choice -- count the
+// options, draw k, select the k-th -- followed by `ctd_apply`.
 #pragma once
 #include "ctd_engine.cuh"
-#include "ctd_warp.cuh"
 
 #ifndef CTD_WARPS_PER_BLOCK
 #define CTD_WARPS_PER_BLOCK 8
 #define CTD_BLOCK (CTD_WARPS_PER_BLOCK * 32)
 #endif
-#define CTD_PLAYOUT_MIN_BLOCKS 8
-#ifndef CTD_FULL
-#define CTD_FULL 0xFFFFFFFFu
+#ifndef CTD_PLAYOUT_MIN_BLOCKS   /* resident blocks per SM the registers are bounded for: 6 x 256 threads (profiles/README.md) */
+#define CTD_PLAYOUT_MIN_BLOCKS 6
 #endif
 #ifndef CTD_PLAYOUT_KERNEL_NAME
 #define CTD_PLAYOUT_KERNEL_NAME ctd_k_playout
+#endif
+#ifndef CTD_CHOOSE_LINKAGE
+#define CTD_CHOOSE_LINKAGE static
 #endif
 
 // move one 256 B record between HBM and the warp's shared staging buffer: 32 lanes x 8 B
@@ -40,83 +47,117 @@ struct CtdPlayoutArgs {
   ctd_state* slots;  // non-null: continue from slots[0..n) instead of dealing new games
 };
 
+// Enumeration visitor of the playout's choice: counts the options and keeps the `want`-th one, stores nothing.  CtdEmit with
+// capacity 0 would do the same with one more compare per option, but as the playout's visitor it measured 17-18 % slower
+// (preset 1.333e9 against 1.603e9 env steps/s, classic 1.416e9 against 1.718e9; profiles/README.md, round 3).
+struct CtdPick {
+  uint32_t n;
+  uint32_t want;
+  uint64_t got;
+  __device__ void one(uint64_t d) {
+    if (n == want) got = d;
+    ++n;
+  }
+  __device__ void range(uint64_t base, uint32_t cnt) {   // cnt options that differ only in the ordinal field j
+    if (want >= n && want - n < cnt) got = base | ctd_f_j(want - n);
+    n += cnt;
+  }
+};
+// the two passes of the choice (ctd_k_choose_check in ctd_kernels.cu tests them against the materialised list for every k)
+__device__ __forceinline__ uint32_t ctd_lane_count(CtdWork& w) {
+  CtdPick e{0, 0xFFFFFFFFu, 0};
+  ctd_enumerate(w, e);
+  return e.n;
+}
+__device__ __forceinline__ uint64_t ctd_lane_select(CtdWork& w, uint32_t k) {
+  CtdPick e{0, k, 0};
+  ctd_enumerate(w, e);
+  return e.got;
+}
+
 #ifndef CTD_NO_PLAYOUT_KERNEL
-// Outcome statistics are accumulated per block in shared memory (one shared atomic per field and game) and flushed
-// to HBM once per block.
+// Agent.get_options, then a uniform draw among them: the counting pass, one draw, and a selecting pass over the same
+// enumeration.  Returns the chosen descriptor, 0 when there is no option.
+// The Seer's and the Scholar's enumerations are not pure (chance draws, a shrinking seven_drawn_cards): for those two
+// states the selecting pass starts from what the counting pass started from, and the game goes on from where the
+// counting pass and the draw left it.  Every other state restores nothing, so the draw's Philox block stays cached.
+CTD_CHOOSE_LINKAGE __device__ __noinline__ uint64_t ctd_lane_choose(CtdWork& w) {
+  CTD_ASSUME_WORK(&w);
+  if (w.state == 8 || w.state == 9) {
+    CTD_NOT_PRESET(); CTD_NOT_CLASSIC();
+    const uint32_t draws0 = w.draws, tape0 = w.tape_pos;
+    const uint8_t n7 = w.n_seven;
+    uint8_t s7[7];
+    for (int i = 0; i < 7; ++i) s7[i] = w.seven[i];
+    const uint32_t n = ctd_lane_count(w);
+    if (n == 0) return 0;
+    const uint32_t k = ctd_randbelow(w, n);
+    const uint32_t draws1 = w.draws, tape1 = w.tape_pos;
+    w.draws = draws0; w.tape_pos = tape0; w.n_seven = n7;
+    for (int i = 0; i < 7; ++i) w.seven[i] = s7[i];
+    const uint64_t d = ctd_lane_select(w, k);
+    w.draws = draws1; w.tape_pos = tape1;
+    return d;
+  }
+  const uint32_t n = ctd_lane_count(w);
+  if (n == 0) return 0;
+  return ctd_lane_select(w, ctd_randbelow(w, n));
+}
+
+// Every thread pulls game ids from a.counter and plays each game to its end.  The loop is flat -- one env step per trip,
+// and a thread whose game has ended records it and starts the next one inside the trip -- so that a warp does not wait
+// for its longest game before any lane starts a new one.  Outcome statistics are accumulated per block in shared memory
+// (one shared atomic per field and game) and flushed to HBM once per block.
 __global__ void __launch_bounds__(CTD_BLOCK, CTD_PLAYOUT_MIN_BLOCKS) CTD_PLAYOUT_KERNEL_NAME(CtdPlayoutArgs a) {
-  __shared__ CtdWork works[CTD_WARPS_PER_BLOCK];
-  // the record staging area (game start / end) and the scalar chooser's option buffer (inside a step) are never live together;
-  // shared memory is kept small because what is left of the 256 KB is the L1 that holds lane 0's stack
-  __shared__ __align__(16) uint64_t scratch_u64[CTD_WARPS_PER_BLOCK][CTD_CHOOSE_BUF];
-  static_assert(sizeof(ctd_state) <= CTD_CHOOSE_BUF * 8, "stage aliases the option buffer");
   __shared__ unsigned long long bst[sizeof(ctd_playout_stats) / 8];
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  ctd_state* const stage = reinterpret_cast<ctd_state*>(scratch_u64[0]);   // stage[wib] == scratch_u64[wib]
-  uint64_t (*choose_buf)[CTD_CHOOSE_BUF] = scratch_u64;
-  CtdWork& w = works[wib];
   if (threadIdx.x < sizeof(ctd_playout_stats) / 8) bst[threadIdx.x] = 0;
   __syncthreads();
   ctd_playout_stats* bs = reinterpret_cast<ctd_playout_stats*>(bst);
+  CtdWork w;
+  unsigned long long g = 0;
+  uint32_t steps0 = 0;
+  bool live = false;
   for (;;) {
-    unsigned long long g = 0;
-    if (lane == 0) g = atomicAdd(a.counter, 1ull);
-    g = __shfl_sync(CTD_FULL, g, 0);
-    if (g >= a.n_games) break;
-    if (a.slots != nullptr) {
-      ctd_record_load(&a.slots[g], &stage[wib], lane);
-      if (lane == 0) {
-        ctd_unpack(&stage[wib], w);
+    if (!live || (w.gflags & 2) || w.err || (w.steps - steps0) >= a.max_steps) {
+      if (live) {  // the game has ended: per-game outputs, block statistics, the record
+        if (!(w.gflags & 2) && !w.err) w.err |= CTD_ERR_MAXSTEPS;
+        const uint32_t ns = w.steps - steps0;
+        for (int q = 0; q < 6; ++q) {
+          const int pts = w.points[q];
+          if (a.points6) a.points6[g * 6 + q] = (int8_t)(pts > 127 ? 127 : (pts < -128 ? -128 : pts));
+          atomicAdd((unsigned long long*)&bs->points_sum[q], (unsigned long long)(long long)pts);
+          atomicAdd((unsigned long long*)&bs->points_sq[q], (unsigned long long)(pts * pts));
+        }
+        if (w.winner >= 0 && w.winner < 6) atomicAdd((unsigned long long*)&bs->wins[w.winner], 1ull);
+        if (a.winner) a.winner[g] = w.winner;
+        if (a.steps) a.steps[g] = (uint16_t)ns;
+        atomicAdd((unsigned long long*)&bs->games, 1ull);
+        atomicAdd((unsigned long long*)&bs->steps, (unsigned long long)ns);
+        atomicAdd((unsigned long long*)&bs->steps_sq, (unsigned long long)ns * ns);
+        if (w.err) atomicAdd((unsigned long long*)&bs->errors, 1ull);
+        atomicMax((unsigned long long*)&bs->max_steps, (unsigned long long)ns);
+        if (a.slots != nullptr) ctd_pack(w, &a.slots[g]);
+      }
+      g = atomicAdd(a.counter, 1ull);
+      if (g >= a.n_games) break;
+      if (a.slots != nullptr) {
+        ctd_unpack(&a.slots[g], w);
         w.k0 = (uint32_t)a.seed; w.k1 = (uint32_t)(a.seed >> 32);
         w.stream = 0;
         w.tape = nullptr; w.tape_len = 0;
-      }
-      __syncwarp();
-    } else {
-      if (lane == 0) {
+      } else {
         ctd_chance_init(w, a.seed, a.first_gid + g, 0);
-      }
-      __syncwarp();
-      if (lane == 0) {
         ctd_deal_preset(w, a.ruleset);
         ctd_setup_round<false>(w);
       }
-      __syncwarp();
+      steps0 = w.steps;
+      live = true;
+      continue;  // a continued record may already have ended
     }
-    const uint32_t steps0 = w.steps;
     // ---- the hot loop: run_utils.py:37-41 ----
-    for (;;) {
-      bool stop = (w.gflags & 2) || w.err || (w.steps - steps0) >= a.max_steps;
-      if (stop) break;
-      uint64_t d = ctd_warp_choose(w, lane, choose_buf[wib]);
-      if (lane == 0) {
-        if (d == 0) w.err |= CTD_ERR_REF_RAISE;
-        else ctd_apply<false>(w, d);
-      }
-      __syncwarp();
-    }
-    if (lane == 0 && !(w.gflags & 2) && !w.err) w.err |= CTD_ERR_MAXSTEPS;
-    __syncwarp();
-    const uint32_t ns = w.steps - steps0;
-    if (lane < 6) {  // per-seat fields: one lane per seat
-      const int pts = w.points[lane];
-      if (a.points6) a.points6[g * 6 + lane] = (int8_t)(pts > 127 ? 127 : (pts < -128 ? -128 : pts));
-      atomicAdd((unsigned long long*)&bs->points_sum[lane], (unsigned long long)(long long)pts);
-      atomicAdd((unsigned long long*)&bs->points_sq[lane], (unsigned long long)(pts * pts));
-      if (w.winner == lane) atomicAdd((unsigned long long*)&bs->wins[lane], 1ull);
-    } else if (lane == 6) {
-      if (a.winner) a.winner[g] = w.winner;
-      if (a.steps) a.steps[g] = (uint16_t)ns;
-      atomicAdd((unsigned long long*)&bs->games, 1ull);
-      atomicAdd((unsigned long long*)&bs->steps, (unsigned long long)ns);
-      atomicAdd((unsigned long long*)&bs->steps_sq, (unsigned long long)ns * ns);
-      if (w.err) atomicAdd((unsigned long long*)&bs->errors, 1ull);
-      atomicMax((unsigned long long*)&bs->max_steps, (unsigned long long)ns);
-    }
-    if (a.slots != nullptr) {
-      if (lane == 0) ctd_pack(w, &stage[wib]);
-      ctd_record_store(&a.slots[g], &stage[wib], lane);
-    }
-    __syncwarp();
+    const uint64_t d = ctd_lane_choose(w);
+    if (d == 0) w.err |= CTD_ERR_REF_RAISE;
+    else ctd_apply<false>(w, d);
   }
   __syncthreads();
   if (a.stats != nullptr && threadIdx.x < sizeof(ctd_playout_stats) / 8 && bst[threadIdx.x] != 0) {

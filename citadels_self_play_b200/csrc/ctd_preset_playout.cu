@@ -9,14 +9,15 @@
 
 #define CTD_DEVICE_ONLY 1
 #define CTD_SMALL_CAPS 1   /* real games only: small containers, small working record (ctd_engine.cuh) */
+#define CTD_WORK_LOCAL 1   /* every thread plays its own game in its own local memory (ctd_playout.cuh) */
 #define CTD_FIXED_PRESET 1
 #define CTD_PLAYOUT_KERNEL_NAME ctd_k_playout_preset
-// where ptxas puts the per-step functions (see the header): worth a few per cent on an instruction-cache-bound kernel
-#ifndef CTD_LAYOUT_HEADER
-#define CTD_LAYOUT_HEADER "ctd_layout_preset.h"
-#endif
-#define CTD_CHOOSE_LINKAGE inline   /* external name: takes part in the ordering */
+#define CTD_CHOOSE_LINKAGE inline   /* ctd_lane_choose with an external name, as measured: its place in the name order follows from it */
+// placement of the device functions by name order (tools/layout_search.py): the functions' own names measured best for this
+// kernel (profiles/README.md, round 3); the hook stays for the next search
+#ifdef CTD_LAYOUT_HEADER
 #include CTD_LAYOUT_HEADER
+#endif
 #include "ctd_playout.cuh"
 
 cudaError_t ctd_playout_preset_launch(const CtdPlayoutArgs& a, int grid, cudaStream_t stream) {
@@ -24,5 +25,8 @@ cudaError_t ctd_playout_preset_launch(const CtdPlayoutArgs& a, int grid, cudaStr
   return cudaGetLastError();
 }
 cudaError_t ctd_playout_preset_blocks_per_sm(int* per_sm) {
+  // the kernel keeps ~200 B of shared memory: what the carveout leaves over is the L1 that caches the threads' records
+  cudaError_t c = cudaFuncSetAttribute(ctd_k_playout_preset, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1);
+  if (c != cudaSuccess) return c;
   return cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, ctd_k_playout_preset, CTD_BLOCK, 0);
 }

@@ -4,6 +4,7 @@
 #pragma once
 #include "ctd_playout.cuh"
 #include "ctd_mccfr.cuh"
+#define CTD_FULL 0xFFFFFFFFu
 
 #ifndef CTD_MCCFR_KERNEL_NAME
 #define CTD_MCCFR_KERNEL_NAME ctd_k_mccfr

@@ -2,7 +2,7 @@
 
 ptxas lays the device functions of a kernel out in the order of their mangled names, and the playout kernels are bound by the SM's
 instruction cache (profiles/README.md), so WHERE the per-step functions sit relative to each other is worth +-5 %.  This script
-writes renaming headers (the format of csrc/ctd_layout_preset.h: `#define ctd_x ctd_hNN_...`) for a set of orders, builds one library per order
+writes renaming headers (the format of csrc/ctd_layout_classic.h: `#define ctd_x ctd_hNN_...`) for a set of orders, builds one library per order
 (only the playout units are recompiled) under citadels_self_play_b200/variants/, and prints the command that times them on the GPU box:
 
     python tools/layout_search.py build N SEED [parent.json ...]   # N random orders, or N mutations of the given plans
