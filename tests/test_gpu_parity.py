@@ -35,7 +35,7 @@ def _replay(engine, name, with_tape):
     for k in range(maxlen):
         live = np.nonzero(lens > k)[0]
         opts, counts = engine.enumerate(n, stride=64)
-        if k % 3 == 0:   # the playout kernel's warp-cooperative chooser: every k of every state vs this list
+        if k % 3 == 0:   # the playout kernel's choice (ctd_lane_count / ctd_lane_select): every k of every state vs this list
             mis = engine.choose_check(n)
             assert not mis[live].any(), ("cooperative chooser differs", name, k, np.nonzero(mis)[0][:5], mis[mis > 0][:5])
         states = engine.store_states(n)
@@ -96,18 +96,35 @@ def test_fused_playout_vs_oracle_fresh_seeds(engine):
 
 
 def test_playout_slots_continues_loaded_states(engine):
-    """ctd_playout_slots == finishing the game from a mid-game state (run_utils.py:37-41 tail)."""
+    """ctd_playout_slots == finishing the game from a mid-game state (run_utils.py:37-41 tail): 100 steps through enumerate /
+    step with the playout's own choice (draw number rng_draws of the game's Philox stream, which the record then counts), then
+    the fused kernel finishes the games."""
+    from oracle.philox import PhiloxChance
+    from citadels_self_play_b200.layout import STATE_DTYPE
     T = Traces("preset_full.npz")
-    n = len(T)
+    n, k = len(T), 100
+    assert np.diff(T.step_off).min() > k
     out = engine.playout(n, seed=T.seed, first_gid=int(T.gids[0]), ruleset=0)
-    # play 100 steps through enumerate/step with the Philox choice, then let the fused kernel finish
     engine.set_tapes(None)
     engine.reset(n, seed=T.seed, first_gid=int(T.gids[0]), ruleset=0)
+    assert np.array_equal(engine.store_states(n)[:, :228], T.states[T.step_off[:-1], :228])
+    for _ in range(k):
+        opts, counts = engine.enumerate(n, stride=64)
+        states = engine.store_states(n)
+        rec = states.view(STATE_DTYPE).reshape(n)
+        chosen = np.zeros(n, dtype=np.uint64)
+        for g in range(n):
+            chance = PhiloxChance(T.seed, int(rec["gid"][g]))
+            chance.i = int(rec["rng_draws"][g])
+            chosen[g] = opts[g, chance.randbelow(int(counts[g]))]
+            rec["rng_draws"][g] = chance.i
+        engine.load_states(states)
+        engine.step(chosen)
     mid = engine.store_states(n)
-    assert np.array_equal(mid[:, :228], T.states[T.step_off[:-1], :228])
+    assert np.array_equal(mid[:, :228], T.states[T.step_off[:-1] + k, :228])
     winner, steps = engine.playout_slots(n)
     assert np.array_equal(winner, out["winner"])
-    assert np.array_equal(steps, out["steps"])
+    assert np.array_equal(steps.astype(np.int64), out["steps"].astype(np.int64) - k)
     fin = engine.store_states(n)
     assert np.array_equal(fin[:, :228], T.final[:, :228])
 
